@@ -9,7 +9,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 # COPTER_B200_LIB: developer knob used by tools/sweep.py to time alternative builds
 LIB_PATH = os.environ.get('COPTER_B200_LIB') or os.path.join(PKG, 'libcopter_b200.so')
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 STATS_LEN = 16
 STATS_SLOTS = 64
 F_AUTO_RESET, F_KEEP_EPISODE = 1, 2
@@ -108,12 +108,15 @@ def load():
         f.argtypes, f.restype = [P, vp, vp, i64, i64, u64, vp], i32
     for f in (lib.copter_rollout_f32, lib.copter_rollout_f64):
         f.argtypes, f.restype = [P, B, C.POINTER(CopterActionSource), i64, i64, u64, i64, i32, i32, i32, vp, vp, vp,
-                                 C.POINTER(CopterPidGains), vp, vp], i32
+                                 C.POINTER(CopterPidGains), vp, vp, vp, vp], i32
     lib.copter_default_pid_gains.argtypes, lib.copter_default_pid_gains.restype = [C.POINTER(CopterPidGains)], None
     lib.copter_policy_mlp_f32.argtypes = [vp, i64, i64, i32, i32, vp, vp, vp, vp, vp, vp, C.c_float, C.c_float, vp, vp]
     lib.copter_policy_mlp_f32.restype = i32
-    lib.copter_policy_rollout_f32.argtypes = [P, B, C.POINTER(CopterMlpPolicy), i64, i64, u64, i64, i32, i32, i32, vp, vp, vp, vp, vp]
+    lib.copter_policy_rollout_f32.argtypes = [P, B, C.POINTER(CopterMlpPolicy), i64, i64, u64, i64, i32, i32, i32, vp, vp, vp, vp,
+                                              vp, vp, vp]
     lib.copter_policy_rollout_f32.restype = i32
+    lib.copter_gae_f32.argtypes = [vp, vp, vp, vp, vp, i64, i32, C.c_float, C.c_float, vp, vp, vp]
+    lib.copter_gae_f32.restype = i32
     lib.copter_pipeline_create.argtypes, lib.copter_pipeline_create.restype = [i32, C.POINTER(vp)], i32
     lib.copter_pipeline_destroy.argtypes, lib.copter_pipeline_destroy.restype = [vp], i32
     for f in (lib.copter_step_host_f32, lib.copter_step_host_f64):

@@ -777,6 +777,7 @@ struct RolloutArgs {
     T* controller;              // [n][16] PID memories (COPTER_SRC_PID), [n][24] (COPTER_SRC_PID_HOVER)
     T rate_kp, rate_ki, rate_kd, rate_windup, rate_big, pos_kp, pos_ki, pos_kd, pos_windup, pos_target, descent_kp, descent_kd;
     T alt_kp, alt_ki, alt_kd, alt_windup, alt_target;
+    uint8_t* cause_tn; float* final_obs_tn;   // ending records (RECORD instantiations only)
 };
 
 __device__ __forceinline__ double log_t(double a) { return log(a); }
@@ -936,8 +937,24 @@ __device__ __forceinline__ void pid_planar_heuristic(const RolloutArgs<T>& a, co
     }
 }
 
+// Row t of a rollout's ending records: the COPTER_CAUSE_* bits env i's episode ended with on this step (0 while
+// it runs) and, where it ended, the observation of the terminal state -- the bytes copter_step_* (k = 1) writes
+// into cause / final_obs.  Called before the reset replaces the state.  The rollout kernels take it in separate
+// RECORD instantiations, so the ones without records compile exactly as before.
+template <int VARIANT, typename T>
+__device__ __forceinline__ void record_ending(uint8_t* cause_tn, float* final_obs_tn, int t, int64_t n, int64_t i,
+                                              bool dn, int cause, const T (&s)[12]) {
+    constexpr int O = Variant<VARIANT>::O;
+    const int64_t row = (int64_t)t * n + i;
+    if (cause_tn) cause_tn[row] = (uint8_t)cause;
+    if (dn && final_obs_tn) {
+#pragma unroll
+        for (int j = 0; j < O; ++j) final_obs_tn[row * O + j] = (float)s[Variant<VARIANT>::first + j];
+    }
+}
+
 // PID: 0 = drawn commands, 1 = landing heuristics (4 controller memories), 2 = hover heuristics (6)
-template <typename T, int VARIANT, bool STATS, int PID>
+template <typename T, int VARIANT, bool STATS, int PID, bool RECORD>
 __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? (PID ? 5 : COPTER_F32_CTAS_PER_SM) : 2)
 copter_rollout_kernel(const __grid_constant__ KParams<T> kp, const __grid_constant__ RolloutArgs<T> a) {
     constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A;
@@ -1017,6 +1034,7 @@ copter_rollout_kernel(const __grid_constant__ KParams<T> kp, const __grid_consta
                     }
                 }
                 if (a.done_tn) a.done_tn[(int64_t)t * a.n + i] = dn ? 1 : 0;
+                if (RECORD) record_ending<VARIANT, T>(a.cause_tn, a.final_obs_tn, t, a.n, i, dn, cause, s);
                 if (dn) {
                     done_any = true;
                     if (STATS) { ep_len = steps - 1; ep_ret = ret; ret = (T)0; }
@@ -1066,13 +1084,14 @@ struct PolicyRolloutArgs {
     int64_t n, stride, env_offset, first_step; uint64_t seed; int n_steps, auto_reset;
     PolicyWeights w;
     const float* action_std;    // [A] or null: Gaussian exploration noise around the network's output
+    uint8_t* cause_tn; float* final_obs_tn;   // ending records (RECORD instantiations only)
 };
 
 #ifndef COPTER_POLICY_ROLLOUT_CTAS_PER_SM
 #define COPTER_POLICY_ROLLOUT_CTAS_PER_SM 5   // measured (tools/sweep_policy.py): 3: 0.413, 4: 0.420, 5: 0.400, 6: 0.425 ms per env-step
 #endif
 
-template <int VARIANT, bool STATS>
+template <int VARIANT, bool STATS, bool RECORD>
 __global__ void __launch_bounds__(128, COPTER_POLICY_ROLLOUT_CTAS_PER_SM)
 copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __grid_constant__ PolicyRolloutArgs a) {
     using T = float;
@@ -1140,6 +1159,7 @@ copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __
                 if (STATS) ret += r;
                 if (a.reward_tn) a.reward_tn[(int64_t)t * a.n + i] = r;
                 if (a.done_tn) a.done_tn[(int64_t)t * a.n + i] = dn ? 1 : 0;
+                if (RECORD) record_ending<VARIANT, T>(a.cause_tn, a.final_obs_tn, t, a.n, i, dn, cause, s);
                 if (dn) {
                     done_any = true;
                     if (STATS) { ep_len = steps - 1; ep_ret = ret; ret = (T)0; }
@@ -1212,7 +1232,7 @@ struct RolloutTcSmem {
 };
 static_assert(4096 + 4 * 32 * 12 * sizeof(float) <= sizeof(tc::SlotSmem), "observation staging fits behind the layer-1 alias");
 
-template <int VARIANT, bool STATS>
+template <int VARIANT, bool STATS, bool RECORD>
 __global__ void __launch_bounds__(tc::kTile + 32, COPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM)
 copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const __grid_constant__ PolicyRolloutArgs a) {
     using T = float;
@@ -1330,6 +1350,7 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
                     if (STATS) ret += r;
                     if (a.reward_tn) a.reward_tn[(int64_t)t * a.n + i] = r;
                     if (a.done_tn) a.done_tn[(int64_t)t * a.n + i] = dn ? 1 : 0;
+                    if (RECORD) record_ending<VARIANT, T>(a.cause_tn, a.final_obs_tn, t, a.n, i, dn, cause, s);
                     if (dn) {
                         done_any = true;
                         if (STATS) { ep_len = steps - 1; ep_ret = ret; ret = (T)0; }
@@ -1357,6 +1378,59 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
     if (warp == kMmaWarp) tc::tmem_free(tmem_base);
 }
 #endif  // COPTER_POLICY_ROLLOUT_TC_AVAILABLE
+
+// ------------------------------------------------------------------------------------------
+// Generalised advantage estimation over the [T][n] rows of a rollout (copter_gae_f32; the
+// recursion is written out in include/copter_b200.h).  One thread per env walks its column from
+// row T-1 back to row 0; every row is one coalesced access of the warp.  Bound by HBM: 17 bytes
+// per element (reward, value, cause in; advantage, return out), plus final_value where a
+// truncation is read.  The loads do not depend on the recursion, so a block of kGaeRows rows is
+// loaded before its arithmetic runs -- kGaeRows rows of loads in flight per thread instead of
+// one dependent round trip per row.  Every byte is touched once: streaming (evict-first) loads
+// and stores.
+// ------------------------------------------------------------------------------------------
+struct GaeArgs {
+    const float* reward; const float* value; const float* last_value; const uint8_t* cause; const float* final_value;
+    float* adv; float* ret;
+    int64_t n; int n_steps; float gamma, lam;
+};
+constexpr int kGaeRows = 8, kGaeBlock = 256;
+
+__global__ void __launch_bounds__(kGaeBlock) copter_gae_kernel(const __grid_constant__ GaeArgs a) {
+    const int64_t i = (int64_t)blockIdx.x * kGaeBlock + threadIdx.x;
+    if (i >= a.n) return;
+    const float gamma = a.gamma, gamma_lam = a.gamma * a.lam;
+    float next = a.last_value[i], adv = 0.0f;            // value of row t + 1 and A_next
+    for (int t0 = a.n_steps - 1; t0 >= 0; t0 -= kGaeRows) {
+        float r[kGaeRows], v[kGaeRows], fv[kGaeRows];
+        int c[kGaeRows];
+#pragma unroll
+        for (int k = 0; k < kGaeRows; ++k) {
+            r[k] = 0.0f; v[k] = 0.0f; c[k] = 0;
+            if (t0 - k >= 0) {
+                const int64_t o = (int64_t)(t0 - k) * a.n + i;
+                r[k] = __ldcs(a.reward + o); v[k] = __ldcs(a.value + o); c[k] = __ldcs(a.cause + o);
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < kGaeRows; ++k) {                 // the terminal state's value: truncations only
+            fv[k] = 0.0f;
+            if (t0 - k >= 0 && a.final_value && (c[k] & CAUSE_TIMEOUT)) fv[k] = __ldcs(a.final_value + (int64_t)(t0 - k) * a.n + i);
+        }
+#pragma unroll
+        for (int k = 0; k < kGaeRows; ++k) {
+            if (t0 - k >= 0) {
+                const int64_t o = (int64_t)(t0 - k) * a.n + i;
+                const float boot = c[k] == 0 ? next : fv[k];
+                const float delta = r[k] + gamma * boot - v[k];
+                adv = delta + gamma_lam * (c[k] == 0 ? adv : 0.0f);
+                __stcs(a.adv + o, adv);
+                if (a.ret) __stcs(a.ret + o, adv + v[k]);
+                next = v[k];
+            }
+        }
+    }
+}
 
 template <typename T, int VARIANT>
 __global__ void __launch_bounds__(kBlock)
@@ -1569,30 +1643,36 @@ int launch_step(const CopterParams* p, const CopterBuffers* b, int64_t n, int64_
     }
 }
 
-template <typename T, int VARIANT>
-int launch_rollout_v(const KParams<T>& kp, const RolloutArgs<T>& a, cudaStream_t s) {
+template <typename T, int VARIANT, bool R>
+int launch_rollout_vr(const KParams<T>& kp, const RolloutArgs<T>& a, cudaStream_t s) {
     if (a.src_kind == COPTER_SRC_PID) {
-        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 1><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 1>>(a.n), kBlock, 0, s>>>(kp, a);
-        else         copter_rollout_kernel<T, VARIANT, false, 1><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 1>>(a.n), kBlock, 0, s>>>(kp, a);
+        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 1, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 1, R>>(a.n), kBlock, 0, s>>>(kp, a);
+        else         copter_rollout_kernel<T, VARIANT, false, 1, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 1, R>>(a.n), kBlock, 0, s>>>(kp, a);
     } else if (a.src_kind == COPTER_SRC_PID_HOVER) {
         if constexpr (Variant<VARIANT>::A == 4 && Variant<VARIANT>::O != 12) {
             return COPTER_E_VARIANT;          // the 3-D hover heuristic reads the yaw rate: full-state observation only
         } else {
-            if (a.stats) copter_rollout_kernel<T, VARIANT, true, 2><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 2>>(a.n), kBlock, 0, s>>>(kp, a);
-            else         copter_rollout_kernel<T, VARIANT, false, 2><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 2>>(a.n), kBlock, 0, s>>>(kp, a);
+            if (a.stats) copter_rollout_kernel<T, VARIANT, true, 2, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 2, R>>(a.n), kBlock, 0, s>>>(kp, a);
+            else         copter_rollout_kernel<T, VARIANT, false, 2, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 2, R>>(a.n), kBlock, 0, s>>>(kp, a);
         }
     } else {
-        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 0><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 0>>(a.n), kBlock, 0, s>>>(kp, a);
-        else         copter_rollout_kernel<T, VARIANT, false, 0><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 0>>(a.n), kBlock, 0, s>>>(kp, a);
+        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 0, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 0, R>>(a.n), kBlock, 0, s>>>(kp, a);
+        else         copter_rollout_kernel<T, VARIANT, false, 0, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 0, R>>(a.n), kBlock, 0, s>>>(kp, a);
     }
     return (int)cudaGetLastError();
+}
+
+// the RECORD instantiations only when an ending record is asked for
+template <typename T, int VARIANT>
+int launch_rollout_v(const KParams<T>& kp, const RolloutArgs<T>& a, cudaStream_t s) {
+    return (a.cause_tn || a.final_obs_tn) ? launch_rollout_vr<T, VARIANT, true>(kp, a, s) : launch_rollout_vr<T, VARIANT, false>(kp, a, s);
 }
 
 template <typename T>
 int launch_rollout(const CopterParams* p, const CopterBuffers* b, const CopterActionSource* src, int64_t n,
                    int64_t env_offset, uint64_t seed, int64_t first_step, int n_steps, int variant, int flags,
                    void* reward_tn, uint8_t* done_tn, void* action_tn, const CopterPidGains* gains, void* controller,
-                   void* stream) {
+                   uint8_t* cause_tn, float* final_obs_tn, void* stream) {
     if (!b) return COPTER_E_ARG;
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
@@ -1607,7 +1687,7 @@ int launch_rollout(const CopterParams* p, const CopterBuffers* b, const CopterAc
     RolloutArgs<T> a;
     a.state = (T*)b->state; a.meta = b->meta; a.meta_hi = b->meta_hi; a.obs = b->obs; a.reward_sum = (T*)b->reward; a.done_any = b->done;
     a.init_force = (const T*)b->init_force; a.ep_return = (T*)b->ep_return; a.stats = b->stats;
-    a.reward_tn = (T*)reward_tn; a.done_tn = done_tn; a.action_tn = (T*)action_tn;
+    a.reward_tn = (T*)reward_tn; a.done_tn = done_tn; a.action_tn = (T*)action_tn; a.cause_tn = cause_tn; a.final_obs_tn = final_obs_tn;
     a.n = n; a.stride = b->state_stride > 0 ? b->state_stride : n; a.env_offset = env_offset; a.first_step = first_step;
     a.seed = seed; a.n_steps = n_steps; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
     a.src_kind = src->kind; a.src_scale = (T)src->scale; a.src_offset = (T)src->offset;
@@ -1741,9 +1821,9 @@ int launch_policy_v(const PolicyArgs& a, cudaStream_t s) {
 }
 
 #if COPTER_POLICY_ROLLOUT_TC_AVAILABLE
-template <int VARIANT, bool STATS>
+template <int VARIANT, bool STATS, bool RECORD>
 int launch_policy_rollout_tc(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
-    constexpr auto kernel = copter_policy_rollout_tc_kernel<VARIANT, STATS>;
+    constexpr auto kernel = copter_policy_rollout_tc_kernel<VARIANT, STATS, RECORD>;
     constexpr int smem = (int)sizeof(RolloutTcSmem) + 128;                     // dynamic: past the 48 KB static limit
     static bool configured[kMaxDevices] = {false};
     const int dev = current_device();
@@ -1757,15 +1837,21 @@ int launch_policy_rollout_tc(const KParams<float>& kp, const PolicyRolloutArgs& 
 }
 #endif
 
-template <int VARIANT>
-int launch_policy_rollout_v(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
+template <int VARIANT, bool R>
+int launch_policy_rollout_vr(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
 #if COPTER_POLICY_ROLLOUT_TC_AVAILABLE
     if (policy_rollout_tc_setting())    // the tcgen05 / TMEM kernel; default: the warp-MMA kernel
-        return a.stats ? launch_policy_rollout_tc<VARIANT, true>(kp, a, s) : launch_policy_rollout_tc<VARIANT, false>(kp, a, s);
+        return a.stats ? launch_policy_rollout_tc<VARIANT, true, R>(kp, a, s) : launch_policy_rollout_tc<VARIANT, false, R>(kp, a, s);
 #endif
-    if (a.stats) copter_policy_rollout_kernel<VARIANT, true><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, true>>(a.n), 128, 0, s>>>(kp, a);
-    else         copter_policy_rollout_kernel<VARIANT, false><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, false>>(a.n), 128, 0, s>>>(kp, a);
+    if (a.stats) copter_policy_rollout_kernel<VARIANT, true, R><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, true, R>>(a.n), 128, 0, s>>>(kp, a);
+    else         copter_policy_rollout_kernel<VARIANT, false, R><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, false, R>>(a.n), 128, 0, s>>>(kp, a);
     return (int)cudaGetLastError();
+}
+
+// the RECORD instantiations only when an ending record is asked for
+template <int VARIANT>
+int launch_policy_rollout_v(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
+    return (a.cause_tn || a.final_obs_tn) ? launch_policy_rollout_vr<VARIANT, true>(kp, a, s) : launch_policy_rollout_vr<VARIANT, false>(kp, a, s);
 }
 
 bool policy_ok(const CopterMlpPolicy* m) {
@@ -1925,13 +2011,15 @@ int copter_step_f64(const CopterParams* p, const CopterBuffers* b, int64_t n, in
 
 int copter_rollout_f32(const CopterParams* p, const CopterBuffers* b, const CopterActionSource* src, int64_t n, int64_t env_offset, uint64_t seed,
                        int64_t first_step, int n_steps, int variant, int flags, float* reward_tn, uint8_t* done_tn, float* action_tn,
-                       const CopterPidGains* gains, float* controller, void* stream) {
-    return launch_rollout<float>(p, b, src, n, env_offset, seed, first_step, n_steps, variant, flags, reward_tn, done_tn, action_tn, gains, controller, stream);
+                       const CopterPidGains* gains, float* controller, uint8_t* cause_tn, float* final_obs_tn, void* stream) {
+    return launch_rollout<float>(p, b, src, n, env_offset, seed, first_step, n_steps, variant, flags, reward_tn, done_tn, action_tn, gains, controller,
+                              cause_tn, final_obs_tn, stream);
 }
 int copter_rollout_f64(const CopterParams* p, const CopterBuffers* b, const CopterActionSource* src, int64_t n, int64_t env_offset, uint64_t seed,
                        int64_t first_step, int n_steps, int variant, int flags, double* reward_tn, uint8_t* done_tn, double* action_tn,
-                       const CopterPidGains* gains, double* controller, void* stream) {
-    return launch_rollout<double>(p, b, src, n, env_offset, seed, first_step, n_steps, variant, flags, reward_tn, done_tn, action_tn, gains, controller, stream);
+                       const CopterPidGains* gains, double* controller, uint8_t* cause_tn, float* final_obs_tn, void* stream) {
+    return launch_rollout<double>(p, b, src, n, env_offset, seed, first_step, n_steps, variant, flags, reward_tn, done_tn, action_tn, gains, controller,
+                              cause_tn, final_obs_tn, stream);
 }
 
 void copter_default_pid_gains(CopterPidGains* g) {
@@ -1983,7 +2071,8 @@ int copter_policy_mlp_f32(const void* state, int64_t state_stride, int64_t n, in
 
 int copter_policy_rollout_f32(const CopterParams* p, const CopterBuffers* b, const CopterMlpPolicy* policy, int64_t n,
                               int64_t env_offset, uint64_t seed, int64_t first_step, int n_steps, int variant, int flags,
-                              float* reward_tn, uint8_t* done_tn, float* action_tn, float* obs_tn, void* stream) {
+                              float* reward_tn, uint8_t* done_tn, float* action_tn, float* obs_tn, uint8_t* cause_tn,
+                              float* final_obs_tn, void* stream) {
     if (!b) return COPTER_E_ARG;
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
@@ -1997,6 +2086,7 @@ int copter_policy_rollout_f32(const CopterParams* p, const CopterBuffers* b, con
     a.state = (float*)b->state; a.meta = b->meta; a.meta_hi = b->meta_hi; a.obs = b->obs; a.reward_sum = (float*)b->reward; a.done_any = b->done;
     a.init_force = (const float*)b->init_force; a.ep_return = (float*)b->ep_return; a.stats = b->stats;
     a.reward_tn = reward_tn; a.done_tn = done_tn; a.action_tn = action_tn; a.obs_tn = obs_tn;
+    a.cause_tn = cause_tn; a.final_obs_tn = final_obs_tn;
     a.n = n; a.stride = b->state_stride > 0 ? b->state_stride : n; a.env_offset = env_offset; a.seed = seed;
     a.first_step = first_step; a.n_steps = n_steps; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
     a.w = policy_weights(policy); a.action_std = policy->action_std;
@@ -2010,6 +2100,20 @@ int copter_policy_rollout_f32(const CopterParams* p, const CopterBuffers* b, con
         case COPTER_HOVER1D:  return launch_policy_rollout_v<COPTER_HOVER1D>(kp, a, s);
         default:              return launch_policy_rollout_v<COPTER_TAKEOFF>(kp, a, s);
     }
+}
+
+int copter_gae_f32(const float* reward_tn, const float* value_tn, const float* last_value, const uint8_t* cause_tn,
+                   const float* final_value_tn, int64_t n, int n_steps, float gamma, float lam, float* adv_tn, float* ret_tn,
+                   void* stream) {
+    if (!reward_tn || !value_tn || !last_value || !cause_tn || !adv_tn || n < 0 || n_steps < 1) return COPTER_E_ARG;
+    if (n == 0) return 0;
+    const int64_t blocks = (n + kGaeBlock - 1) / kGaeBlock;
+    if (blocks > 0x7fffffff) return COPTER_E_RANGE;
+    GaeArgs a;
+    a.reward = reward_tn; a.value = value_tn; a.last_value = last_value; a.cause = cause_tn; a.final_value = final_value_tn;
+    a.adv = adv_tn; a.ret = ret_tn; a.n = n; a.n_steps = n_steps; a.gamma = gamma; a.lam = lam;
+    copter_gae_kernel<<<(int)blocks, kGaeBlock, 0, (cudaStream_t)stream>>>(a);
+    return (int)cudaGetLastError();
 }
 
 int copter_pipeline_create(int n_streams, void** out) {

@@ -224,44 +224,57 @@ class CopterVecEnv:
             self.controller.zero_()
         return self.obs, {}
 
-    def step(self, action, reward_out=None, done_out=None):
+    def step(self, action, reward_out=None, done_out=None, cause_out=None, final_obs_out=None):
         """
         One batched `_Task.step` (envs/task.py:77-137), k_substeps times under one action.
         Returns (obs f32 [N,O], reward [N], terminated bool [N], truncated bool [N], info).
         The returned tensors are the env's own output buffers: they are overwritten by the
         next step (clone them to keep them) -- or pass `reward_out` ([N], env dtype) and
         `done_out` ([N] uint8) to have the kernel write this step's reward / done flags
-        straight into a slice of a rollout buffer.
+        straight into a slice of a rollout buffer.  `cause_out` ([N] uint8) and `final_obs_out`
+        ([N,O] f32) do the same for the ending's COPTER_CAUSE_* bits (0 where the episode goes
+        on; reported as info['cause'] and `truncated` as with report_cause) and the terminal
+        observation (written only where an episode ended; info['final_obs']).
         """
         if not self._is_reset:
             raise CopterError('step() called before reset()')    # gymnasium's OrderEnforcing
         t = self._as_action(action)
-        for o, dt in ((reward_out, self.dtype), (done_out, torch.uint8)):
-            if o is not None and (o.dtype != dt or o.numel() != self.num_envs or not o.is_contiguous()
+        n = self.num_envs
+        for o, dt, numel in ((reward_out, self.dtype, n), (done_out, torch.uint8, n), (cause_out, torch.uint8, n),
+                             (final_obs_out, torch.float32, n * self.obs_size)):
+            if o is not None and (o.dtype != dt or o.numel() != numel or not o.is_contiguous()
                                   or o.device != self.device):
-                raise ValueError('reward_out/done_out must be contiguous [N] tensors of the env dtype / uint8 on the env device')
+                raise ValueError('reward_out/done_out/cause_out/final_obs_out must be contiguous [N] tensors of the env dtype / '
+                                 'uint8 / uint8 and an [N,O] float32 tensor on the env device')
         with torch.cuda.device(self.device):
             fn = self._lib.copter_step_f32 if self._f32 else self._lib.copter_step_f64
             b = self._buffers(t, self._force, reward_out, done_out)
+            if cause_out is not None:
+                b.cause = cause_out.data_ptr()
+            if final_obs_out is not None:
+                b.final_obs = final_obs_out.data_ptr()
             _lib.check(fn(C.byref(self.params), C.byref(b), self.num_envs, self.env_offset,
                           self.seed_value & 0xFFFFFFFFFFFFFFFF, self.k_substeps,
                           VARIANT_IDS[self.variant], _lib.F_AUTO_RESET if self.auto_reset else 0,
                           self._stream()), 'copter_step')
         self.launches += 1
         info = {}
-        if self.final_obs is not None:
-            info['final_obs'] = self.final_obs
+        final_obs = self.final_obs if final_obs_out is None else final_obs_out
+        if final_obs is not None:
+            info['final_obs'] = final_obs
         truncated = self._truncated
-        if self.cause is not None:
-            info['cause'] = self.cause
-            truncated = (self.cause & _lib.CAUSE_TIMEOUT) != 0
+        cause = self.cause if cause_out is None else cause_out
+        if cause is not None:
+            info['cause'] = cause
+            truncated = (cause & _lib.CAUSE_TIMEOUT) != 0
         return (self.obs if self.write_obs else None, self.reward if reward_out is None else reward_out,
                 (self.done if done_out is None else done_out).view(torch.bool), truncated, info)
 
     # ---- fused multi-step rollout with on-device action sources -----------------------
 
     def rollout(self, n_steps, source='const', scale=None, offset=None, record_rewards=False,
-                record_dones=False, record_actions=False, pid_gains=None):
+                record_dones=False, record_actions=False, pid_gains=None, record_causes=False,
+                record_final_obs=False):
         """
         `n_steps` env steps in ONE kernel launch, the commands generated on the device:
           source='const'    action = offset                 (default offset 1.625e-2: the
@@ -280,7 +293,14 @@ class CopterVecEnv:
                             command) holds the live vehicle at the target with the reference's gains
         Step for step identical to `n_steps` calls of step() with k_substeps=1 on the same
         commands.  Returns a dict: 'obs' (after the last step), 'reward_sum' [N], 'done_any'
-        [N] bool, plus 'rewards' [T,N], 'dones' [T,N] bool, 'actions' [T,N,A] when recorded.
+        [N] bool, plus 'rewards' [T,N], 'dones' [T,N] bool, 'actions' [T,N,A] when recorded, and
+        the episode endings a learner needs to bootstrap a truncation:
+          'causes' [T,N] uint8      (record_causes) COPTER_CAUSE_* bits of the episode that ended on
+                                    step t, 0 where it goes on; `causes & CAUSE_TIMEOUT` is the
+                                    step limit (gymnasium's `truncated`), any other ending terminates
+          'final_obs' [T,N,O] f32   (record_final_obs) the terminal observation where causes != 0
+                                    (with auto-reset obs of step t + 1 is the next episode's first);
+                                    zeros elsewhere
         """
         if not self._is_reset:
             raise CopterError('rollout() called before reset()')
@@ -303,6 +323,8 @@ class CopterVecEnv:
         rew = torch.empty((T, n), dtype=self.dtype, device=self.device) if record_rewards else None
         dn = torch.empty((T, n), dtype=torch.uint8, device=self.device) if record_dones else None
         act = torch.empty((T, n, self.action_size), dtype=self.dtype, device=self.device) if record_actions else None
+        cause = torch.empty((T, n), dtype=torch.uint8, device=self.device) if record_causes else None
+        fin = torch.zeros((T, n, self.obs_size), dtype=torch.float32, device=self.device) if record_final_obs else None
         with torch.cuda.device(self.device):
             fn = self._lib.copter_rollout_f32 if self._f32 else self._lib.copter_rollout_f64
             b = self._buffers(None, self._force)
@@ -314,6 +336,8 @@ class CopterVecEnv:
                           act.data_ptr() if act is not None else None,
                           C.byref(gains) if gains is not None else None,
                           self.controller.data_ptr() if self.controller is not None else None,
+                          cause.data_ptr() if cause is not None else None,
+                          fin.data_ptr() if fin is not None else None,
                           self._stream()), 'copter_rollout')
         self.launches += 1
         self.rollout_step += T
@@ -324,6 +348,10 @@ class CopterVecEnv:
             out['dones'] = dn.view(torch.bool)
         if act is not None:
             out['actions'] = act
+        if cause is not None:
+            out['causes'] = cause
+        if fin is not None:
+            out['final_obs'] = fin
         return out
 
     # ---- host-array API (numpy in / numpy out, as the reference's callers use it) ------

@@ -7,6 +7,11 @@ policy reads the env's observation tensor in place, the step kernel reads the po
 tensor in place and writes reward / done straight into row t of the [T, N] rollout buffers
 (GAE-ready layout), and the whole T-step horizon is captured once in a CUDA graph and replayed,
 so a rollout costs one graph launch instead of T x (policy kernels + 1) launches.
+
+Both rollout classes can also record how each step ended (`store_causes`: the COPTER_CAUSE_* bits,
+so that a step-limit truncation is told apart from a termination) and the terminal observation
+(`store_final_obs`: with auto-reset, obs of step t + 1 already belongs to the next episode).  `gae`
+turns rewards, the learner's values and those records into advantages and returns in one kernel.
 """
 
 import ctypes as C
@@ -17,7 +22,26 @@ from . import _lib
 from ._lib import CopterError, VARIANT_IDS
 
 
-class PolicyRollout:
+class _EndingRecords:
+    """`terminated` / `truncated` [T,N] bool of a rollout that stores its causes: truncated = the env's own step
+    limit (CAUSE_TIMEOUT, gymnasium's TimeLimit `truncated`), terminated = any other ending."""
+
+    def _causes(self):
+        if self.causes is None:
+            raise CopterError('construct the rollout with store_causes=True')
+        return self.causes
+
+    @property
+    def truncated(self):
+        return (self._causes() & _lib.CAUSE_TIMEOUT) != 0
+
+    @property
+    def terminated(self):
+        c = self._causes()
+        return (c != 0) & ((c & _lib.CAUSE_TIMEOUT) == 0)
+
+
+class PolicyRollout(_EndingRecords):
     """
     env      a CopterVecEnv (already constructed on the target device)
     policy   callable obs[N,O] f32 -> action[N,A] (torch module or function; runs under no_grad)
@@ -25,9 +49,14 @@ class PolicyRollout:
     store_obs  also keep obs_t (the observation the policy saw) in a [T, N, O] buffer
     planar     the policy takes the env's fp32 state planes [3,N,4] in place (see PlanarLinear)
                instead of the packed observation; combine with CopterVecEnv(write_obs=False)
+    store_causes     also keep `causes` [T,N] uint8: the COPTER_CAUSE_* bits of the episode that ended
+                     on step t, 0 where it goes on (`terminated` / `truncated` are derived from it)
+    store_final_obs  also keep `final_obs` [T,N,O] f32: the terminal observation where causes != 0
+                     (zero-initialised; rows of steps where nothing ended are left as they were)
     """
 
-    def __init__(self, env, policy, horizon, store_obs=False, use_cuda_graph=True, planar=False):
+    def __init__(self, env, policy, horizon, store_obs=False, use_cuda_graph=True, planar=False,
+                 store_causes=False, store_final_obs=False):
         self.env, self.policy, self.horizon = env, policy, int(horizon)
         self.planar = bool(planar)
         if not planar and not env.write_obs:
@@ -38,6 +67,8 @@ class PolicyRollout:
         self.rewards = torch.zeros((self.horizon, n), dtype=env.dtype, device=dev)
         self.dones = torch.zeros((self.horizon, n), dtype=torch.uint8, device=dev)
         self.obs = torch.zeros((self.horizon, n, env.obs_size), dtype=torch.float32, device=dev) if store_obs else None
+        self.causes = torch.zeros((self.horizon, n), dtype=torch.uint8, device=dev) if store_causes else None
+        self.final_obs = torch.zeros((self.horizon, n, env.obs_size), dtype=torch.float32, device=dev) if store_final_obs else None
         self.last_obs = env.obs                       # observation after the last step (bootstrap value input)
         self.use_cuda_graph = use_cuda_graph
         self._graph = None
@@ -51,7 +82,9 @@ class PolicyRollout:
             action = self.policy(env.planar_obs() if self.planar else env.obs)
             if action.dtype != env.dtype:
                 action = action.to(env.dtype)
-            env.step(action, reward_out=self.rewards[t], done_out=self.dones[t])
+            env.step(action, reward_out=self.rewards[t], done_out=self.dones[t],
+                     cause_out=self.causes[t] if self.causes is not None else None,
+                     final_obs_out=self.final_obs[t] if self.final_obs is not None else None)
 
     @torch.no_grad()
     def run(self):
@@ -146,7 +179,7 @@ class FusedMLPPolicy:
         return self.action
 
 
-class FusedPolicyRollout:
+class FusedPolicyRollout(_EndingRecords):
     """
     The whole policy-in-the-loop horizon as ONE kernel launch (copter_policy_rollout_f32): every
     warp evaluates the tanh MLP O -> 64 -> 64 -> A for its 32 envs from the state its lanes hold
@@ -163,10 +196,13 @@ class FusedPolicyRollout:
                 log-std, read in place): Gaussian exploration, action = policy(obs) + std * N(0,1), the
                 noise from Philox keyed by (seed, global env id, env.rollout_step + t) -- reproducible and
                 independent of how the rollout is cut into horizons
+    store_causes / store_final_obs   also record `causes` [T,N] uint8 and `final_obs` [T,N,O] as
+                PolicyRollout does (the step-limit truncations a learner bootstraps from the value of
+                final_obs; `terminated` / `truncated` [T,N] bool are derived from causes)
     """
 
     def __init__(self, env, net, horizon, out_scale=1.0, out_offset=0.0, store_obs=False, store_actions=False,
-                 action_std=None):
+                 action_std=None, store_causes=False, store_final_obs=False):
         probe = FusedMLPPolicy(env, net, out_scale, out_offset)       # same parameter checks
         if env.k_substeps != 1:
             raise CopterError('FusedPolicyRollout steps with k_substeps == 1')
@@ -187,6 +223,8 @@ class FusedPolicyRollout:
         self.dones = torch.zeros((self.horizon, n), dtype=torch.uint8, device=dev)
         self.obs = torch.zeros((self.horizon, n, env.obs_size), dtype=torch.float32, device=dev) if store_obs else None
         self.actions = torch.zeros((self.horizon, n, env.action_size), dtype=torch.float32, device=dev) if store_actions else None
+        self.causes = torch.zeros((self.horizon, n), dtype=torch.uint8, device=dev) if store_causes else None
+        self.final_obs = torch.zeros((self.horizon, n, env.obs_size), dtype=torch.float32, device=dev) if store_final_obs else None
         self.launches_per_rollout = 1
 
     def run(self):
@@ -204,10 +242,59 @@ class FusedPolicyRollout:
                 _lib.F_AUTO_RESET if env.auto_reset else 0, self.rewards.data_ptr(), self.dones.data_ptr(),
                 self.actions.data_ptr() if self.actions is not None else None,
                 self.obs.data_ptr() if self.obs is not None else None,
+                self.causes.data_ptr() if self.causes is not None else None,
+                self.final_obs.data_ptr() if self.final_obs is not None else None,
                 C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)), 'copter_policy_rollout')
         env.launches += 1
         env.rollout_step += self.horizon
         return self.rewards, self.dones.view(torch.bool), env.obs if env.write_obs else None
+
+
+def gae(rewards, values, last_values, causes, final_values=None, gamma=0.99, lam=0.95):
+    """
+    Generalised advantage estimation on the device (copter_gae_f32, one kernel over the [T,N] rows).
+    rewards, values [T,N] f32; last_values [N] f32 (value of the observation after the last step);
+    causes [T,N] uint8 (a rollout's `causes`); final_values [T,N] f32 or None (value of `final_obs`,
+    read only where a step-limit truncation is).  For t = T-1 .. 0:
+        next  = last_values if t == T-1 else values[t+1]
+        boot  = next where causes[t] == 0; final_values[t] where the step limit fired (CAUSE_TIMEOUT) and
+                final_values is given; 0 otherwise (with final_values None, truncations are terminations)
+        delta = rewards[t] + gamma * boot - values[t]
+        A[t]  = delta + gamma * lam * (A[t+1] where causes[t] == 0, else 0)
+    Returns (advantages [T,N], returns = advantages + values), fp32.  fp32 arithmetic in that order.
+    """
+    if not all(isinstance(x, torch.Tensor) for x in (rewards, values, last_values, causes)) or \
+            (final_values is not None and not isinstance(final_values, torch.Tensor)):
+        raise ValueError('gae takes torch tensors')
+    if rewards.dim() != 2:
+        raise ValueError('rewards must be [T, N], got %s' % (tuple(rewards.shape),))
+    T, n = rewards.shape
+    if T < 1:
+        raise ValueError('gae needs at least one step')
+    named = [('rewards', rewards, torch.float32, (T, n)), ('values', values, torch.float32, (T, n)),
+             ('last_values', last_values, torch.float32, (n,)), ('causes', causes, torch.uint8, (T, n))]
+    if final_values is not None:
+        named.append(('final_values', final_values, torch.float32, (T, n)))
+    for name, x, dt, shape in named:
+        if x.dtype == torch.float64:
+            raise ValueError('%s is float64: gae computes in fp32; pass %s.float()' % (name, name))
+        if x.dtype != dt:
+            raise ValueError('%s must be %s, got %s' % (name, dt, x.dtype))
+        if tuple(x.shape) != shape:
+            raise ValueError('%s must have shape %s (T, N of rewards), got %s' % (name, shape, tuple(x.shape)))
+    for name, x, _, _ in named:
+        if x.device.type != 'cuda' or x.device != rewards.device:
+            raise CopterError('%s must be on the CUDA device of rewards (there is no CPU fallback)' % name)
+        if not x.is_contiguous():
+            raise CopterError('%s must be contiguous' % name)
+    adv, ret = torch.empty_like(rewards), torch.empty_like(rewards)
+    with torch.cuda.device(rewards.device):
+        _lib.check(_lib.load().copter_gae_f32(
+            rewards.data_ptr(), values.data_ptr(), last_values.data_ptr(), causes.data_ptr(),
+            final_values.data_ptr() if final_values is not None else None, n, T, C.c_float(gamma), C.c_float(lam),
+            adv.data_ptr(), ret.data_ptr(), C.c_void_p(torch.cuda.current_stream(rewards.device).cuda_stream)),
+            'copter_gae')
+    return adv, ret
 
 
 def mlp_policy(obs_size, action_size, hidden=64, dtype=torch.bfloat16, device='cuda', seed=0):

@@ -57,7 +57,7 @@
 extern "C" {
 #endif
 
-#define COPTER_ABI_VERSION 3
+#define COPTER_ABI_VERSION 4
 
 /* dynamics/__init__.py:65-68 */
 enum { COPTER_STATUS_CRASHED = 0, COPTER_STATUS_LANDED = 1, COPTER_STATUS_LEVELING = 2, COPTER_STATUS_AIRBORNE = 3 };
@@ -187,7 +187,16 @@ int copter_step_f64(const CopterParams* p, const CopterBuffers* b, int64_t n, in
  * b->action is unused; b->reward / b->done (nullable here) receive the per-env reward SUM and
  * "any episode finished" flag of the launch, b->obs the observation after the last step.
  * Optional per-step outputs: reward_tn T[n_steps][n], done_tn uint8[n_steps][n] (GAE-ready
- * layout), action_tn T[n_steps][n][A] (the commands used, before clipping).
+ * layout), action_tn T[n_steps][n][A] (the commands used, before clipping), and the episode
+ * endings a learner needs to tell a termination from a truncation:
+ *   cause_tn uint8[n_steps][n]       the COPTER_CAUSE_* bits of the episode env i ended on step t,
+ *                                    else 0; written for every env on every step, so
+ *                                    done_tn[t][i] == (cause_tn[t][i] != 0)
+ *   final_obs_tn float[n_steps][n][O] the observation of that terminal state (with auto-reset,
+ *                                    obs of step t + 1 already belongs to the next episode);
+ *                                    written only where cause_tn[t][i] != 0, other rows untouched
+ * Per step these are exactly the bytes copter_step_* (k_substeps = 1) writes into b->cause and
+ * b->final_obs, which the rollout calls leave unused.
  */
 enum { COPTER_SRC_CONST = 0, COPTER_SRC_RANDN = 1, COPTER_SRC_UNIFORM = 2, COPTER_SRC_PID = 3, COPTER_SRC_PID_HOVER = 4 };
 typedef struct CopterActionSource { int32_t kind; int32_t reserved; double scale; double offset; } CopterActionSource;
@@ -229,11 +238,13 @@ void copter_default_pid_gains(CopterPidGains* g);
 int copter_rollout_f32(const CopterParams* p, const CopterBuffers* b, const CopterActionSource* src,
                        int64_t n, int64_t env_offset, uint64_t seed, int64_t first_step, int n_steps,
                        int variant, int flags, float* reward_tn, uint8_t* done_tn, float* action_tn,
-                       const CopterPidGains* gains_or_null, float* controller_or_null, void* stream);
+                       const CopterPidGains* gains_or_null, float* controller_or_null,
+                       uint8_t* cause_tn, float* final_obs_tn, void* stream);
 int copter_rollout_f64(const CopterParams* p, const CopterBuffers* b, const CopterActionSource* src,
                        int64_t n, int64_t env_offset, uint64_t seed, int64_t first_step, int n_steps,
                        int variant, int flags, double* reward_tn, uint8_t* done_tn, double* action_tn,
-                       const CopterPidGains* gains_or_null, double* controller_or_null, void* stream);
+                       const CopterPidGains* gains_or_null, double* controller_or_null,
+                       uint8_t* cause_tn, float* final_obs_tn, void* stream);
 
 /*
  * Batched Dynamics.setMotors: state T[12/V][n][V], status uint8[n], ticks int32[n],
@@ -285,7 +296,8 @@ int copter_policy_mlp_f32(const void* state, int64_t state_stride, int64_t n, in
  * b->obs (nullable) the observation after the last step.  Optional per-step outputs (nullable):
  * reward_tn float[n_steps][n], done_tn uint8[n_steps][n], action_tn float[n_steps][n][A] (the
  * commands before the env's clip), obs_tn float[n_steps][n][O] (the observation the policy
- * acted on at step t).
+ * acted on at step t), cause_tn uint8[n_steps][n] and final_obs_tn float[n_steps][n][O] (the
+ * episode endings and terminal observations, as for copter_rollout_*).
  * Exploration (what an on-policy learner such as PPO rolls out): with policy->action_std set
  * (A floats, device memory) the command is drawn around the network's output,
  *     action_j = out_offset + out_scale * tanh(.)_j + action_std[j] * xi_j,   xi ~ N(0,1),
@@ -303,7 +315,30 @@ typedef struct CopterMlpPolicy {
 int copter_policy_rollout_f32(const CopterParams* p, const CopterBuffers* b, const CopterMlpPolicy* policy,
                               int64_t n, int64_t env_offset, uint64_t seed, int64_t first_step, int n_steps,
                               int variant, int flags, float* reward_tn, uint8_t* done_tn, float* action_tn,
-                              float* obs_tn, void* stream);
+                              float* obs_tn, uint8_t* cause_tn, float* final_obs_tn, void* stream);
+
+/*
+ * Generalised advantage estimation over the [T][n] rows of a rollout, one pass on the device.
+ * For each env i and t = n_steps-1 .. 0 (fp32, evaluated in this order):
+ *     next  = t == T-1 ? last_value[i] : value[t+1][i]
+ *     c     = cause[t][i];  trunc = (c & COPTER_CAUSE_TIMEOUT) != 0
+ *     boot  = c == 0 ? next : (trunc && final_value ? final_value[t][i] : 0)
+ *     delta = reward[t][i] + gamma * boot - value[t][i]
+ *     A     = delta + gamma * lam * (c == 0 ? A_next : 0)            (A_next = 0 at t = T-1)
+ *     adv[t][i] = A;  ret[t][i] = A + value[t][i]
+ * cause_tn is the cause_tn row block of copter_rollout_* / copter_policy_rollout_f32.  A step
+ * that ended by the env's own step limit (COPTER_CAUSE_TIMEOUT, gymnasium's `truncated`) is
+ * bootstrapped from final_value, the caller's value of the terminal observation (final_obs_tn);
+ * with final_value NULL every ending, truncations included, is treated as a termination (boot 0).
+ * value_tn float[n_steps][n], last_value float[n] (value of the observation after the last
+ * step), final_value float[n_steps][n] (read only where a truncation is), adv_tn float[n_steps][n],
+ * ret_tn float[n_steps][n] (nullable).  COPTER_E_ARG for a NULL required pointer, n < 0 or
+ * n_steps < 1 (checked before anything touches the device).
+ */
+int copter_gae_f32(const float* reward_tn, const float* value_tn, const float* last_value,
+                   const uint8_t* cause_tn, const float* final_value_tn_or_null,
+                   int64_t n, int n_steps, float gamma, float lam,
+                   float* adv_tn, float* ret_tn_or_null, void* stream);
 
 /*
  * The same step for callers that hold HOST arrays (the reference's callers pass numpy
