@@ -11,9 +11,8 @@
 //     polynomials below behind an exact fp64 Cody-Waite reduction, sqrt is the IEEE one, and the two
 //     approximate reward helpers of the DEVICE path (MUFU.RSQ / MUFU.RCP, reward_sqrt / reward_div below)
 //     touch the reward only, never the state or a flag;
-//   * the arithmetic is a template over a LANE type L: float, double, or (device only) a packed pair
-//     of floats that steps two envs with fma.rn.f32x2 -- two independent IEEE operations per
-//     instruction, so the packed K-fused loop produces the bits of the scalar one.
+//   * the arithmetic is a template over a LANE type L (float or double): any type with the lane
+//     operations below instantiates the same sequence of IEEE operations.
 //
 // What each function restates (paths relative to the reference root):
 //   motor_forces()        gym_copter/dynamics/__init__.py:120-132, 231-247   (Eq. 6)
@@ -45,10 +44,6 @@
 #define COPTER_HD __host__ __device__ __forceinline__
 #else
 #define COPTER_HD inline
-#endif
-
-#ifndef COPTER_LIBM_ONLY
-#define COPTER_LIBM_ONLY 0      // 1 (A/B knob, device only): library sincosf, IEEE sqrt and division everywhere
 #endif
 
 namespace copter {
@@ -138,8 +133,7 @@ inline KParams<T> make_kparams(const CopterParams& p, bool wide = false) {
 
 // ------------------------------------------------------------------------------------------
 // lane operations.  A lane type L supports L(scalar) (broadcast), unary minus, + - * as separate
-// IEEE operations, and fma_ as ONE fused operation.  float and double are lanes as they are; the
-// packed pair of floats (F2) is defined in copter_physics.cuh.
+// IEEE operations, and fma_ as ONE fused operation.  float and double are lanes as they are.
 // ------------------------------------------------------------------------------------------
 COPTER_HD float  fma_(float a, float b, float c)    { return fmaf(a, b, c); }
 COPTER_HD double fma_(double a, double b, double c) { return fma(a, b, c); }
@@ -266,8 +260,8 @@ COPTER_HD Forces<T> motor_forces(const KParams<T>& kp, T m0, T m1, T m2, T m3) {
 // envs/task.py:179-184; 6 for the Dynamics facade).  `na` / `nc` receive the shaping numerators
 // sum_j inc_j (2 s_j + inc_j) over (x,dx,y,dy,z,dz) and (psi,dpsi), inc_j = dt*ds_j being the Euler
 // increment BEFORE it is rounded into the state -- see shaping_delta.  Shared by dynamics_update and
-// the straight-line substeps of the K-fused loops (scalar and packed), which therefore produce the
-// same bits.  Every operation below is one IEEE operation; the comments give the reference expression.
+// the straight-line substeps of the K-fused loop, which therefore produce the same bits.  Every
+// operation below is one IEEE operation; the comments give the reference expression.
 template <typename L, typename T, int NP, bool PERT>
 COPTER_HD void airborne_integrate(const KParams<T>& kp, L (&s)[12], const Forces<L>& f, const L (&p)[NP],
                                   L sph, L cph, L sth, L cth, L sps, L cps, L& na, L& nc) {
@@ -352,7 +346,7 @@ COPTER_HD void shaping_sums(const T (&s)[12], T& spos, T& spsi) {
 // budget); the host restatement and the fp64 path use the IEEE operations, so fp32 rewards agree
 // between device and host to ~1e-6 relative while states and flags agree bit for bit.
 COPTER_HD float reward_sqrt(float a) {
-#if defined(__CUDA_ARCH__) && !COPTER_LIBM_ONLY
+#if defined(__CUDA_ARCH__)
     return a > 0.0f ? a * rsqrtf(a) : 0.0f;
 #else
     return sqrtf(a);
@@ -360,7 +354,7 @@ COPTER_HD float reward_sqrt(float a) {
 }
 COPTER_HD double reward_sqrt(double a) { return sqrt(a); }
 COPTER_HD float reward_div(float n, float d) {
-#if defined(__CUDA_ARCH__) && !COPTER_LIBM_ONLY
+#if defined(__CUDA_ARCH__)
     return __fdividef(n, d);
 #else
     return n / d;
@@ -540,8 +534,8 @@ COPTER_HD void motors_from_action(const T* act, T (&m)[4]) {
 // ------------------------------------------------------------------------------------------
 // One launch of the step for ONE env, the plain way: k substeps under one action through the general
 // env_advance, rewards telescoped per run exactly as the kernels do (K = 1 uses env_substep).  This is
-// the definition the kernels' fast paths (straight-line substeps, calm streaks, packed pairs, warp
-// votes) must reproduce; the host restatement (oracle/copter_host.cpp) is a loop over it.
+// the definition the kernels' fast paths (straight-line substeps, calm streaks, warp votes) must
+// reproduce; the host restatement (oracle/copter_host.cpp) is a loop over it.
 // ------------------------------------------------------------------------------------------
 template <typename T> struct EnvOut { T reward; bool done; int cause; int executed; int final_steps; bool has_final; T final_state[12]; };
 

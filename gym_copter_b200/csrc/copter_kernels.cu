@@ -27,8 +27,8 @@ struct StepArgs {
     int64_t n, stride, env_offset; uint64_t seed; int k; int auto_reset;
 };
 
-// One env's inputs exactly as they sit in HBM (128-bit vectors), so that the loads of the
-// NEXT tile can be issued before the arithmetic of the current one without being decoded.
+// One env's inputs exactly as they sit in HBM (128-bit vectors): load_raw issues every load, and
+// ties the fp64 action row to the loaded words, before decode_raw unpacks anything.
 template <typename T, int A> struct RawEnv {
     typename Vec<T>::type plane[12 / Vec<T>::V];
     T act[A];
@@ -40,10 +40,6 @@ __device__ __forceinline__ uint32_t low_word(double v) { return (uint32_t)__doub
 __device__ __forceinline__ float  or_words(float v, uint32_t m)  { return __uint_as_float(__float_as_uint(v) | m); }
 __device__ __forceinline__ double or_words(double v, uint32_t m) { return __hiloint2double(__double2hiint(v) | (int)m, __double2loint(v) | (int)m); }
 
-#ifndef COPTER_TIE_LOADS
-#define COPTER_TIE_LOADS 1        // 0 (A/B knob): leave the placement of the action row's first use to ptxas
-#endif
-
 template <typename T, int A>
 __device__ __forceinline__ void load_raw(const StepArgs<T>& a, int64_t i, RawEnv<T, A>& r) {
     using V4 = typename Vec<T>::type;
@@ -51,7 +47,7 @@ __device__ __forceinline__ void load_raw(const StepArgs<T>& a, int64_t i, RawEnv
     const V4* planes = reinterpret_cast<const V4*>(a.state);
 #pragma unroll
     for (int pl = 0; pl < 12 / V; ++pl)
-        r.plane[pl] = COPTER_STREAMING ? __ldcs(&planes[(int64_t)pl * a.stride + i]) : planes[(int64_t)pl * a.stride + i];
+        r.plane[pl] = planes[(int64_t)pl * a.stride + i];
     r.meta = a.meta[i];
     r.meta_hi = a.meta_hi ? a.meta_hi[i] : 0u;
     if constexpr (A == 4 && sizeof(T) == 4) {
@@ -80,7 +76,7 @@ __device__ __forceinline__ void load_raw(const StepArgs<T>& a, int64_t i, RawEnv
     // had the good order anyway (0.1908 vs 0.1887 ms fp64; fp32 K = 1 0.4191 vs 0.4176, K = 4 0.593 vs
     // 0.585) and saves 14 % where it had not, so it is applied to the fp64 kernels, where the bad
     // order has been seen; the fp32 kernels keep ptxas' own schedule, pinned by tests/test_sass_guards.py.
-    if (COPTER_TIE_LOADS && sizeof(T) == 8) {
+    if (sizeof(T) == 8) {
         uint32_t mix = r.meta;
 #pragma unroll
         for (int pl = 0; pl < 12 / V; ++pl) mix |= low_word(r.plane[pl].x);
@@ -153,12 +149,11 @@ __device__ __forceinline__ void debit_idle_steps(double* stats, int lane, int id
 // kernels
 // ------------------------------------------------------------------------------------------
 
-// One tile (this thread's env `i`, already loaded as `cur`) through K substeps and out to HBM.
+// One tile (this thread's env `i`) in from HBM, through K substeps and out to HBM.
 // SINGLE = the K == 1 specialisation: no substep loop, no idle bookkeeping (about 40 fewer
 // instructions per env-step on the HBM-bound path).
-template <typename T, int VARIANT, bool STATS, bool SINGLE, bool PRELOADED>
-__device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T>& a,
-                                          const RawEnv<T, Variant<VARIANT>::A>& preloaded, float* tiles, int64_t tile_id) {
+template <typename T, int VARIANT, bool STATS, bool SINGLE>
+__device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T>& a, float* tiles, int64_t tile_id) {
     constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A;
     // (recomputed here rather than passed in: cheaper than keeping five values live across the body)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -175,13 +170,9 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
     T ret = (T)0, ep_ret = (T)0; int ep_cause = 0, ep_len = 0, n_steps = 0;     // STATS only
 
     if (valid) {
-        if constexpr (PRELOADED) {
-            decode_raw<T, VARIANT>(preloaded, a.meta_hi != nullptr, s, m, st, steps, episode);
-        } else {
-            RawEnv<T, A> cur;
-            load_raw<T, A>(a, i, cur);
-            decode_raw<T, VARIANT>(cur, a.meta_hi != nullptr, s, m, st, steps, episode);
-        }
+        RawEnv<T, A> cur;
+        load_raw<T, A>(a, i, cur);
+        decode_raw<T, VARIANT>(cur, a.meta_hi != nullptr, s, m, st, steps, episode);
         if (STATS && a.ep_return) ret = a.ep_return[i];
     } else {
 #pragma unroll
@@ -228,33 +219,18 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
         RewardRun<T> run;
         run_begin<T, VARIANT>(kp, run, s);
         T na = (T)0, nc = (T)0, dz_prev = s[5]; int cause = 0;
-        constexpr int kUnroll = COPTER_K_UNROLL;
         bool live = valid;                                             // has an env that still takes substeps in this launch
         bool ended = false;                                            // its episode ended in this launch
-#pragma unroll kUnroll
+#pragma unroll 1
         for (int k = 0; k < a.k; ++k) {
             if (__all_sync(0xffffffffu, !live)) break;                 // whole warp finished: idle
             // Straight-line substep when every live env of the warp is in the common case (airborne,
             // clear of the ground, past the first step of its episode, small angles): no status
             // machine, no perturbation, one predicated region.  Anything else takes the general step.
             const bool hot = airborne_hot<T>(s, st, steps);
-            const bool fast = COPTER_FAST_SUBSTEP && __all_sync(0xffffffffu, (int)!live | (int)hot);
-            // Substep 0 of a launch on a batch whose episodes are spread over all phases: some lane of almost every
-            // warp starts a fresh episode (it reset inside the previous launch) and owes the reset perturbation, which
-            // used to send the whole warp through the general step.  The straight-line step with the perturbation
-            // terms (exactly dynamics_update's airborne case, zeros for the lanes that are not fresh) covers it.
-            bool fresh = false;
-            if (COPTER_FAST_SUBSTEP && COPTER_FRESH_FAST && !fast && k == 0)
-                fresh = __all_sync(0xffffffffu, (int)!live | (int)airborne_hot_fresh<T>(s, st));
-            // A crash takes three steps (touch-down, CRASHED, done; dynamics/__init__.py:162-177, task.py:121), a landing
-            // more: while such a lane is the only thing between the warp and the straight-line step, the airborne
-            // lanes take it anyway and the lane on the ground runs the status machine beside them (divergent, but
-            // its step has no arithmetic), instead of everybody going through the general step.
-            bool mixed = false;
-            if (COPTER_FAST_SUBSTEP && COPTER_GROUND_SPLIT && !Variant<VARIANT>::direct && !fast)
-                mixed = __all_sync(0xffffffffu, (int)!live | (int)hot | (int)on_ground<T>(s, st));
+            const bool fast = __all_sync(0xffffffffu, (int)!live | (int)hot);
             bool dn = false;
-            if (COPTER_CALM_STREAK && fast) {                           // warp-uniform
+            if (fast) {                                                // warp-uniform
                 // Streak of straight-line substeps: as long as every live lane stays calm (airborne_calm:
                 // nothing ended, still in the common case) the next substep needs neither the ending flags
                 // nor the hot test -- one compare chain and one vote per substep.  The loop is executed by
@@ -265,7 +241,7 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
                     if (live) {
                         dz_prev = s[5];
                         tmo = steps == kp.max_steps;
-                        airborne_arith<T, T>(kp, s, forces, na, nc);
+                        airborne_arith<T>(kp, s, forces, na, nc);
                         ++steps;
                         calm = airborne_calm<T>(kp, s[0], s[2], s[4], s[5], s[6], s[8], s[10], tmo);
                         if (calm) { run.na += na; run.nc += nc; }
@@ -286,38 +262,9 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
                 }
             } else if (live) {
                 dz_prev = s[5];
-                if (fast || fresh || (mixed && hot)) {
-                    const bool tmo = steps == kp.max_steps;
-                    if (fresh) { airborne_arith_pert<T, T>(kp, s, forces, pert, na, nc); pert[0] = (T)0; pert[1] = (T)0; pert[2] = (T)0; }
-                    else airborne_arith<T, T>(kp, s, forces, na, nc);
-                    steps = min(steps + 1, kp.steps_cap);
-                    const int end = airborne_flags<T, VARIANT>(kp, s[0], s[2], s[6], s[8], tmo);
-                    ++run.steps;
-                    if (!(end & END_ANGLE)) { run.na += na; run.nc += nc; }
-                    dn = end != 0;
-                    if (dn) cause = airborne_cause(end);
-                } else {
-                    env_advance<T, VARIANT>(kp, s, st, steps, forces, pert, na, nc, dn, cause);
-                    pert[0] = (T)0; pert[1] = (T)0; pert[2] = (T)0;
-                    run_step<T>(run, na, nc, cause);
-                }
-            }
-            // A vehicle that has reached the ground finishes there: touch-down, CRASHED or LEVELING -> LANDED, done
-            // (dynamics/__init__.py:152-177, task.py:121, lander.py:64-72) -- steps of the status machine alone, no
-            // arithmetic, the state does not move.  Left to the loop, every one of them sent the WHOLE warp through the
-            // general step (5.7 of a K = 16 launch's substeps on a desynchronised batch, profiles/r2_step_kernel_k16_*).
-            // COPTER_GROUND_FF (A/B knob, off: measured slower, see copter_physics.cuh): the lane takes them here instead,
-            // alone, at once, as far as the launch's substeps reach, and is out of the loop afterwards -- finished, or
-            // parked in its ground status for the next launch.
-            if (COPTER_GROUND_FF && !Variant<VARIANT>::direct && live && !dn && on_ground<T>(s, st)) {
-                if (COPTER_GROUND_FF == 2) { na = (T)0; nc = (T)0; }        // (what env_advance reports for a step that moves nothing)
-                for (int kk = k + 1; kk < a.k && !dn; ++kk) {
-                    dz_prev = s[5];
-                    if (COPTER_GROUND_FF == 2) ground_advance<T, VARIANT>(kp, s, st, steps, dn, cause);
-                    else env_advance<T, VARIANT>(kp, s, st, steps, forces, pert, na, nc, dn, cause);
-                    run_step<T>(run, na, nc, cause);
-                }
-                live = false;
+                env_advance<T, VARIANT>(kp, s, st, steps, forces, pert, na, nc, dn, cause);
+                pert[0] = (T)0; pert[1] = (T)0; pert[2] = (T)0;
+                run_step<T>(run, na, nc, cause);
             }
             // An env that ends idles for the rest of the launch, so everything its ending needs -- the run's reward, the
             // terminal observation, the reset -- waits until after the loop, where the lanes that did not end take the
@@ -360,406 +307,16 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
 template <typename T, int VARIANT, bool STATS>
 __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? COPTER_STEP_CTAS_PER_SM : 2)
 copter_step_kernel(const __grid_constant__ KParams<T> kp, const __grid_constant__ StepArgs<T> a) {
-    constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A;
+    constexpr int O = Variant<VARIANT>::O;
     __shared__ __align__(16) float tiles[kWarpsPerBlock][32 * O];
 
     if (STATS) credit_env_steps(a.stats, a.n, a.k);
 
-    // COPTER_PREFETCH (A/B knob, persistent grids): the raw vectors of this thread's env in the
-    // NEXT tile are requested before the current tile's arithmetic starts.
-    constexpr bool kPrefetch = COPTER_PREFETCH && sizeof(T) == 4;
-    if constexpr (!COPTER_PERSISTENT && !kPrefetch) {
-        // the shipped shape: the grid holds exactly one CTA per tile (launch_step_v), so there is no
-        // tile loop and no tile count to derive
-        RawEnv<T, A> none;
-        if (COPTER_K1_SPECIALIZE && a.k == 1) step_tile<T, VARIANT, STATS, true, false>(kp, a, none, &tiles[0][0], (int64_t)blockIdx.x);
-        else                                  step_tile<T, VARIANT, STATS, false, false>(kp, a, none, &tiles[0][0], (int64_t)blockIdx.x);
-        return;
-    }
-    const int64_t n_tiles = (a.n + kBlock - 1) / kBlock;
-    RawEnv<T, A> cur, nxt;
-    if (kPrefetch) {
-        const int64_t i0 = (int64_t)blockIdx.x * kBlock + threadIdx.x;
-        if (blockIdx.x < n_tiles && i0 < a.n) load_raw<T, A>(a, i0, cur);
-    }
-    for (int64_t tile_id = blockIdx.x; tile_id < n_tiles; tile_id += gridDim.x) {
-        if (kPrefetch) {
-            const int64_t inext = (tile_id + gridDim.x) * kBlock + threadIdx.x;
-            if (inext < a.n) load_raw<T, A>(a, inext, nxt);
-        }
-        if (COPTER_K1_SPECIALIZE && a.k == 1) step_tile<T, VARIANT, STATS, true, kPrefetch>(kp, a, cur, &tiles[0][0], tile_id);
-        else                                  step_tile<T, VARIANT, STATS, false, kPrefetch>(kp, a, cur, &tiles[0][0], tile_id);
-        if (kPrefetch) cur = nxt;
-    }
+    // the grid holds exactly one CTA per tile (launch_step_v), so there is no tile loop and no tile
+    // count to derive
+    if (a.k == 1) step_tile<T, VARIANT, STATS, true>(kp, a, &tiles[0][0], (int64_t)blockIdx.x);
+    else          step_tile<T, VARIANT, STATS, false>(kp, a, &tiles[0][0], (int64_t)blockIdx.x);
 }
-
-// ------------------------------------------------------------------------------------------
-// K-fused launches on the fp32 path: TWO envs per thread, stepped together by the packed FP32 forms
-// of sm_100 (fma.rn.f32x2 / mul / add: SASS FFMA2, FMUL2, FADD2 -- two independent IEEE operations
-// per issue slot).  Launches with K >= 3 are bound by instruction issue, not by HBM (profiles/
-// r1_step_kernel_k16_*), and ~85 of the ~146 instructions of a straight-line substep are FP32
-// arithmetic: packing two envs halves their issue slots.  A lane holds env (base + lane) in the .x
-// halves and env (base + 32 + lane) in the .y halves of every quantity, so loads and stores stay
-// fully coalesced (a warp covers 64 consecutive envs).
-//   * While every live env of the warp is "calm" the substep is airborne_arith<F2>: the same
-//     airborne_integrate as the scalar kernels, instantiated on the packed lane -- bit-identical.
-//   * Anything else (first step of an episode, ground contact, large angles, an episode ending)
-//     drops to the scalar env_advance for the env concerned, exactly as copter_step_kernel does.
-//   * An env that finishes inside the launch idles afterwards (DESIGN.md section 2).  Its half of the
-//     packed registers keeps being computed on (results unused); its final state waits in a
-//     per-thread shared-memory stash and is stored with everything else, coalesced, at the end.
-// ------------------------------------------------------------------------------------------
-#ifndef COPTER_PAIR_CTAS_PER_SM
-#define COPTER_PAIR_CTAS_PER_SM 4         // x 128 threads x 2 envs = 1024 resident envs per SM at <= 128 registers
-#endif
-
-__device__ __forceinline__ float lane_get(const F2& v, int e) { return e ? v.v.y : v.v.x; }
-__device__ __forceinline__ void lane_set(F2& v, int e, float x) { if (e) v.v.y = x; else v.v.x = x; }
-
-template <int VARIANT, bool STATS>
-__global__ void __launch_bounds__(kBlock, COPTER_PAIR_CTAS_PER_SM)
-copter_step_pair_kernel(const __grid_constant__ KParams<float> kp, const __grid_constant__ StepArgs<float> a) {
-    using T = float;
-    constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A, FIRST = Variant<VARIANT>::first;
-    __shared__ __align__(16) float tiles[kWarpsPerBlock][32 * O];
-    __shared__ float stash[2][12][kBlock];
-    const unsigned full = 0xffffffffu;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (STATS) credit_env_steps(a.stats, a.n, a.k);
-    const int64_t base = (int64_t)blockIdx.x * (2 * kBlock) + warp * 64;     // first env of this warp
-    const bool wide = a.meta_hi != nullptr;
-
-    // Per-env registers are indexed by the half E in {0, 1}; every loop over E is fully unrolled, so E is a
-    // compile-time constant wherever it is used and nothing below lives in local memory.
-    F2 S[12];
-    Forces<T> fe[2];
-    T pert[2][3];
-    int st[2], steps[2], rsteps[2] = {0, 0}, ep_cause[2] = {0, 0}, ep_len[2] = {0, 0};
-    uint32_t episode[2];
-    bool valid[2], live[2], ended[2] = {false, false};
-    T total[2] = {(T)0, (T)0}, ret[2] = {(T)0, (T)0}, ep_ret[2] = {(T)0, (T)0};
-    Shaping<T> start[2];
-
-    RawEnv<T, A> raw[2];
-#pragma unroll
-    for (int E = 0; E < 2; ++E) {
-        const int64_t i = base + 32 * E + lane;
-        valid[E] = i < a.n;
-        if (valid[E]) load_raw<T, A>(a, i, raw[E]);
-    }
-#pragma unroll
-    for (int E = 0; E < 2; ++E) {
-        const int64_t i = base + 32 * E + lane;
-        T se[12], m[4] = {(T)0, (T)0, (T)0, (T)0};
-        st[E] = ST_LANDED; steps[E] = 1; episode[E] = 0;
-        if (valid[E]) {
-            decode_raw<T, VARIANT>(raw[E], wide, se, m, st[E], steps[E], episode[E]);
-            if (STATS && a.ep_return) ret[E] = a.ep_return[i];
-        } else {
-#pragma unroll
-            for (int j = 0; j < 12; ++j) se[j] = (T)0;
-        }
-#pragma unroll
-        for (int j = 0; j < 12; ++j) lane_set(S[j], E, se[j]);
-        fe[E] = motor_forces<T>(kp, m[0], m[1], m[2], m[3]);       // Eq. 6 once per launch (fp64 stage)
-        pert[E][0] = (T)0; pert[E][1] = (T)0; pert[E][2] = (T)0;
-        if (valid[E] && steps[E] == 1) {                            // the reset perturbation of a fresh episode
-            T f[3];
-            if (a.init_force) { f[0] = a.init_force[3 * i]; f[1] = a.init_force[3 * i + 1]; f[2] = a.init_force[3 * i + 2]; }
-            else reset_force<T>(kp, a.seed, (uint64_t)(a.env_offset + i), episode[E], f);
-#pragma unroll
-            for (int j = 0; j < 3; ++j) pert[E][j] = f[j] * kp.invM;
-        }
-        RewardRun<T> r0;
-        run_begin<T, VARIANT>(kp, r0, se);
-        start[E] = r0.start;
-        live[E] = valid[E];
-    }
-    Forces<F2> F;
-    F.bz = F2(fe[0].bz, fe[1].bz); F.u2 = F2(fe[0].u2, fe[1].u2); F.u3 = F2(fe[0].u3, fe[1].u3);
-    F.u4 = F2(fe[0].u4, fe[1].u4); F.jxom = F2(fe[0].jxom, fe[1].jxom); F.jyom = F2(fe[0].jyom, fe[1].jyom);
-
-    F2 RNA(0.0f), RNC(0.0f), NA(0.0f), NC(0.0f), DZP = S[5];
-    for (int k = 0; k < a.k; ++k) {
-        if (__all_sync(full, !(live[0] | live[1]))) break;             // every env of the warp has finished: idle
-        bool hot[2], dn[2] = {false, false};
-        int cause[2] = {0, 0};
-#pragma unroll
-        for (int E = 0; E < 2; ++E)
-            hot[E] = airborne_hot_c<T>(lane_get(S[4], E), lane_get(S[5], E), lane_get(S[6], E), lane_get(S[8], E), lane_get(S[10], E), st[E], steps[E]);
-        const bool fast = __all_sync(full, ((int)!live[0] | (int)hot[0]) & ((int)!live[1] | (int)hot[1]));
-        if (fast) {                                                     // warp-uniform
-            // calm streak (see step_tile): packed straight-line substeps until some live env of the warp
-            // needs the exact tests again
-            bool calm[2] = {true, true}, tmo[2] = {false, false};
-            int streak = 0;
-            F2 PNA, PNC;
-            do {
-                DZP = S[5];
-                tmo[0] = steps[0] == kp.max_steps; tmo[1] = steps[1] == kp.max_steps;
-                airborne_arith<F2, T>(kp, S, F, NA, NC);
-                steps[0] += (int)live[0]; steps[1] += (int)live[1];
-#pragma unroll
-                for (int E = 0; E < 2; ++E)
-                    calm[E] = (int)!live[E] | (int)airborne_calm<T>(kp, lane_get(S[0], E), lane_get(S[2], E), lane_get(S[4], E), lane_get(S[5], E),
-                                                                    lane_get(S[6], E), lane_get(S[8], E), lane_get(S[10], E), tmo[E]);
-                PNA = RNA; PNC = RNC;                                   // an over-angle ending takes its own numerators back
-                RNA = RNA + NA; RNC = RNC + NC;
-                ++streak; ++k;
-            } while (k < a.k && __all_sync(full, (int)calm[0] & (int)calm[1]));
-            --k;                                                        // the for statement counts the last one
-#pragma unroll
-            for (int E = 0; E < 2; ++E) {
-                if (live[E]) {
-                    rsteps[E] += streak;
-                    steps[E] = min(steps[E], kp.steps_cap);
-                    int end = 0;
-                    if (!calm[E]) {                                     // back to the exact tests for this env's last step
-                        end = airborne_flags<T, VARIANT>(kp, lane_get(S[0], E), lane_get(S[2], E), lane_get(S[6], E), lane_get(S[8], E), tmo[E]);
-                        if (end & END_ANGLE) { lane_set(RNA, E, lane_get(PNA, E)); lane_set(RNC, E, lane_get(PNC, E)); }
-                    }
-                    dn[E] = end != 0;
-                    if (dn[E]) cause[E] = airborne_cause(end);
-                }
-            }
-        } else {
-#pragma unroll
-            for (int E = 0; E < 2; ++E) {
-                if (live[E]) {
-                    T se[12], na, nc;
-#pragma unroll
-                    for (int j = 0; j < 12; ++j) se[j] = lane_get(S[j], E);
-                    lane_set(DZP, E, se[5]);
-                    env_advance<T, VARIANT>(kp, se, st[E], steps[E], fe[E], pert[E], na, nc, dn[E], cause[E]);
-                    pert[E][0] = (T)0; pert[E][1] = (T)0; pert[E][2] = (T)0;
-#pragma unroll
-                    for (int j = 0; j < 12; ++j) lane_set(S[j], E, se[j]);
-                    lane_set(NA, E, na); lane_set(NC, E, nc);
-                    ++rsteps[E];
-                    if (!(cause[E] & CAUSE_ANGLE)) { lane_set(RNA, E, lane_get(RNA, E) + na); lane_set(RNC, E, lane_get(RNC, E) + nc); }
-                }
-            }
-        }
-#pragma unroll
-        for (int E = 0; E < 2; ++E) {
-            if (dn[E]) {                                                // only a live env can have ended
-                T se[12];
-#pragma unroll
-                for (int j = 0; j < 12; ++j) se[j] = lane_get(S[j], E);
-                live[E] = false; ended[E] = true; ep_cause[E] = cause[E];
-                RewardRun<T> run;
-                run.start = start[E]; run.na = lane_get(RNA, E); run.nc = lane_get(RNC, E); run.steps = rsteps[E];
-                total[E] = run_reward<T, VARIANT>(kp, run, se, cause[E], lane_get(NA, E), lane_get(NC, E), lane_get(DZP, E));
-                if (STATS) ep_len[E] = steps[E] - 1;                    // `steps` is 1 right after reset (task.py:191,197)
-                if (a.final_obs) {   // terminal observation; rows of unfinished envs stay untouched
-                    const int64_t i = base + 32 * E + lane;
-#pragma unroll
-                    for (int j = 0; j < O; ++j) a.final_obs[i * O + j] = (float)se[FIRST + j];
-                }
-                if (a.auto_reset) {
-                    reset_state<T>(kp, se, st[E], steps[E]);
-                    episode[E] = (episode[E] + 1) & kp.ep_mask;
-                }
-#pragma unroll
-                for (int j = 0; j < 12; ++j) stash[E][j][threadIdx.x] = se[j];
-            }
-        }
-    }
-
-#pragma unroll
-    for (int E = 0; E < 2; ++E) {
-        const int64_t row0 = base + 32 * E, i = row0 + lane;
-        const int64_t left = a.n - row0;
-        const int rows = left >= 32 ? 32 : (left > 0 ? (int)left : 0);
-        T se[12];
-#pragma unroll
-        for (int j = 0; j < 12; ++j) se[j] = ended[E] ? stash[E][j][threadIdx.x] : lane_get(S[j], E);
-        if (valid[E]) {
-            if (!ended[E]) {
-                RewardRun<T> run;
-                run.start = start[E]; run.na = lane_get(RNA, E); run.nc = lane_get(RNC, E); run.steps = rsteps[E];
-                total[E] = run_reward<T, VARIANT>(kp, run, se, 0, lane_get(NA, E), lane_get(NC, E), lane_get(DZP, E));
-            }
-            if (STATS) {
-                ret[E] += total[E];
-                if (ended[E]) { ep_ret[E] = ret[E]; ret[E] = (T)0; }
-            }
-            store_state<T>(a.state, a.stride, i, se);
-            store_meta(a.meta, a.meta_hi, i, st[E], steps[E], episode[E]);
-            a.reward[i] = total[E];
-            a.done[i] = ended[E] ? 1 : 0;
-            if (a.cause) a.cause[i] = (uint8_t)ep_cause[E];
-            if (STATS && a.ep_return) a.ep_return[i] = ret[E];
-        }
-        if (a.obs) write_obs_rows<VARIANT, T>(a.obs, tiles[warp], lane, row0, rows, se);
-        if (STATS) flush_episode_stats<T>(a.stats, lane, ended[E], ep_cause[E], ep_len[E], ep_ret[E], a.ep_return != nullptr);
-    }
-    if (STATS) debit_idle_steps(a.stats, lane, (valid[0] ? a.k - rsteps[0] : 0) + (valid[1] ? a.k - rsteps[1] : 0));
-}
-
-// ------------------------------------------------------------------------------------------
-// A/B shape (compiled in with -DCOPTER_TMA_MIN_K=1|2, off by default): persistent CTAs that fetch
-// their NEXT tile's inputs with the TMA engine (cp.async.bulk 1-D: three 2 KB state planes, the
-// action rows and the meta words of 128 envs per stage, two stages, one full/empty mbarrier pair
-// per stage) while their warps compute the current tile, and that get their tiles from cluster
-// launch control: the grid still holds one CTA per tile, a running CTA cancels a not-yet-launched
-// CTA and takes over its block index (hardware work stealing, no counter in memory).
-// Measured on B200 (Lander3D fp32, 2^24 envs; profiles/r1_sweep_tma_clc.txt):
-//   * static grid-stride tiles lose 17 % at K = 1 (0.486 vs 0.414 ms) however the loads are issued
-//     (plain, register-prefetched or TMA-prefetched; staggering the CTAs' start changes nothing):
-//     SMs do not all see the same memory bandwidth, and a static split waits for the slowest;
-//   * with cluster launch control the persistent kernel is level with the one-tile-per-CTA kernel
-//     at K = 1 (0.4140 vs 0.4134 ms) -- the hardware CTA scheduler was doing that balancing;
-//   * the prefetch itself buys nothing at any K (K = 4: 0.604 vs 0.584 ms, K = 16: 1.627 vs 1.614):
-//     launches with K >= 3 are bound by instruction issue (t = 0.24 ms + K x 0.086 ms), not by
-//     exposed load latency, and K <= 2 by HBM.
-// So the shipped step kernel stays the simple one; this one documents the alternative.
-// ------------------------------------------------------------------------------------------
-#ifndef COPTER_TMA_MIN_K
-#define COPTER_TMA_MIN_K 0        // k_substeps >= this use copter_step_tma_kernel (0: never)
-#endif
-#ifndef COPTER_TMA_CTAS_PER_SM
-#define COPTER_TMA_CTAS_PER_SM COPTER_F32_CTAS_PER_SM     // fp32 occupancy target of that kernel (A/B knob)
-#endif
-
-#if COPTER_TMA_MIN_K > 0
-template <typename T, int A> struct alignas(128) TileStage {     // one tile (kBlock envs) of inputs, laid out as in HBM
-    typename Vec<T>::type plane[12 / Vec<T>::V][kBlock];
-    T act[kBlock * A];
-    uint32_t meta[kBlock];
-};
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\t"
-                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                 "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" :: "r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* dst_smem, const void* src_global, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_u32(dst_smem)), "l"(src_global), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
-// Cluster launch control (sm_100): a running CTA cancels a CTA of the grid that has not been launched
-// yet and takes over its block index -- dynamic tile scheduling done by the hardware, no counter in
-// memory.  The 16-byte response lands in shared memory through an mbarrier like a TMA copy.  (One definition,
-// shared with the tcgen05 policy kernels: copter_policy_tc.cuh.)
-using tc::clc_try_cancel;       // arrive.expect_tx(16) on the barrier + clusterlaunchcontrol.try_cancel into resp16
-using tc::clc_response;         // the cancelled CTA's blockIdx.x, or 0xFFFFFFFF when nothing was left to cancel
-
-#ifndef COPTER_TMA_CLC
-#define COPTER_TMA_CLC 1          // 1: one CTA per tile in the grid, running CTAs steal the pending ones (cluster launch
-#endif                            //    control); 0 (A/B knob): one resident wave, tiles assigned by a grid stride
-
-template <typename T, int VARIANT, bool STATS, bool SINGLE>
-__global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? COPTER_TMA_CTAS_PER_SM : 2)
-copter_step_tma_kernel(const __grid_constant__ KParams<T> kp, const __grid_constant__ StepArgs<T> a) {
-    constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A, V = Vec<T>::V, NP = 12 / V;
-    using V4 = typename Vec<T>::type;
-    __shared__ __align__(16) float tiles[kWarpsPerBlock][32 * O];
-    __shared__ TileStage<T, A> stage[2];
-    __shared__ __align__(16) uint4 clc_resp;
-    __shared__ __align__(8) uint64_t full[2], empty[2], clc_bar;
-    __shared__ uint32_t sh_next[2];
-    const int lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        mbar_init(&full[0], 1); mbar_init(&full[1], 1);                       // the producer's expect_tx arrival
-        mbar_init(&empty[0], kWarpsPerBlock); mbar_init(&empty[1], kWarpsPerBlock);   // one arrival per consumer warp
-        mbar_init(&clc_bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");    // visible to the async proxy
-    }
-    __syncthreads();
-    if (STATS) credit_env_steps(a.stats, a.n, a.k);
-
-    constexpr uint32_t kPlaneBytes = kBlock * sizeof(V4), kActBytes = kBlock * A * sizeof(T), kMetaBytes = kBlock * 4;
-    // thread 0: arm the stage's barrier with the tile's byte count and hand the copies to the TMA engine
-    auto fetch = [&](uint32_t tile, int st) {
-        TileStage<T, A>& dst = stage[st];
-        const int64_t row0 = (int64_t)tile * kBlock;
-        const V4* planes = reinterpret_cast<const V4*>(a.state);
-        mbar_expect_tx(&full[st], NP * kPlaneBytes + kActBytes + kMetaBytes);
-#pragma unroll
-        for (int pl = 0; pl < NP; ++pl) bulk_load(dst.plane[pl], planes + (int64_t)pl * a.stride + row0, kPlaneBytes, &full[st]);
-        bulk_load(dst.act, a.action + row0 * A, kActBytes, &full[st]);
-        bulk_load(dst.meta, a.meta + row0, kMetaBytes, &full[st]);
-    };
-    // Tiles below n_full are complete and go through the staging; a ragged last tile takes direct loads.
-    // Loop state is one word.  All threads: bit 0 = stage, bits 1-2 = next phase of full[0..1].
-    // Thread 0 only: bits 3-4 = next phase of empty[0..1], bits 5-6 = stage 0/1 has been filled before,
-    // bit 7 = a try_cancel is in flight, bit 8 = next phase of clc_bar.
-    constexpr uint32_t kNone = 0xFFFFFFFFu;
-    const uint32_t n_tiles = (uint32_t)((a.n + kBlock - 1) / kBlock), n_full = (uint32_t)(a.n / kBlock);
-    uint32_t tile = blockIdx.x, ring = 0;
-    if (tile >= n_tiles) return;
-    if (threadIdx.x == 0) {
-        if (tile < n_full) { fetch(tile, 0); ring |= 1u << 5; }
-        if (COPTER_TMA_CLC) { clc_try_cancel(&clc_resp, &clc_bar); ring |= 1u << 7; }
-    }
-    for (;; ring ^= 1u) {
-        const int st = ring & 1u;
-        if (threadIdx.x == 0) {
-            uint32_t nxt = kNone;
-            if (COPTER_TMA_CLC) {
-                if (ring & (1u << 7)) {
-                    mbar_wait(&clc_bar, (ring >> 8) & 1u);
-                    ring ^= 1u << 8;
-                    nxt = clc_response(&clc_resp);
-                    if (nxt != kNone) {
-                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // response read before the buffer is rewritten
-                        clc_try_cancel(&clc_resp, &clc_bar);
-                    } else {
-                        ring &= ~(1u << 7);                         // a failed try_cancel is the last one
-                    }
-                }
-            } else if (tile + gridDim.x < n_tiles) {
-                nxt = tile + gridDim.x;
-            }
-            if (nxt < n_full) {
-                const int o = st ^ 1;
-                if (ring & (1u << (5 + o))) {                       // filled before: wait until all four warps have read it
-                    mbar_wait(&empty[o], (ring >> (3 + o)) & 1u);
-                    ring ^= 8u << o;
-                }
-                fetch(nxt, o);
-                ring |= 1u << (5 + o);
-            }
-            sh_next[st] = nxt;
-        }
-        __syncthreads();
-        const uint32_t nxt = sh_next[st];
-        RawEnv<T, A> cur;
-        const int64_t row0 = (int64_t)tile * kBlock + (threadIdx.x >> 5) * 32;
-        if (tile < n_full) {                                        // CTA-uniform
-            mbar_wait(&full[st], (ring >> (1 + st)) & 1u);
-            ring ^= 2u << st;
-            const TileStage<T, A>& src = stage[st];
-#pragma unroll
-            for (int pl = 0; pl < NP; ++pl) cur.plane[pl] = src.plane[pl][threadIdx.x];
-#pragma unroll
-            for (int j = 0; j < A; ++j) cur.act[j] = src.act[threadIdx.x * A + j];
-            cur.meta = src.meta[threadIdx.x];
-            cur.meta_hi = a.meta_hi ? a.meta_hi[(int64_t)tile * kBlock + threadIdx.x] : 0u;
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty[st]);
-        } else if (row0 + lane < a.n) {
-            load_raw<T, A>(a, row0 + lane, cur);
-        }
-        step_tile<T, VARIANT, STATS, SINGLE, true>(kp, a, cur, &tiles[0][0], (int64_t)tile);
-        if (nxt == kNone) break;
-        tile = nxt;
-    }
-}
-
-#endif  // COPTER_TMA_MIN_K > 0
 
 // ------------------------------------------------------------------------------------------
 // Multi-step rollout with on-device action sources: n_steps reference steps per launch, the
@@ -1536,17 +1093,16 @@ int ctas_per_sm(int block) {
 // B200 (Lander3D fp32, 2^24 envs, K = 1): 6.7 TB/s, against 5.6 TB/s for a persistent grid of
 // SMs x resident CTAs walking the tiles with a grid stride.  The loss is the static split (the SMs
 // do not all see the same memory bandwidth; a persistent grid fed by cluster launch control is
-// level with this shape -- see copter_step_tma_kernel), so the hardware scheduler does the balancing.
-// (COPTER_PERSISTENT=1 / COPTER_PREFETCH=1 keep the old shape for A/B runs; profiles/README.md has
-// the sweep.)  The kernels keep their tile loop, so a grid capped at 2^31-1 CTAs still covers any n.
-template <auto Kernel>
+// level with this shape -- DESIGN.md, "Grid shape"), so the hardware scheduler does the balancing.
+// (profiles/README.md has the sweep.)  The other kernels keep their tile loop, so a grid capped at
+// 2^31-1 CTAs still covers any n.
 int grid_for(int64_t n) {
     const int64_t tiles = (n + kBlock - 1) / kBlock;
-    const int64_t cap = COPTER_PERSISTENT ? (int64_t)sm_count() * ctas_per_sm<Kernel>(kBlock) : (int64_t)0x7fffffff;
+    const int64_t cap = (int64_t)0x7fffffff;
     return (int)(tiles < cap ? (tiles > 0 ? tiles : 1) : cap);
 }
-// the step kernel's shipped shape has no tile loop: every tile needs its own CTA
-constexpr int64_t kMaxEnvsPerLaunch = COPTER_PERSISTENT ? INT64_MAX : (int64_t)0x7fffffff * kBlock;
+// the step kernel has no tile loop: every tile needs its own CTA
+constexpr int64_t kMaxEnvsPerLaunch = (int64_t)0x7fffffff * kBlock;
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -1557,60 +1113,10 @@ int check_params(const CopterParams* p, bool wide = false) {
     return 0;
 }
 
-// resident-wave grid for the persistent-warp kernels
-template <auto Kernel>
-int resident_grid_for(int64_t n) {
-    const int64_t tiles = (n + kBlock - 1) / kBlock, cap = (int64_t)sm_count() * ctas_per_sm<Kernel>(kBlock);
-    return (int)(tiles < cap ? (tiles > 0 ? tiles : 1) : cap);
-}
-
-// k_substeps threshold of the packed two-env kernel: the build default, or COPTER_B200_PAIR_MIN_K from the environment
-int pair_min_k_setting() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("COPTER_B200_PAIR_MIN_K");
-        v = e ? atoi(e) : COPTER_PAIR_MIN_K;
-        if (v < 0) v = 0;
-    }
-    return v;
-}
-
 template <typename T, int VARIANT>
 int launch_step_v(const KParams<T>& kp, const StepArgs<T>& a, cudaStream_t s) {
-    // K-fused launches: TMA-prefetched inputs (every bulk copy needs 16-byte aligned sources; the
-    // state planes and the action rows are checked by the caller, the meta words here)
-#if COPTER_TMA_MIN_K > 0
-    if (a.k >= COPTER_TMA_MIN_K && aligned16(a.meta) && a.n <= (int64_t)0x7fffffff * kBlock) {
-        constexpr bool kSingle = COPTER_TMA_MIN_K == 1 && COPTER_K1_SPECIALIZE;      // only an A/B build sends K = 1 here
-        // cluster launch control: the grid holds one CTA per tile and the resident CTAs steal the rest
-        const int64_t n_tiles = (a.n + kBlock - 1) / kBlock;
-#define COPTER_TMA_GRID(K) (COPTER_TMA_CLC ? (int)n_tiles : resident_grid_for<K>(a.n))
-        if (kSingle && a.k == 1) {
-            if (a.stats) copter_step_tma_kernel<T, VARIANT, true, kSingle><<<COPTER_TMA_GRID((copter_step_tma_kernel<T, VARIANT, true, kSingle>)), kBlock, 0, s>>>(kp, a);
-            else         copter_step_tma_kernel<T, VARIANT, false, kSingle><<<COPTER_TMA_GRID((copter_step_tma_kernel<T, VARIANT, false, kSingle>)), kBlock, 0, s>>>(kp, a);
-        } else {
-            if (a.stats) copter_step_tma_kernel<T, VARIANT, true, false><<<COPTER_TMA_GRID((copter_step_tma_kernel<T, VARIANT, true, false>)), kBlock, 0, s>>>(kp, a);
-            else         copter_step_tma_kernel<T, VARIANT, false, false><<<COPTER_TMA_GRID((copter_step_tma_kernel<T, VARIANT, false, false>)), kBlock, 0, s>>>(kp, a);
-        }
-#undef COPTER_TMA_GRID
-        return (int)cudaGetLastError();
-    }
-#endif
-    // K-fused fp32 launches can take the two-envs-per-thread kernel on packed fma.rn.f32x2
-    // (copter_step_pair_kernel).  Measured, it loses to the one-env-per-thread loop (profiles/README.md:
-    // the loop is bound by register-file operand bandwidth, which FFMA2 does not relieve), so it is off by
-    // default and kept as a run-time A/B: COPTER_B200_PAIR_MIN_K=<k> in the environment sends k_substeps >= k to it.
-    if constexpr (sizeof(T) == 4) {
-        const int pair_min_k = pair_min_k_setting();
-        if (pair_min_k > 0 && a.k >= pair_min_k) {
-            const int grid = (int)((a.n + 2 * kBlock - 1) / (2 * kBlock));
-            if (a.stats) copter_step_pair_kernel<VARIANT, true><<<grid, kBlock, 0, s>>>(kp, a);
-            else         copter_step_pair_kernel<VARIANT, false><<<grid, kBlock, 0, s>>>(kp, a);
-            return (int)cudaGetLastError();
-        }
-    }
-    if (a.stats) copter_step_kernel<T, VARIANT, true><<<grid_for<copter_step_kernel<T, VARIANT, true>>(a.n), kBlock, 0, s>>>(kp, a);
-    else         copter_step_kernel<T, VARIANT, false><<<grid_for<copter_step_kernel<T, VARIANT, false>>(a.n), kBlock, 0, s>>>(kp, a);
+    if (a.stats) copter_step_kernel<T, VARIANT, true><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
+    else         copter_step_kernel<T, VARIANT, false><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
     return (int)cudaGetLastError();
 }
 
@@ -1646,18 +1152,18 @@ int launch_step(const CopterParams* p, const CopterBuffers* b, int64_t n, int64_
 template <typename T, int VARIANT, bool R>
 int launch_rollout_vr(const KParams<T>& kp, const RolloutArgs<T>& a, cudaStream_t s) {
     if (a.src_kind == COPTER_SRC_PID) {
-        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 1, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 1, R>>(a.n), kBlock, 0, s>>>(kp, a);
-        else         copter_rollout_kernel<T, VARIANT, false, 1, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 1, R>>(a.n), kBlock, 0, s>>>(kp, a);
+        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 1, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
+        else         copter_rollout_kernel<T, VARIANT, false, 1, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
     } else if (a.src_kind == COPTER_SRC_PID_HOVER) {
         if constexpr (Variant<VARIANT>::A == 4 && Variant<VARIANT>::O != 12) {
             return COPTER_E_VARIANT;          // the 3-D hover heuristic reads the yaw rate: full-state observation only
         } else {
-            if (a.stats) copter_rollout_kernel<T, VARIANT, true, 2, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 2, R>>(a.n), kBlock, 0, s>>>(kp, a);
-            else         copter_rollout_kernel<T, VARIANT, false, 2, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 2, R>>(a.n), kBlock, 0, s>>>(kp, a);
+            if (a.stats) copter_rollout_kernel<T, VARIANT, true, 2, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
+            else         copter_rollout_kernel<T, VARIANT, false, 2, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
         }
     } else {
-        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 0, R><<<grid_for<copter_rollout_kernel<T, VARIANT, true, 0, R>>(a.n), kBlock, 0, s>>>(kp, a);
-        else         copter_rollout_kernel<T, VARIANT, false, 0, R><<<grid_for<copter_rollout_kernel<T, VARIANT, false, 0, R>>(a.n), kBlock, 0, s>>>(kp, a);
+        if (a.stats) copter_rollout_kernel<T, VARIANT, true, 0, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
+        else         copter_rollout_kernel<T, VARIANT, false, 0, R><<<grid_for(a.n), kBlock, 0, s>>>(kp, a);
     }
     return (int)cudaGetLastError();
 }
@@ -1712,7 +1218,7 @@ int launch_rollout(const CopterParams* p, const CopterBuffers* b, const CopterAc
 
 template <typename T, int VARIANT>
 int launch_reset_v(const KParams<T>& kp, const CopterBuffers* b, int64_t n, int keep_episode, cudaStream_t s) {
-    copter_reset_kernel<T, VARIANT><<<grid_for<copter_reset_kernel<T, VARIANT>>(n), kBlock, 0, s>>>(kp, (T*)b->state, b->meta, b->meta_hi, b->obs, (T*)b->ep_return, n, b->state_stride > 0 ? b->state_stride : n, keep_episode);
+    copter_reset_kernel<T, VARIANT><<<grid_for(n), kBlock, 0, s>>>(kp, (T*)b->state, b->meta, b->meta_hi, b->obs, (T*)b->ep_return, n, b->state_stride > 0 ? b->state_stride : n, keep_episode);
     return (int)cudaGetLastError();
 }
 
@@ -1750,7 +1256,7 @@ int launch_dynamics(const CopterParams* p, void* state, uint8_t* status, int32_t
     if (!aligned16(state)) return COPTER_E_ALIGN;
     if (n == 0) return 0;
     const KParams<T> kp = make_kparams<T>(*p);
-    copter_dynamics_kernel<T><<<grid_for<copter_dynamics_kernel<T>>(n), kBlock, 0, (cudaStream_t)stream>>>(kp, (T*)state, status, ticks, (T*)perturb, (const T*)motors, n);
+    copter_dynamics_kernel<T><<<grid_for(n), kBlock, 0, (cudaStream_t)stream>>>(kp, (T*)state, status, ticks, (T*)perturb, (const T*)motors, n);
     return (int)cudaGetLastError();
 }
 
@@ -1763,7 +1269,7 @@ int launch_reset_force(const CopterParams* p, T* out, const uint32_t* episode, i
     if (n < 0 || env_offset < 0) return COPTER_E_RANGE;
     if (n == 0) return 0;
     const KParams<T> kp = make_kparams<T>(*p);
-    copter_reset_force_kernel<T><<<grid_for<copter_reset_force_kernel<T>>(n), kBlock, 0, (cudaStream_t)stream>>>(kp, out, episode, n, env_offset, seed);
+    copter_reset_force_kernel<T><<<grid_for(n), kBlock, 0, (cudaStream_t)stream>>>(kp, out, episode, n, env_offset, seed);
     return (int)cudaGetLastError();
 }
 

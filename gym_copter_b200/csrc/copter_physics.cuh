@@ -1,6 +1,6 @@
-// copter_physics.cuh -- device-side glue around the shared arithmetic (copter_core.h): build knobs,
-// vector-plane state access, the packed two-env lane type (fma.rn.f32x2), the straight-line /
-// calm-streak substep pieces of the K-fused loops, and the observation staging.
+// copter_physics.cuh -- device-side glue around the shared arithmetic (copter_core.h): launch-shape
+// constants, vector-plane state access, the straight-line / calm-streak substep pieces of the
+// K-fused loop, and the observation staging.
 // Included by copter_kernels.cu (kernels, launchers, C ABI).
 //
 // The arithmetic itself -- Eq. 6 / Eq. 12 dynamics with the flight-status machine, the lander
@@ -32,51 +32,6 @@ namespace copter {
 #ifndef COPTER_BLOCK
 #define COPTER_BLOCK 128
 #endif
-#ifndef COPTER_PREFETCH
-#define COPTER_PREFETCH 0       // (A/B knob, persistent grids only) request the NEXT tile's loads before this tile's arithmetic
-#endif
-#ifndef COPTER_PERSISTENT
-#define COPTER_PERSISTENT 0     // 1 (A/B knob): one resident wave of CTAs walking the tiles with a grid stride
-#endif
-#ifndef COPTER_K1_SPECIALIZE
-#define COPTER_K1_SPECIALIZE 1   // dedicated code path for k_substeps == 1 (the HBM-bound case)
-#endif
-#ifndef COPTER_K_UNROLL
-#define COPTER_K_UNROLL 1         // unroll factor of the substep loop (A/B knob)
-#endif
-#ifndef COPTER_FAST_SUBSTEP
-#define COPTER_FAST_SUBSTEP 1     // 0 (A/B knob): every substep of a K-fused launch takes the general env_advance
-#endif
-#ifndef COPTER_FRESH_FAST
-#define COPTER_FRESH_FAST 0      // 1 (A/B knob): a warp with a fresh episode in it takes a straight-line step WITH the reset perturbation
-                                 // at substep 0 instead of the general step.  Measured slower (K = 16: 1.484 vs 1.443 ms): off.
-#endif
-#ifndef COPTER_GROUND_SPLIT
-#define COPTER_GROUND_SPLIT 0    // 1 (A/B knob): while a lane on the ground is all that keeps a warp from the straight-line step, the airborne
-                                 // lanes take it and that lane runs the status machine beside them.  Measured slower (K = 16: 1.511 vs
-                                 // 1.444 ms, profiles/r2_ab_k_loop.txt): the general step is only ~35 % dearer than the straight-line one,
-                                 // two divergent passes cost more.  Off.
-#endif
-#ifndef COPTER_GROUND_FF
-#define COPTER_GROUND_FF 0       // 1 (A/B knob): a lane that has reached the ground takes its remaining status-machine steps at once, alone, and
-                                 // leaves the loop, instead of one per substep with the whole warp in the general step (5.7 of the 16
-                                 // substeps of a K = 16 launch on a desynchronised batch).  Bit-identical, measured SLOWER (K = 16: 1.533 vs
-                                 // 1.391 ms, K = 2: 0.485 vs 0.453, profiles/r2_ab_k_loop2.txt): a lone lane's env_advance costs the
-                                 // warp almost what a general step of all 32 lanes does.  2: the same with the status machine written
-                                 // out for a grounded vehicle (ground_advance, ~25 instructions per step): 1.462 vs 1.392 ms, K = 2 0.479
-                                 // vs 0.466 (profiles/r2_ab_k_loop4.txt) -- still slower, and already at K = 2 where hardly any vehicle
-                                 // lands: the extra block costs the loop more than the general steps it saves.  Off.
-#endif
-#ifndef COPTER_CALM_STREAK
-#define COPTER_CALM_STREAK 1     // 0 (A/B knob): every straight-line substep re-derives the ending flags and the hot test
-#endif
-#ifndef COPTER_STREAMING
-#define COPTER_STREAMING 0      // 1: evict-first (ld/st .cs) hints on the state planes
-#endif
-#ifndef COPTER_PAIR_MIN_K
-#define COPTER_PAIR_MIN_K 0     // k_substeps >= this (fp32) use the two-envs-per-thread packed kernel (0: never; run-time override:
-                                // COPTER_B200_PAIR_MIN_K in the environment).  Measured slower than the scalar loop: off.
-#endif
 
 constexpr int kBlock = COPTER_BLOCK;
 constexpr int kWarpsPerBlock = kBlock / 32;
@@ -95,7 +50,7 @@ __device__ __forceinline__ void load_state(const T* __restrict__ state, int64_t 
     const V4* planes = reinterpret_cast<const V4*>(state);
 #pragma unroll
     for (int pl = 0; pl < 12 / V; ++pl) {
-        V4 v = COPTER_STREAMING ? __ldcs(&planes[(int64_t)pl * stride + i]) : planes[(int64_t)pl * stride + i];
+        V4 v = planes[(int64_t)pl * stride + i];
         const T* e = reinterpret_cast<const T*>(&v);
 #pragma unroll
         for (int j = 0; j < V; ++j) s[pl * V + j] = e[j];
@@ -113,7 +68,7 @@ __device__ __forceinline__ void store_state(T* __restrict__ state, int64_t strid
         T* e = reinterpret_cast<T*>(&v);
 #pragma unroll
         for (int j = 0; j < V; ++j) e[j] = s[pl * V + j];
-        if (COPTER_STREAMING) __stcs(&planes[(int64_t)pl * stride + i], v); else planes[(int64_t)pl * stride + i] = v;
+        planes[(int64_t)pl * stride + i] = v;
     }
 }
 
@@ -129,127 +84,31 @@ __device__ __forceinline__ void store_meta(uint32_t* meta, uint32_t* hi, int64_t
 }
 
 // ------------------------------------------------------------------------------------------
-// F2: a lane of TWO envs, one packed 64-bit register pair per quantity, every operation one FFMA2
-// (fma.rn.f32x2: two independent round-to-nearest IEEE operations in one issue slot), so
-// airborne_integrate<F2> produces exactly the bits of two airborne_integrate<float>.
-// Measured on B200 (tools/microbench/ffma2_rates.cu, profiles/r2_ffma2_rates.txt): FFMA2 issues every
-// 2 cycles per scheduler -- the element rate of scalar FFMA in half the issue slots -- while the packed
-// multiply and add (FMUL2 / FADD2) issue only every ~6.6 cycles.  Products and sums are therefore
-// written as fused operations that are EXACTLY the plain ones: a*b = fma(a, b, -0) (adding -0 changes
-// no value, not even the sign of a zero product) and a+b = fma(a, 1, b).
-// ------------------------------------------------------------------------------------------
-#ifndef COPTER_F2_PLAIN_MUL_ADD
-#define COPTER_F2_PLAIN_MUL_ADD 0     // 1 (A/B knob): FMUL2 / FADD2 for the packed products and sums
-#endif
-// -0 and 1 as the compiler cannot see them (constant memory can be rewritten by the host, so neither
-// nvcc nor ptxas may fold them): with literal constants ptxas turns fma(a, b, -0) straight back into FMUL2
-__constant__ float kF2NegZero = -0.0f;
-__constant__ float kF2One = 1.0f;
-struct F2 {
-    float2 v;
-    __device__ __forceinline__ F2() {}
-    __device__ __forceinline__ explicit F2(float x) { v.x = x; v.y = x; }
-    __device__ __forceinline__ F2(float x, float y) { v.x = x; v.y = y; }
-};
-__device__ __forceinline__ F2 fma_(F2 a, F2 b, F2 c) {
-    // inline PTX rather than __ffma2_rn: the compiler must not "simplify" the exact forms below back into mul / add
-    F2 r;
-    asm("{\n\t.reg .b64 a, b, c, d;\n\t"
-        "mov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tmov.b64 c, {%6, %7};\n\t"
-        "fma.rn.f32x2 d, a, b, c;\n\t"
-        "mov.b64 {%0, %1}, d;\n\t}"
-        : "=f"(r.v.x), "=f"(r.v.y) : "f"(a.v.x), "f"(a.v.y), "f"(b.v.x), "f"(b.v.y), "f"(c.v.x), "f"(c.v.y));
-    return r;
-}
-__device__ __forceinline__ F2 operator*(F2 a, F2 b) {
-    if (COPTER_F2_PLAIN_MUL_ADD) { F2 r; r.v = __fmul2_rn(a.v, b.v); return r; }
-    return fma_(a, b, F2(kF2NegZero));
-}
-__device__ __forceinline__ F2 operator+(F2 a, F2 b) {
-    if (COPTER_F2_PLAIN_MUL_ADD) { F2 r; r.v = __fadd2_rn(a.v, b.v); return r; }
-    return fma_(a, F2(kF2One), b);
-}
-__device__ __forceinline__ F2 operator-(F2 a) { return F2(-a.v.x, -a.v.y); }
-
-// ------------------------------------------------------------------------------------------
-// The common case of env_advance as straight-line code, for the K-fused loops: an AIRBORNE env that
+// The common case of env_advance as straight-line code, for the K-fused loop: an AIRBORNE env that
 // is not touching the ground, is past the first step of its episode (no reset perturbation left)
 // and -- fp32 -- has all three angles inside the polynomial range of sincos_poly.  airborne_hot()
 // is that precondition; under it airborne_arith() + airborne_flags() give exactly what env_advance gives.
 // ------------------------------------------------------------------------------------------
 template <typename T>
-__device__ __forceinline__ bool airborne_hot_c(T z, T dz, T phi, T the, T psi, int st, int steps) {
+__device__ __forceinline__ bool airborne_hot(const T (&s)[12], int st, int steps) {
+    const T z = s[4], dz = s[5], phi = s[6], the = s[8], psi = s[10];
     // (bitwise on purpose: one straight run of compares, no short-circuit branches)
     int hot = (int)(st == ST_AIRBORNE) & (int)(steps != 1) & (int)!(z > (T)0 && dz > (T)0);
     if constexpr (sizeof(T) == 4) hot &= (int)(fmaxf(fmaxf(fabsf(phi), fabsf(the)), fabsf(psi)) <= 0.78539816f);
     return hot != 0;
 }
-template <typename T>
-__device__ __forceinline__ bool airborne_hot(const T (&s)[12], int st, int steps) {
-    return airborne_hot_c<T>(s[4], s[5], s[6], s[8], s[10], st, steps);
-}
-// A vehicle the airborne arithmetic does not apply to (on the ground, touching it, levelling, crashed): its step is
-// the status machine alone -- env_advance without sines, cosines or integration (dynamics_update skips them).
-template <typename T>
-__device__ __forceinline__ bool on_ground(const T (&s)[12], int st) {
-    return st != ST_AIRBORNE || (s[4] > (T)0 && s[5] > (T)0);
-}
-// env_advance for such a vehicle, written out: dynamics_update (dynamics/__init__.py:147-177) is then the status
-// machine alone and _Task.step's tests (task.py:111-130, lander.py:64-72) follow unchanged.  Not for the `direct`
-// variants (a LANDED vehicle can take off there).  COPTER_GROUND_FF = 2 steps a grounded lane with this instead of
-// the general env_advance.
-template <typename T, int VARIANT>
-__device__ __forceinline__ void ground_advance(const KParams<T>& kp, T (&s)[12], int& st, int& steps, bool& done, int& cause) {
-    using V = Variant<VARIANT>;
-    const int st0 = st;                                            // task.py:81 stale status
-    if (st0 == ST_LEVELING) { s[6] = (T)0; s[8] = (T)0; st = ST_LANDED; }                                  // :152-156
-    else if (st0 == ST_AIRBORNE)                                   // touching the ground: :162-177 (early return, nothing moves)
-        st = (s[5] > kp.lvy || abs_t(s[3]) > kp.lvx || abs_t(s[6]) > kp.lang) ? ST_CRASHED : ST_LEVELING;
-    cause = 0;
-    done = false;
-    if (V::lander && st0 == ST_LANDED) {                           // lander.py:64-72
-        done = true; cause |= CAUSE_LANDED;
-        if (sqrt_t(s[0] * s[0] + s[2] * s[2]) < kp.target_radius) cause |= CAUSE_BONUS;
-    }
-    if (abs_t(s[0]) >= kp.bounds || abs_t(s[2]) >= kp.bounds) {    // task.py:111
-        done = true; cause |= CAUSE_OOB;
-    } else if (abs_t(s[6]) >= kp.max_angle || abs_t(s[8]) >= kp.max_angle) {   // :116
-        done = true; cause |= CAUSE_ANGLE;
-    } else if (st0 == ST_CRASHED) {                                // :121
-        done = true;
-    }
-    if (st0 == ST_CRASHED) cause |= CAUSE_CRASHED;
-    if (steps == kp.max_steps) { done = true; cause |= CAUSE_TIMEOUT; }          // :128
-    steps = steps < kp.steps_cap ? steps + 1 : kp.steps_cap;       // :130
-    if (!done) cause = 0;
-}
-// the same without the "past the first step" condition: the precondition of airborne_arith_pert()
-template <typename T>
-__device__ __forceinline__ bool airborne_hot_fresh(const T (&s)[12], int st) {
-    return airborne_hot_c<T>(s[4], s[5], s[6], s[8], s[10], st, 0);
-}
-
 // Returns the step's ending flags: bit 0 out of bounds, bit 1 over-angle (exclusive: the reference
 // tests them with if / elif, task.py:111-118), bit 2 the env's own step limit; 0 = the episode goes
 // on.  airborne_cause() turns them into the CAUSE_* bits env_advance reports.
 enum { END_OOB = 1, END_ANGLE = 2, END_TIMEOUT = 4 };
-// the arithmetic of one such step (no flags, no step counter); L = float, double or F2
-template <typename L, typename T>
-__device__ __forceinline__ void airborne_arith(const KParams<T>& kp, L (&s)[12], const Forces<L>& f, L& na, L& nc) {
-    L sph, cph, sth, cth, sps, cps;
-    if constexpr (sizeof(T) == 4) { sincos_poly<L>(s[6], sph, cph); sincos_poly<L>(s[8], sth, cth); sincos_poly<L>(s[10], sps, cps); }
+// the arithmetic of one such step (no flags, no step counter)
+template <typename T>
+__device__ __forceinline__ void airborne_arith(const KParams<T>& kp, T (&s)[12], const Forces<T>& f, T& na, T& nc) {
+    T sph, cph, sth, cth, sps, cps;
+    if constexpr (sizeof(T) == 4) { sincos_poly<T>(s[6], sph, cph); sincos_poly<T>(s[8], sth, cth); sincos_poly<T>(s[10], sps, cps); }
     else sincos3_t(s[6], s[8], s[10], sph, cph, sth, cth, sps, cps);
-    const L none[3] = {L((T)0), L((T)0), L((T)0)};
-    airborne_integrate<L, T, 3, false>(kp, s, f, none, sph, cph, sth, cth, sps, cps, na, nc);
-}
-// the same with the reset perturbation `p` of a fresh episode (zeros for an env past its first step): exactly the
-// airborne case of dynamics_update, which always carries the perturbation terms
-template <typename L, typename T>
-__device__ __forceinline__ void airborne_arith_pert(const KParams<T>& kp, L (&s)[12], const Forces<L>& f, const L (&p)[3], L& na, L& nc) {
-    L sph, cph, sth, cth, sps, cps;
-    if constexpr (sizeof(T) == 4) { sincos_poly<L>(s[6], sph, cph); sincos_poly<L>(s[8], sth, cth); sincos_poly<L>(s[10], sps, cps); }
-    else sincos3_t(s[6], s[8], s[10], sph, cph, sth, cth, sps, cps);
-    airborne_integrate<L, T, 3, true>(kp, s, f, p, sph, cph, sth, cth, sps, cps, na, nc);
+    const T none[3] = {(T)0, (T)0, (T)0};
+    airborne_integrate<T, T, 3, false>(kp, s, f, none, sph, cph, sth, cth, sps, cps, na, nc);
 }
 // task.py:111-130 with the stale status AIRBORNE, on the state after the step
 template <typename T, int VARIANT>

@@ -6,9 +6,8 @@ north_star asks for done / terminated flags and step counts that are bit-exact. 
 numpy reference that can only hold away from thresholds (an fp32 rounding may flip `z > 0 && dz > 0`,
 `|x| >= 10`, `|phi| >= pi/4` one step early or late; tests/test_host_restatement.py measures that rate
 on the CPU).  What the GPU path itself owes is that it EXECUTES the fp32 arithmetic it is defined by
-exactly: every fast path (K = 1 specialisation, straight-line substeps, calm streaks, two envs per
-thread on fma.rn.f32x2), every warp vote, and ptxas' code generation have to reproduce the plain
-one-env-at-a-time loop.  Here, on every action stream, variant and K:
+exactly: every fast path (K = 1 specialisation, straight-line substeps, calm streaks), every warp
+vote, and ptxas' code generation have to reproduce the plain one-env-at-a-time loop.  Here, on every action stream, variant and K:
     state (all 12 components), observation, flight status, step counter, episode index, done flag,
     ending cause and terminal observation: identical bits / values, ZERO flips allowed;
     reward: the device takes the two square roots and the quotient of the shaping difference on the
@@ -203,42 +202,3 @@ def test_fp32_dynamics_facade_equals_the_host_instantiation(pkg):
         assert np.array_equal(bits(d.state.cpu().numpy()), bits(h.x)), t
     assert len(set(h.status.tolist())) >= 3
 
-
-def test_packed_two_env_kernel_is_bit_exact_too():
-    """The A/B kernel (two envs per thread on fma.rn.f32x2, off by default because it is slower): the same
-    bit-for-bit check, in a subprocess because the switch COPTER_B200_PAIR_MIN_K is read once per process."""
-    import os
-    import subprocess
-    import sys
-    code = r'''
-import sys, numpy as np, torch
-sys.path.insert(0, %r)
-import gym_copter_b200 as g
-from oracle.host_restatement import HostEnvBatch
-sys.path.insert(0, %r)
-from test_gpu_host_exact import mixed_streams, bits
-for variant, A in (('Lander3D', 4), ('Hover2D', 2)):
-    for k in (3, 16):
-        N, T = 2048 + 77, 640 // k
-        act = mixed_streams(np.random.default_rng(k), N, T, A)
-        env = g.CopterVecEnv(variant, N, dtype=torch.float32, seed=9, k_substeps=k, track_returns=True, report_cause=True, keep_final_obs=True)
-        host = HostEnvBatch(variant, N, dtype=np.float32, seed=9)
-        env.reset(); host.reset()
-        ep = 0
-        for t in range(T):
-            obs, r, term, trunc, info = env.step(torch.as_tensor(act[t]))
-            h_obs, h_r, h_done, h_info = host.step(act[t], k)
-            assert np.array_equal(bits(env.state.cpu().numpy()), bits(host.x)), (variant, k, t)
-            assert np.array_equal(term.cpu().numpy(), h_done) and np.array_equal(env.steps.cpu().numpy(), host.steps)
-            assert np.array_equal(env.status.cpu().numpy(), host.status) and np.array_equal(info['cause'].cpu().numpy(), h_info['cause'])
-            assert np.array_equal(bits(obs.cpu().numpy()), bits(h_obs))
-            assert np.array_equal(bits(info['final_obs'].cpu().numpy()[h_done]), bits(h_info['final_obs'][h_done]))
-            assert (np.abs(r.cpu().numpy() - h_r) / np.maximum(np.abs(h_r), 1)).max() <= 5e-5
-            ep += int(h_done.sum())
-        s = env.stats()
-        assert s['episodes'] == ep and ep > N // 2, (s['episodes'], ep)
-print('PAIR-OK')
-''' % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, '-c', code], env=dict(os.environ, COPTER_B200_PAIR_MIN_K='3'),
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and 'PAIR-OK' in r.stdout, (r.stdout[-500:], r.stderr[-1500:])

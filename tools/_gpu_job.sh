@@ -12,7 +12,6 @@ timeout 900 python bench.py --steps 20 --warmup 5 > gpurun_out/r2_bench_1gpu_dri
 timeout 300 python bench.py --impl reference --steps 20 --warmup 3 > gpurun_out/r2_bench_reference_arm.json 2>/dev/null; echo "ref exit $?"
 timeout 900 python tools/bench_extra.py > gpurun_out/r2_bench_extra.txt 2>&1; echo "extra exit $?"
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 120 --csv --log-file gpurun_out/r2_launches.csv python bench.py --steps 3 --warmup 3 --repeats 1 --no-cpu-baseline --e2e-steps 1 > /tmp/ncu_launch.log 2>&1; echo "ncu launches exit $?"
-COPTER_B200_PAIR_MIN_K=3 bash tools/_ncu_capture.sh step_pair_kernel_k16 copter_step 2 1 8388608 -- python tools/profile_k.py 16
 bash tools/_ncu_capture.sh policy_kernels policy 0 8 262144 -- python tools/profile_policy.py
 bash tools/_ncu_capture.sh other_kernels copter_ 0 24 1 -- python tools/profile_misc.py
 timeout 900 compute-sanitizer --tool memcheck python tools/sanitize.py > gpurun_out/r2_sanitizer_memcheck.txt 2>&1; echo "memcheck exit $?"; tail -n 3 gpurun_out/r2_sanitizer_memcheck.txt

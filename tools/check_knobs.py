@@ -1,9 +1,9 @@
 #!/usr/bin/env python3
 """
-Developer tool: cross-compiles the library once per A/B knob combination (no GPU needed) so that
-the alternative shapes kept for measurements -- persistent grids, register / TMA prefetch, cluster
-launch control, the untied loads, the plain K loop, the library-only math, the policy variants --
-do not rot.  Runs the builds in parallel; prints one line per combination.
+Developer tool: cross-compiles the library once per A/B knob combination of the policy kernels
+(no GPU needed) so that the alternative shapes kept for measurements -- tcgen05 slots and splits,
+polynomial tanh, cluster launch control, the warp-MMA kernel -- do not rot.  Runs the builds in
+parallel; prints one line per combination.
 
     python tools/check_knobs.py
 """
@@ -17,21 +17,13 @@ sys.path.insert(0, ROOT)
 from gym_copter_b200.build import NVCC_FLAGS          # noqa: E402
 SRC = os.path.join(ROOT, 'gym_copter_b200', 'csrc', 'copter_kernels.cu')
 COMBOS = [
-    ['-DCOPTER_PERSISTENT=1'],
-    ['-DCOPTER_PERSISTENT=1', '-DCOPTER_PREFETCH=1'],
-    ['-DCOPTER_TMA_MIN_K=1'],
-    ['-DCOPTER_TMA_MIN_K=2', '-DCOPTER_TMA_CLC=0', '-DCOPTER_TMA_CTAS_PER_SM=7'],
-    ['-DCOPTER_TIE_LOADS=0', '-DCOPTER_CALM_STREAK=0'],
-    ['-DCOPTER_FAST_SUBSTEP=0', '-DCOPTER_LIBM_ONLY=1', '-DCOPTER_PAIR_MIN_K=0'],
-    ['-DCOPTER_PAIR_MIN_K=2', '-DCOPTER_PAIR_CTAS_PER_SM=3'],
-    ['-DCOPTER_STREAMING=1', '-DCOPTER_K1_SPECIALIZE=0', '-DCOPTER_K_UNROLL=4'],
     ['-DCOPTER_POLICY_POLY_MASK=0x88', '-DCOPTER_POLICY_MT=1'],
     ['-DCOPTER_POLICY_POLY_MASK=0xff', '-DCOPTER_POLICY_POLY_F32X2=0', '-DCOPTER_POLICY_TANH_BF16X2=1'],
     ['-DCOPTER_POLICY_TC_SLOTS=2', '-DCOPTER_POLICY_TC_SPLIT=2', '-DCOPTER_POLICY_TC_POLY=0'],        # (no tcgen05 fused rollout in these shapes)
     ['-DCOPTER_POLICY_TC_POLY=8', '-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=3', '-DCOPTER_POLICY_TC=0'],
     ['-DCOPTER_POLICY_TC_CLC=0', '-DCOPTER_POLICY_TC_ONES_ROWS=128', '-DCOPTER_POLICY_TC_CTAS_PER_SM=5', '-DCOPTER_POLICY_ROLLOUT_TC=0'],
-    ['-DCOPTER_GROUND_FF=1', '-DCOPTER_GROUND_SPLIT=1', '-DCOPTER_FRESH_FAST=1', '-DCOPTER_POLICY_TC_WAIT=2'],
-    ['-DCOPTER_GROUND_FF=2', '-DCOPTER_POLICY_TC_F16=2', '-DCOPTER_POLICY_TC_POLY=6'],
+    ['-DCOPTER_POLICY_TC_WAIT=2'],
+    ['-DCOPTER_POLICY_TC_F16=2', '-DCOPTER_POLICY_TC_POLY=6'],
 ]
 
 

@@ -1,5 +1,5 @@
 """Developer tool: a few K-fused step launches on a desynchronised batch, for `ncu -k regex:copter_step`.
-    python tools/profile_k.py [k] [envs]      (COPTER_B200_PAIR_MIN_K=3 selects the packed two-env kernel)"""
+    python tools/profile_k.py [k] [envs]"""
 import os
 import sys
 

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """
-Developer tool: build-time parameter sweep of the step kernel (CTAs/SM target, block size,
-cache hints).  `build` cross-compiles the variants here (no GPU needed) into tools/variants/;
-`run` times each on the GPU box (one subprocess per variant) and prints achieved GB/s.
+Developer tool: build-time parameter sweep (step kernel: CTAs/SM target, block size; policy
+kernels: the COPTER_POLICY_* knobs).  `build` cross-compiles the variants here (no GPU needed) into
+tools/variants/; `run` times each on the GPU box (one subprocess per variant) and prints achieved GB/s.
 
     python tools/sweep.py build
     gpurun -- python tools/sweep.py run [--envs N] [--k K]
@@ -21,10 +21,6 @@ from gym_copter_b200.build import NVCC_FLAGS          # noqa: E402  (the product
 
 VARIANTS = {}
 VARIANTS['current'] = []
-VARIANTS['nopair'] = ['-DCOPTER_PAIR_MIN_K=0']        # K-fused fp32 launches on the one-env-per-thread kernel
-VARIANTS['pair_plainmul'] = ['-DCOPTER_F2_PLAIN_MUL_ADD=1']   # packed kernel with FMUL2 / FADD2 instead of FFMA2-only
-VARIANTS['pair_c5'] = ['-DCOPTER_PAIR_CTAS_PER_SM=5']         # packed kernel at 5 CTAs per SM (<= 96 registers)
-VARIANTS['pair_k2'] = ['-DCOPTER_PAIR_MIN_K=2']               # packed kernel from K = 2 on
 VARIANTS['tc_s1'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=1']    # tcgen05 policy kernel: 1 tile in flight per CTA, 4 CTAs per SM, one thread per row
 VARIANTS['tc_s1x2'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=2']  # two threads per row, 3 CTAs per SM
 VARIANTS['tc_s1x2c4'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=2', '-DCOPTER_POLICY_TC_CTAS_PER_SM=4']  # 4 CTAs per SM (<= 56 registers)
@@ -40,14 +36,6 @@ VARIANTS['tc_ro5'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=5']  # fused rollo
 VARIANTS['tc_ro5c5'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=5', '-DCOPTER_POLICY_TC_CTAS_PER_SM=5']
 VARIANTS['tc_ro3'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=3']
 VARIANTS['tc_s2x2'] = ['-DCOPTER_POLICY_TC_SLOTS=2', '-DCOPTER_POLICY_TC_SPLIT=2']  # 2 tiles in flight, 2 CTAs per SM, two threads per row
-VARIANTS['nofast'] = ['-DCOPTER_FAST_SUBSTEP=0']      # K-fused loop without the straight-line substep
-VARIANTS['nostreak'] = ['-DCOPTER_CALM_STREAK=0']     # K-fused loop: flags + hot test + two votes on every substep
-VARIANTS['tma_k2'] = ['-DCOPTER_TMA_MIN_K=2']         # K-fused launches through the TMA-prefetch + cluster-launch-control kernel
-VARIANTS['tma_k2_c7'] = ['-DCOPTER_TMA_MIN_K=2', '-DCOPTER_TMA_CTAS_PER_SM=7']
-VARIANTS['tma_k1'] = ['-DCOPTER_TMA_MIN_K=1']         # K = 1 through the TMA kernel too
-VARIANTS['tma_k1_c6'] = ['-DCOPTER_TMA_MIN_K=1', '-DCOPTER_TMA_CTAS_PER_SM=6']
-VARIANTS['tma_k2_noclc'] = ['-DCOPTER_TMA_MIN_K=2', '-DCOPTER_TMA_CLC=0']         # static grid-stride tiles instead of cluster launch control
-VARIANTS['tma_k1_noclc'] = ['-DCOPTER_TMA_MIN_K=1', '-DCOPTER_TMA_CLC=0']
 if os.environ.get('COPTER_SWEEP_ONLY'):
     VARIANTS = {k: v for k, v in VARIANTS.items() if k.startswith(tuple(os.environ['COPTER_SWEEP_ONLY'].split(',')))}
 
