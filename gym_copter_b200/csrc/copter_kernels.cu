@@ -644,12 +644,10 @@ struct PolicyRolloutArgs {
     uint8_t* cause_tn; float* final_obs_tn;   // ending records (RECORD instantiations only)
 };
 
-#ifndef COPTER_POLICY_ROLLOUT_CTAS_PER_SM
-#define COPTER_POLICY_ROLLOUT_CTAS_PER_SM 5   // measured (tools/sweep_policy.py): 3: 0.413, 4: 0.420, 5: 0.400, 6: 0.425 ms per env-step
-#endif
+constexpr int kPolicyRolloutCtasPerSm = 5;   // measured (profiles/r1_sweep_policy_occupancy.txt): 3: 0.413, 4: 0.420, 5: 0.400, 6: 0.425 ms per env-step
 
 template <int VARIANT, bool STATS, bool RECORD>
-__global__ void __launch_bounds__(128, COPTER_POLICY_ROLLOUT_CTAS_PER_SM)
+__global__ void __launch_bounds__(128, kPolicyRolloutCtasPerSm)
 copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __grid_constant__ PolicyRolloutArgs a) {
     using T = float;
     static_assert(kBlock == 128, "policy kernels are written for 4 warps per CTA");
@@ -769,28 +767,22 @@ copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __
 // observation staging folded into the A tile (profiles/r2_sweep_policy_tc_rollout2.txt):
 //   4 CTAs/SM 0.376, 5 CTAs/SM 0.373, 6 CTAs/SM (64 registers, no spills) 0.342, 7 CTAs/SM (56 registers) 0.348
 // -- 2.45e10 env-steps/s, 15 % faster than the warp-MMA kernel, so this kernel is the default of the fused rollout
-// (COPTER_B200_POLICY_ROLLOUT_TC=0 or -DCOPTER_POLICY_ROLLOUT_TC=0 selects the warp-MMA kernel).
-#ifndef COPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM
-#define COPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM 6      // x 64 TMEM columns <= the SM's 512; 64 registers, 31.7 KB of shared memory (4: 0.376, 5: 0.373, 6: 0.342, 7: 0.348 ms per env-step)
-#endif
-#ifndef COPTER_POLICY_ROLLOUT_TC_PIPELINED
-#define COPTER_POLICY_ROLLOUT_TC_PIPELINED 0        // TMEM read-back double-buffered in registers (16 more registers; no gain)
-#endif
-// (the A/B shapes of the standalone kernel with several tiles in flight or two threads per row do not apply here)
-#define COPTER_POLICY_ROLLOUT_TC_AVAILABLE (COPTER_POLICY_TC_SLOTS == 1 && COPTER_POLICY_TC_SPLIT == 1)
-#if COPTER_POLICY_ROLLOUT_TC_AVAILABLE
+// (COPTER_B200_POLICY_ROLLOUT_TC=0 selects the warp-MMA kernel).  The TMEM read-back stays single-buffered in registers
+// (hidden_epilogue<false>): double-buffered it costs 16 more registers for no gain (the knob is removed; the last tree
+// that has it is commit d11af01).
+constexpr int kPolicyRolloutTcCtasPerSm = 6;      // x 64 TMEM columns <= the SM's 512; 64 registers, 31.7 KB of shared memory (4: 0.376, 5: 0.373, 6: 0.342, 7: 0.348 ms per env-step)
 
 struct RolloutTcSmem {
-    tc::Smem mlp;                                   // weights, the slot's A tiles, the mbarriers
-    // The per-warp observation staging of write_obs_rows (4 x 1.5 KB) lives INSIDE the slot's hidden A tile, past the
+    tc::Smem mlp;                                   // weights, the A tile, the mbarriers
+    // The per-warp observation staging of write_obs_rows (4 x 1.5 KB) lives INSIDE the hidden A tile, past the
     // 4 KB its layer-1 alias occupies: observations are recorded at the start of an env-step and after the last one,
     // when no MMA reads that tile and no thread writes it before layer 1 has completed (6 KB less per CTA).
-    __device__ __forceinline__ float* stage(int warp) { return reinterpret_cast<float*>(reinterpret_cast<char*>(mlp.slot[0].a) + 4096) + warp * (32 * 12); }
+    __device__ __forceinline__ float* stage(int warp) { return reinterpret_cast<float*>(reinterpret_cast<char*>(mlp.slot.a) + 4096) + warp * (32 * 12); }
 };
 static_assert(4096 + 4 * 32 * 12 * sizeof(float) <= sizeof(tc::SlotSmem), "observation staging fits behind the layer-1 alias");
 
 template <int VARIANT, bool STATS, bool RECORD>
-__global__ void __launch_bounds__(tc::kTile + 32, COPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM)
+__global__ void __launch_bounds__(tc::kThreads, kPolicyRolloutTcCtasPerSm)
 copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const __grid_constant__ PolicyRolloutArgs a) {
     using T = float;
     constexpr int O = Variant<VARIANT>::O, A = Variant<VARIANT>::A, FIRST = Variant<VARIANT>::first;
@@ -800,8 +792,8 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
     const int t_id = threadIdx.x, warp = t_id >> 5, lane = t_id & 31;
     constexpr int kMmaWarp = tc::kTile / 32;
     if (t_id == 0) {
-        tc::bar_init(&sm.done[0], 1);
-        tc::bar_init(&sm.ready[0], tc::kTile);
+        tc::bar_init(&sm.done, 1);
+        tc::bar_init(&sm.ready, tc::kTile);
         tc::bar_init(&sm.clc_bar[0], 1); tc::bar_init(&sm.clc_bar[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -813,31 +805,30 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
     tc::fence_after_sync();
     const uint32_t tmem_base = sm.tmem_base;
     if (STATS) credit_env_steps(a.stats, a.n, a.n_steps);
-    const int64_t n_tiles = (a.n + tc::kTile - 1) / tc::kTile;
 
     if (warp == kMmaWarp) {
         // ===== MMA issuer: 3 layers per env-step, n_steps env-steps per tile.  Warp-uniform, the issuing lane elected per
         // layer (tc::issue_layer_uniform); tiles by cluster launch control, one request in flight (tc::next_tile) =====
-        const tc::LayerDescs d = tc::make_layer_descs(sm, 0, tmem_base);
+        const tc::LayerDescs d = tc::make_layer_descs(sm, tmem_base);
         uint32_t phase = 0, clc_phase = 0, tile_id = blockIdx.x;
         tc::request_tile(sm, 0);
         for (int k = 0; tile_id != tc::kNoTile; ++k) {
             for (int t = 0; t < a.n_steps; ++t)
 #pragma unroll
                 for (int layer = 1; layer <= 3; ++layer) {
-                    tc::bar_wait(&sm.ready[0], phase); phase ^= 1u;
-                    tc::issue_layer_uniform(d, layer, &sm.done[0]);
+                    tc::bar_wait(&sm.ready, phase); phase ^= 1u;
+                    tc::issue_layer_uniform(d, layer, &sm.done);
                 }
-            tile_id = tc::next_tile(sm, k, tile_id, clc_phase, n_tiles);
+            tile_id = tc::next_tile(sm, k, clc_phase);
             if (tile_id != tc::kNoTile) tc::request_tile(sm, k + 1);      // clc_resp[(k + 1) & 1] was last read at the end of tile k - 1
         }
     } else {
         // ===== epilogue warps: thread <-> env row <-> TMEM lane =====
         const int row = t_id;                                                        // 0..127
         const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);        // this warp's quarter of the TMEM lanes
-        tc::SlotSmem& ss = sm.slot[0];
+        tc::SlotSmem& ss = sm.slot;
         uint32_t phase = 0, clc_phase = 0, tile_id = blockIdx.x;
-        for (int k = 0; tile_id != tc::kNoTile; tile_id = tc::next_tile(sm, k, tile_id, clc_phase, n_tiles), ++k) {
+        for (int k = 0; tile_id != tc::kNoTile; tile_id = tc::next_tile(sm, k, clc_phase), ++k) {
             const int64_t row0 = (int64_t)tile_id * tc::kTile + warp * 32, i = row0 + lane;
             const bool valid = i < a.n;
             const int64_t left = a.n - row0;
@@ -859,20 +850,20 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
                 if (a.obs_tn && rows > 0) write_obs_rows<VARIANT, T>(a.obs_tn + (int64_t)t * a.n * O, rs.stage(warp), lane, row0, rows, s);
                 tc::write_obs_row<FIRST, O>(ss, row, s);
                 tc::fence_before_sync();
-                tc::bar_arrive(&sm.ready[0]);
+                tc::bar_arrive(&sm.ready);
 #pragma unroll
                 for (int layer = 1; layer <= 2; ++layer) {
-                    tc::bar_wait(&sm.done[0], phase); phase ^= 1u;
+                    tc::bar_wait(&sm.done, phase); phase ^= 1u;
                     tc::fence_after_sync();
-                    tc::hidden_epilogue<4, COPTER_POLICY_ROLLOUT_TC_PIPELINED != 0>(lane_base + tc::col_hidden(0), ss.a, row, 0);
+                    tc::hidden_epilogue<false>(lane_base + tc::kColHidden, ss.a, row);
                     tc::fence_async_smem();
                     tc::fence_before_sync();
-                    tc::bar_arrive(&sm.ready[0]);
+                    tc::bar_arrive(&sm.ready);
                 }
-                tc::bar_wait(&sm.done[0], phase); phase ^= 1u;
+                tc::bar_wait(&sm.done, phase); phase ^= 1u;
                 tc::fence_after_sync();
                 float pre[4];
-                tc::tmem_ld4(lane_base + tc::col_out(0), pre);
+                tc::tmem_ld4(lane_base + tc::kColOut, pre);
                 T act[A];
 #pragma unroll
                 for (int j = 0; j < A; ++j) act[j] = fmaf(a.w.out_scale, tc::tanh_mufu(pre[j]), a.w.out_offset);
@@ -934,7 +925,6 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
     __syncthreads();
     if (warp == kMmaWarp) tc::tmem_free(tmem_base);
 }
-#endif  // COPTER_POLICY_ROLLOUT_TC_AVAILABLE
 
 // ------------------------------------------------------------------------------------------
 // Generalised advantage estimation over the [T][n] rows of a rollout (copter_gae_f32; the
@@ -1280,24 +1270,18 @@ int persistent_grid_for(int64_t n) {
     return (int)(tiles < cap ? tiles : cap);
 }
 
-// Which policy kernel: 1 = tcgen05 / TMEM (copter_policy_tc.cuh), 0 = warp-level mma.sync (copter_policy.cuh).
-// COPTER_B200_POLICY_TC in the environment overrides the build default (A/B runs, tests of both).
-#ifndef COPTER_POLICY_TC
-#define COPTER_POLICY_TC 1
-#endif
+// Which policy kernel: 1 = tcgen05 / TMEM (copter_policy_tc.cuh, the default), 0 = warp-level mma.sync (copter_policy.cuh),
+// from COPTER_B200_POLICY_TC in the environment (A/B runs, tests of both).
 int policy_tc_setting() {
     const char* e = getenv("COPTER_B200_POLICY_TC");        // read on every call: tests and A/B runs flip it inside one process
-    return e ? (atoi(e) != 0) : COPTER_POLICY_TC;
+    return e ? (atoi(e) != 0) : 1;
 }
 // The same choice for the fused policy + step rollout (copter_policy_rollout_f32).  Until the tcgen05 kernel took its
 // tiles by cluster launch control and issued its MMAs warp-uniformly the warp-MMA kernel won (0.404 vs 0.424 ms per
 // env-step at 2^23 envs); since then the tcgen05 kernel does (0.342 ms, 6 CTAs per SM), so it is the default.
-#ifndef COPTER_POLICY_ROLLOUT_TC
-#define COPTER_POLICY_ROLLOUT_TC 1
-#endif
 int policy_rollout_tc_setting() {
     const char* e = getenv("COPTER_B200_POLICY_ROLLOUT_TC");
-    return e ? (atoi(e) != 0) : COPTER_POLICY_ROLLOUT_TC;
+    return e ? (atoi(e) != 0) : 1;
 }
 
 template <int VARIANT>
@@ -1316,17 +1300,15 @@ int launch_policy_v(const PolicyArgs& a, cudaStream_t s) {
             if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
             configured[dev] = true;
         }
-        const int64_t tiles = (a.n + tc::kTile - 1) / tc::kTile, pairs = (tiles + tc::kSlots - 1) / tc::kSlots;
-        const int64_t cap = (int64_t)sm_count() * COPTER_POLICY_TC_CTAS_PER_SM;
+        const int64_t tiles = (a.n + tc::kTile - 1) / tc::kTile;
         // cluster launch control: one CTA per tile in the grid, the resident CTAs take the pending ones over
-        kernel<<<(int)(tc::kClc ? tiles : (pairs < cap ? pairs : cap)), tc::kThreads, smem, s>>>(t);
+        kernel<<<(int)tiles, tc::kThreads, smem, s>>>(t);
         return (int)cudaGetLastError();
     }
     copter_mlp_policy_kernel<V::first, V::O, V::A><<<persistent_grid_for<copter_mlp_policy_kernel<V::first, V::O, V::A>>(a.n), 128, 0, s>>>(a);
     return (int)cudaGetLastError();
 }
 
-#if COPTER_POLICY_ROLLOUT_TC_AVAILABLE
 template <int VARIANT, bool STATS, bool RECORD>
 int launch_policy_rollout_tc(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
     constexpr auto kernel = copter_policy_rollout_tc_kernel<VARIANT, STATS, RECORD>;
@@ -1337,18 +1319,15 @@ int launch_policy_rollout_tc(const KParams<float>& kp, const PolicyRolloutArgs& 
         if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
         configured[dev] = true;
     }
-    const int64_t tiles = (a.n + tc::kTile - 1) / tc::kTile, cap = (int64_t)sm_count() * COPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM;
-    kernel<<<(int)(tc::kClc ? tiles : (tiles < cap ? tiles : cap)), tc::kTile + 32, smem, s>>>(kp, a);
+    const int64_t tiles = (a.n + tc::kTile - 1) / tc::kTile;
+    kernel<<<(int)tiles, tc::kThreads, smem, s>>>(kp, a);           // cluster launch control, as above
     return (int)cudaGetLastError();
 }
-#endif
 
 template <int VARIANT, bool R>
 int launch_policy_rollout_vr(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
-#if COPTER_POLICY_ROLLOUT_TC_AVAILABLE
-    if (policy_rollout_tc_setting())    // the tcgen05 / TMEM kernel; default: the warp-MMA kernel
+    if (policy_rollout_tc_setting())    // the tcgen05 / TMEM kernel (the default); otherwise the warp-MMA kernel
         return a.stats ? launch_policy_rollout_tc<VARIANT, true, R>(kp, a, s) : launch_policy_rollout_tc<VARIANT, false, R>(kp, a, s);
-#endif
     if (a.stats) copter_policy_rollout_kernel<VARIANT, true, R><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, true, R>>(a.n), 128, 0, s>>>(kp, a);
     else         copter_policy_rollout_kernel<VARIANT, false, R><<<persistent_grid_for<copter_policy_rollout_kernel<VARIANT, false, R>>(a.n), 128, 0, s>>>(kp, a);
     return (int)cudaGetLastError();

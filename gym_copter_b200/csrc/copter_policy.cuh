@@ -55,80 +55,12 @@ __device__ __forceinline__ float tanh_fast(float x) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-// hidden activations.  COPTER_POLICY_TANH_BF16X2 (A/B knob) rounds the pair to bf16 first and
-// uses tanh.approx.bf16x2; it is not faster on B200 (the packed form costs two XU slots) and is
-// less accurate, so the default is two fp32 MUFU.TANH.
-#ifndef COPTER_POLICY_MT
-#define COPTER_POLICY_MT 2             // row tiles of 16 envs carried through the layers together (A/B knob: 1)
-#endif
-#ifndef COPTER_POLICY_TANH_BF16X2
-#define COPTER_POLICY_TANH_BF16X2 0      // measured on B200: 0.435 ms vs 0.412 ms for two fp32 tanh (2^23 envs)
-#endif
+// hidden activations: two fp32 MUFU.TANH, then one bf16 pair.  (tanh.approx.bf16x2 on the pair rounded to bf16 first is
+// not faster on B200 -- measured 0.435 ms vs 0.412 ms for 2^23 envs: the packed form costs two XU slots -- and is less
+// accurate; an FMA-pipe polynomial for some of the n-tiles gained 2 % at 1/8 of them and lost beyond
+// (profiles/r1_sweep_policy_poly_tanh.txt).  Both knobs are removed; the last tree that has them is commit d11af01.)
 __device__ __forceinline__ uint32_t tanh_pack(float lo, float hi) {
-#if COPTER_POLICY_TANH_BF16X2
-    uint32_t y;
-    asm("tanh.approx.bf16x2 %0, %1;" : "=r"(y) : "r"(pack_bf16(lo, hi)));
-    return y;
-#else
     return pack_bf16(tanh_fast(lo), tanh_fast(hi));
-#endif
-}
-// The same pair on the FMA pipe instead of the XU: clamp to |x| <= 3.25 and evaluate the odd
-// degree-13 polynomial x P(x^2) (weighted minimax fit, tools/fit_tanh_poly.py).  |error| <= 2.0e-3
-// absolute and <= 2.3e-3 relative, i.e. inside the half-ulp (2^-9 .. 2^-8 relative) of the bf16
-// rounding that follows; MUFU.TANH is 5e-4.  The policy kernels are bound by the XU pipe while the
-// FMA pipe idles (10 % busy, profiles/r1_policy_kernel_ncu_full.txt), so the n-tiles selected by
-// COPTER_POLICY_POLY_MASK take this route (the FlashAttention-4 exp2 trick, applied to tanh).
-#ifndef COPTER_POLICY_POLY_MASK
-#define COPTER_POLICY_POLY_MASK 0x00     // bit nt set: hidden n-tile nt (8 columns) of both layers uses the polynomial
-#endif
-#ifndef COPTER_POLICY_POLY_F32X2
-#define COPTER_POLICY_POLY_F32X2 1       // packed fma.rn.f32x2 (one issue slot per pair) vs scalar FFMA with immediates
-#endif
-constexpr float kTanhClamp = 3.25f;
-__host__ __device__ constexpr float tanh_poly_coef(int k) {    // coefficient of x^(2k+1)
-    constexpr float c[7] = {9.977270291e-01f, -3.117916466e-01f, 9.229137325e-02f, -1.838625564e-02f,
-                            2.184749761e-03f, -1.380842544e-04f, 3.552717362e-06f};
-    return c[k];
-}
-__device__ __forceinline__ uint64_t f32x2(float lo, float hi) {
-    uint64_t r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ uint64_t fma_f32x2(uint64_t a, uint64_t b, uint64_t c) {
-    uint64_t d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-    return d;
-}
-__device__ __forceinline__ uint64_t mul_f32x2(uint64_t a, uint64_t b) {
-    uint64_t d;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-    return d;
-}
-__device__ __forceinline__ uint32_t tanh_pack_poly(float lo, float hi) {
-    lo = fminf(fmaxf(lo, -kTanhClamp), kTanhClamp);
-    hi = fminf(fmaxf(hi, -kTanhClamp), kTanhClamp);
-#if COPTER_POLICY_POLY_F32X2
-    const uint64_t x = f32x2(lo, hi), u = mul_f32x2(x, x);
-    uint64_t p = f32x2(tanh_poly_coef(6), tanh_poly_coef(6));
-#pragma unroll
-    for (int k = 5; k >= 0; --k) p = fma_f32x2(p, u, f32x2(tanh_poly_coef(k), tanh_poly_coef(k)));
-    const uint64_t r = mul_f32x2(p, x);
-    float rl, rh;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(rl), "=f"(rh) : "l"(r));
-    return pack_bf16(rl, rh);
-#else
-    const float ul = lo * lo, uh = hi * hi;
-    float pl = tanh_poly_coef(6), ph = tanh_poly_coef(6);
-#pragma unroll
-    for (int k = 5; k >= 0; --k) { pl = fmaf(pl, ul, tanh_poly_coef(k)); ph = fmaf(ph, uh, tanh_poly_coef(k)); }
-    return pack_bf16(pl * lo, ph * hi);
-#endif
-}
-// hidden n-tile nt: XU or FMA-pipe tanh (nt is a constant once the layer loops are unrolled)
-__device__ __forceinline__ uint32_t tanh_pack_nt(int nt, float lo, float hi) {
-    return ((COPTER_POLICY_POLY_MASK >> nt) & 1) ? tanh_pack_poly(lo, hi) : tanh_pack(lo, hi);
 }
 // D = A B + D
 __device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
@@ -206,79 +138,76 @@ __device__ __forceinline__ void policy_forward_warp(const PolicySmem& sm, Policy
     xrow[1] = make_uint4(xin[4], xin[5], xin[6], xin[7]);
     __syncwarp();
 
-    // COPTER_POLICY_MT rows tiles of 16 envs are carried through the layers together (2: every weight
-    // fragment load serves both tiles and the two accumulator chains interleave; 1: half the live
-    // registers, twice the fragment loads)
-    constexpr int MT = COPTER_POLICY_MT;
-#pragma unroll 1
-    for (int m0 = 0; m0 < 2; m0 += MT) {
-        // layer-1 A fragments: four 8x8 matrices per row tile (rows 0-7 / 8-15 x k 0-7 / 8-15)
-        uint32_t a1[MT][4];
+    // both row tiles of 16 envs are carried through the layers together: every weight fragment load serves
+    // both tiles and the two accumulator chains interleave (one tile at a time: half the live registers, twice
+    // the fragment loads -- slower, profiles/r1_sweep_policy_occupancy.txt)
+    constexpr int MT = 2;
+    // layer-1 A fragments: four 8x8 matrices per row tile (rows 0-7 / 8-15 x k 0-7 / 8-15)
+    uint32_t a1[MT][4];
+#pragma unroll
+    for (int mt = 0; mt < MT; ++mt) {
+        const int j = lane >> 3, r = lane & 7;
+        ldmatrix_x4(a1[mt], wt.x + (16 * mt + 8 * (j & 1) + r) * kPolXStride + 8 * (j >> 1));
+    }
+
+    // ---- layer 1: [16 MT x 16] x [16 x 64], activations kept as the A fragments of layer 2 ----
+    uint32_t h[MT][4][4];
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) {
+        const uint2 b = sm.w1[nt][lane];
+        const float4 bias = sm.b1[nt][t];
 #pragma unroll
         for (int mt = 0; mt < MT; ++mt) {
-            const int j = lane >> 3, r = lane & 7;
-            ldmatrix_x4(a1[mt], wt.x + (16 * (m0 + mt) + 8 * (j & 1) + r) * kPolXStride + 8 * (j >> 1));
+            float c[4];
+            mma_bf16_bias(c, a1[mt], b.x, b.y, bias);
+            h[mt][nt >> 1][(nt & 1) * 2 + 0] = tanh_pack(c[0], c[1]);      // rows g
+            h[mt][nt >> 1][(nt & 1) * 2 + 1] = tanh_pack(c[2], c[3]);      // rows g + 8
         }
+    }
 
-        // ---- layer 1: [16 MT x 16] x [16 x 64], activations kept as the A fragments of layer 2 ----
-        uint32_t h[MT][4][4];
+    // ---- layer 2: [16 MT x 64] x [64 x 64], two n-tiles at a time, each pair feeding one k-tile of
+    // ---- layer 3: [16 MT x 64] x [64 x 8]
+    float c3[MT][4];
 #pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-            const uint2 b = sm.w1[nt][lane];
-            const float4 bias = sm.b1[nt][t];
+    for (int kt3 = 0; kt3 < 4; ++kt3) {
+        uint32_t a3[MT][4];
 #pragma unroll
-            for (int mt = 0; mt < MT; ++mt) {
-                float c[4];
-                mma_bf16_bias(c, a1[mt], b.x, b.y, bias);
-                h[mt][nt >> 1][(nt & 1) * 2 + 0] = tanh_pack_nt(nt, c[0], c[1]);      // rows g
-                h[mt][nt >> 1][(nt & 1) * 2 + 1] = tanh_pack_nt(nt, c[2], c[3]);      // rows g + 8
-            }
-        }
-
-        // ---- layer 2: [16 MT x 64] x [64 x 64], two n-tiles at a time, each pair feeding one k-tile of
-        // ---- layer 3: [16 MT x 64] x [64 x 8]
-        float c3[MT][4];
+        for (int half = 0; half < 2; ++half) {
+            const int nt = 2 * kt3 + half;
+            const float4 bias = sm.b2[nt][t];
+            float c[MT][4];
 #pragma unroll
-        for (int kt3 = 0; kt3 < 4; ++kt3) {
-            uint32_t a3[MT][4];
-#pragma unroll
-            for (int half = 0; half < 2; ++half) {
-                const int nt = 2 * kt3 + half;
-                const float4 bias = sm.b2[nt][t];
-                float c[MT][4];
-#pragma unroll
-                for (int kp = 0; kp < 2; ++kp) {
-                    const uint4 b = sm.w2[nt][kp][lane];
-#pragma unroll
-                    for (int mt = 0; mt < MT; ++mt) {
-                        if (kp == 0) mma_bf16_bias(c[mt], h[mt][0], b.x, b.y, bias);
-                        else         mma_bf16(c[mt], h[mt][2], b.x, b.y);
-                        mma_bf16(c[mt], h[mt][2 * kp + 1], b.z, b.w);
-                    }
-                }
+            for (int kp = 0; kp < 2; ++kp) {
+                const uint4 b = sm.w2[nt][kp][lane];
 #pragma unroll
                 for (int mt = 0; mt < MT; ++mt) {
-                    a3[mt][half * 2 + 0] = tanh_pack_nt(nt, c[mt][0], c[mt][1]);
-                    a3[mt][half * 2 + 1] = tanh_pack_nt(nt, c[mt][2], c[mt][3]);
+                    if (kp == 0) mma_bf16_bias(c[mt], h[mt][0], b.x, b.y, bias);
+                    else         mma_bf16(c[mt], h[mt][2], b.x, b.y);
+                    mma_bf16(c[mt], h[mt][2 * kp + 1], b.z, b.w);
                 }
             }
-            const uint4 b = sm.w3[kt3 >> 1][lane];
-            const uint32_t b0 = (kt3 & 1) ? b.z : b.x, b1 = (kt3 & 1) ? b.w : b.y;
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt) {
-                if (kt3 == 0) mma_bf16_bias(c3[mt], a3[mt], b0, b1, sm.b3[t]);
-                else          mma_bf16(c3[mt], a3[mt], b0, b1);
+                a3[mt][half * 2 + 0] = tanh_pack(c[mt][0], c[mt][1]);
+                a3[mt][half * 2 + 1] = tanh_pack(c[mt][2], c[mt][3]);
             }
         }
-
-        // lanes t < 2 hold columns 2t, 2t+1 (< 4) of rows g and g + 8 of each row tile: hand every
-        // env's pre-activation row back to its own lane, which applies the output tanh once
-        if (t < 2) {
+        const uint4 b = sm.w3[kt3 >> 1][lane];
+        const uint32_t b0 = (kt3 & 1) ? b.z : b.x, b1 = (kt3 & 1) ? b.w : b.y;
 #pragma unroll
-            for (int mt = 0; mt < MT; ++mt) {
-                *reinterpret_cast<float2*>(wt.act + (16 * (m0 + mt) + g) * 4 + 2 * t) = make_float2(c3[mt][0], c3[mt][1]);
-                *reinterpret_cast<float2*>(wt.act + (16 * (m0 + mt) + g + 8) * 4 + 2 * t) = make_float2(c3[mt][2], c3[mt][3]);
-            }
+        for (int mt = 0; mt < MT; ++mt) {
+            if (kt3 == 0) mma_bf16_bias(c3[mt], a3[mt], b0, b1, sm.b3[t]);
+            else          mma_bf16(c3[mt], a3[mt], b0, b1);
+        }
+    }
+
+    // lanes t < 2 hold columns 2t, 2t+1 (< 4) of rows g and g + 8 of each row tile: hand every
+    // env's pre-activation row back to its own lane, which applies the output tanh once
+    if (t < 2) {
+#pragma unroll
+        for (int mt = 0; mt < MT; ++mt) {
+            *reinterpret_cast<float2*>(wt.act + (16 * mt + g) * 4 + 2 * t) = make_float2(c3[mt][0], c3[mt][1]);
+            *reinterpret_cast<float2*>(wt.act + (16 * mt + g + 8) * 4 + 2 * t) = make_float2(c3[mt][2], c3[mt][3]);
         }
     }
     __syncwarp();
@@ -295,13 +224,11 @@ struct PolicyArgs {
     float* action;                                   // [n][act]
 };
 
-#ifndef COPTER_POLICY_CTAS_PER_SM
-#define COPTER_POLICY_CTAS_PER_SM 5      // measured (tools/sweep_policy.py, 2^23 envs): 3: 0.386, 4: 0.373, 5: 0.359, 6: 0.368 ms
-#endif
+constexpr int kPolicyCtasPerSm = 5;      // measured (profiles/r1_sweep_policy_occupancy.txt, 2^23 envs): 3: 0.386, 4: 0.373, 5: 0.359, 6: 0.368 ms
 
 // state planes -> action rows.  Persistent CTAs: the weights are converted once per CTA.
 template <int FIRST, int OBS, int ACT>
-__global__ void __launch_bounds__(128, COPTER_POLICY_CTAS_PER_SM)
+__global__ void __launch_bounds__(128, kPolicyCtasPerSm)
 copter_mlp_policy_kernel(const __grid_constant__ PolicyArgs a) {
     __shared__ __align__(16) PolicySmem sm;
     __shared__ __align__(16) PolicyWarpTile wtile[4];

@@ -5,20 +5,20 @@
 //   the MMA warp's elected lane issues the layer's MMAs (A = the tile's activations in shared memory,
 //   B = the layer's weights in shared memory, D = 128 x 64 fp32 in TMEM)  ->  tcgen05.commit on an mbarrier
 //   ->  every epilogue thread pulls ITS OWN row of D out of TMEM (tcgen05.ld 32x32b), applies tanh, rounds
-//   to 16 bits (fp16, COPTER_POLICY_TC_F16) and writes the row back to shared memory as the next layer's A operand  ->  mbarrier arrive.
+//   to fp16 and writes the row back to shared memory as the next layer's A operand  ->  mbarrier arrive.
 // The epilogue warps issue no MMA, no fragment loads and no bias adds (the biases ride along as one extra
 // K-step: a constant A tile of ones times a B tile holding each bias split into two 16-bit halves, hi + lo,
 // so the bias keeps ~16 bits).  What is left per env is 132 tanh + 66 packs + the TMEM loads; the floor is
 // the MUFU pipe, and because three quarters of the issue slots and the whole FMA pipe are free here, a
-// quarter of the hidden tanh are evaluated as a polynomial on the FMA pipe instead (COPTER_POLICY_TC_POLY).
+// quarter of the hidden tanh are evaluated as a polynomial on the FMA pipe instead (kPolyLanes).
 //
 // Operand layout: the canonical K-major, no-swizzle UMMA layout -- 8-row x 16-byte "core matrices" of
 // 128 contiguous bytes; core matrices adjacent in K are LBO = 128 B apart, 8-row groups SBO = (K/8) x
 // 128 B apart.  A thread writing its own 128-byte activation row therefore writes eight 16-byte chunks
 // 128 B apart; consecutive threads are 16 B apart inside a core matrix, so a warp's store is conflict-free.
-// TMEM: 64 accumulator columns per tile in flight (the 16 output columns of layer 3 reuse the hidden ones, see
-// col_out); with one tile in flight per CTA (64 columns allocated) up to eight CTAs could share an SM's 512
-// columns -- registers and shared memory allow five or six -- and overlap one another's phases.
+// TMEM: one tile in flight per CTA, 64 accumulator columns (the 16 output columns of layer 3 reuse the hidden ones,
+// see kColOut), so up to eight CTAs could share an SM's 512 columns -- registers and shared memory allow seven --
+// and overlap one another's phases.
 // Measured history and the A/B against the warp-MMA kernel (copter_policy.cuh): the comment on the kernel.
 #pragma once
 
@@ -30,24 +30,13 @@ namespace copter {
 namespace tc {
 
 constexpr int kTile = 128, kH = 64, kK1 = 16, kN3 = 16;
-#ifndef COPTER_POLICY_TC_SLOTS
-#define COPTER_POLICY_TC_SLOTS 1             // tiles in flight per CTA
-#endif
-constexpr int kSlots = COPTER_POLICY_TC_SLOTS;
-#ifndef COPTER_POLICY_TC_ONES_ROWS
-#define COPTER_POLICY_TC_ONES_ROWS 8
-#endif
-constexpr int kOnesRows = COPTER_POLICY_TC_ONES_ROWS;
-static_assert(kOnesRows == 8 || kOnesRows == 128, "the ones tile: one 8-row group read 16 times, or all 128 rows");
-constexpr uint32_t kOnesSBO = kOnesRows == 8 ? 0u : 256u;       // = (kK1 / 8) * 128 for the full tile
-static_assert(kSlots >= 1 && kSlots <= 4, "TMEM budget: 64 columns per slot, <= 256 columns per CTA");
-// TMEM columns of a CTA: 64 per slot.  The 16 output accumulator columns of layer 3 REUSE the first columns of the
-// slot's hidden accumulator: layer 3 is issued only after every epilogue thread has pulled its layer-2 row out of
-// TMEM (the ready barrier), and layer 1 of the next tile only after every thread has read its output columns.
-// 64 columns per tile instead of 128 is what lets more than four CTAs share an SM's 512 columns.
-constexpr uint32_t kTmemCols = kSlots == 1 ? 64 : (kSlots == 2 ? 128 : 256);          // tcgen05.alloc takes powers of two >= 32
-__host__ __device__ constexpr uint32_t col_hidden(int slot) { return 64u * slot; }
-__host__ __device__ constexpr uint32_t col_out(int slot) { return 64u * slot; }
+// TMEM columns of a CTA: 64.  The 16 output accumulator columns of layer 3 REUSE the first columns of the hidden
+// accumulator: layer 3 is issued only after every epilogue thread has pulled its layer-2 row out of TMEM (the ready
+// barrier), and layer 1 of the next tile only after every thread has read its output columns.  64 columns per tile
+// instead of 128 is what lets more than four CTAs share an SM's 512 columns.
+constexpr uint32_t kTmemCols = 64;                  // tcgen05.alloc takes powers of two >= 32
+constexpr uint32_t kColHidden = 0, kColOut = 0;
+constexpr uint32_t kOnesSBO = 0;                    // the ones tile: one 8-row group, read 16 times (Smem::ones)
 
 // element offset of (row r, column k) in a canonical K-major tile with KC = K/8 chunks per row
 __device__ __forceinline__ int canon(int r, int k, int KC) { return (((r >> 3) * KC + (k >> 3)) << 6) + ((r & 7) << 3) + (k & 7); }
@@ -65,13 +54,13 @@ struct alignas(128) Smem {
     __nv_bfloat16 b2[kH * kK1];          // layer 2 bias step [64 x 16] (column 0 = hi, 1 = lo)
     __nv_bfloat16 w3[kN3 * kH];          // layer 3 weights  [16 x 64]  (rows ACT.. are zero)
     __nv_bfloat16 b3[kN3 * kK1];         // layer 3 bias step [16 x 16]
-    // A tile of the bias steps: columns 0, 1 = 1.  All 128 rows are the same, so (COPTER_POLICY_TC_ONES_ROWS = 8) only ONE
-    // 8-row group is stored and the descriptor's stride between row groups is 0: 256 B instead of 4 KB, which is what
-    // lets a seventh CTA fit into an SM's shared memory.
-    __nv_bfloat16 ones[kOnesRows * kK1];
-    SlotSmem slot[kSlots];               // kSlots tiles in flight per CTA (see the kernel)
-    uint64_t done[kSlots];               // MMA warp -> epilogue warps: the slot's accumulator is complete (tcgen05.commit)
-    uint64_t ready[kSlots];              // epilogue threads -> MMA warp: the slot's next A tile is in shared memory (128 arrivals)
+    // A tile of the bias steps: columns 0, 1 = 1.  All 128 rows are the same, so only ONE 8-row group is stored and
+    // the descriptor's stride between row groups is 0 (kOnesSBO): 256 B instead of 4 KB, which is what lets a seventh
+    // CTA fit into an SM's shared memory.
+    __nv_bfloat16 ones[8 * kK1];
+    SlotSmem slot;                       // the tile in flight
+    uint64_t done;                       // MMA warp -> epilogue warps: the accumulator is complete (tcgen05.commit)
+    uint64_t ready;                      // epilogue threads -> MMA warp: the next A tile is in shared memory (128 arrivals)
     uint64_t clc_bar[2];                 // cluster launch control: response k has landed in clc_resp[k & 1] (see next_tile)
     alignas(16) uint4 clc_resp[2];
     uint32_t tmem_base;
@@ -84,18 +73,14 @@ __device__ __forceinline__ uint64_t make_desc(const void* tile, uint32_t lbo_byt
     return (uint64_t)((smem_addr(tile) >> 4) & 0x3FFFu) | ((uint64_t)(lbo_bytes >> 4) << 16) | ((uint64_t)(sbo_bytes >> 4) << 32) | (1ull << 46);
 }
 // instruction descriptor: D = fp32, A and B of one 16-bit format, both K-major, M = 128
-// COPTER_POLICY_TC_F16 != 0: the HIDDEN activations (the A operand of layers 2 and 3) are fp16 instead of bf16 -- three
-// more significand bits for values in [-1, 1]: the error against the fp64 network halves (max 0.0046 / mean 0.0007
-// instead of 0.0092 / 0.0016 on the microbenchmark's network).  1: tanh as before (two tanh.approx.f32 or two
-// polynomials, then one cvt.rn.f16x2.f32).  2: the MUFU share as `cvt.rn.f16x2.f32` + `tanh.approx.f16x2`, two issue
-// slots per pair instead of three -- measured SLOWER (0.275 vs 0.267 ms, profiles/r2_sweep_policy_tc_f16.txt: the packed
-// tanh costs the XU pipe its two slots and then some), kept as a knob.  The observation rows (layer 1's A operand, unbounded
-// magnitudes) and layer 1's weights stay bf16; the weights and bias tiles of layers 2 and 3 are fp16 as well (an MMA
-// whose descriptor mixes an fp16 A with a bf16 B raises "illegal instruction" on sm_100a: measured).
-#ifndef COPTER_POLICY_TC_F16
-#define COPTER_POLICY_TC_F16 1
-#endif
-constexpr bool kF16 = COPTER_POLICY_TC_F16 != 0, kPackedTanh = COPTER_POLICY_TC_F16 == 2;
+// The HIDDEN activations (the A operand of layers 2 and 3) are fp16, not bf16 -- three more significand bits for
+// values in [-1, 1]: the error against the fp64 network halves (max 0.0046 / mean 0.0007 instead of 0.0092 / 0.0016
+// on the microbenchmark's network).  A pair is two tanh.approx.f32 or two polynomials, then one cvt.rn.f16x2.f32; the
+// packed `cvt.rn.f16x2.f32` + `tanh.approx.f16x2` (two issue slots per pair instead of three) was measured SLOWER
+// (0.275 vs 0.267 ms, profiles/r2_sweep_policy_tc_f16.txt: the packed tanh costs the XU pipe its two slots and then
+// some; the knob is removed, the last tree that has it is commit d11af01).  The observation rows (layer 1's A operand,
+// unbounded magnitudes) and layer 1's weights stay bf16; the weights and bias tiles of layers 2 and 3 are fp16 as well
+// (an MMA whose descriptor mixes an fp16 A with a bf16 B raises "illegal instruction" on sm_100a: measured).
 // ab_bf16: format of the A and B operands (bits 7-9 and 10-12: 0 = fp16, 1 = bf16)
 __host__ __device__ constexpr uint32_t make_idesc(int n, bool ab_bf16 = true) { return (1u << 4) | ((ab_bf16 ? 1u : 0u) << 7) | ((ab_bf16 ? 1u : 0u) << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(kTile >> 4) << 24); }
 
@@ -116,32 +101,14 @@ __device__ __forceinline__ void bar_arrive(uint64_t* bar) {
 // Waiting warps must not eat the issue slots of the working ones: a warp's TMEM lane quarter ties it to the SM
 // sub-partition warp % 4, so the MMA warps of ALL resident CTAs (warp 4) sit on sub-partition 0, and a tight
 // try_wait loop there starves that sub-partition's epilogue warps -- whose tiles cannot finish before they do.
-// COPTER_POLICY_TC_WAIT: 0 = tight loop (try_wait's default, short suspension), 1 = try_wait with a suspend-time
-// hint (the thread sleeps in hardware until the phase completes or the hint expires), 2 = tight loop + __nanosleep.
-#ifndef COPTER_POLICY_TC_WAIT
-#define COPTER_POLICY_TC_WAIT 1
-#endif
-#ifndef COPTER_POLICY_TC_WAIT_NS
-#define COPTER_POLICY_TC_WAIT_NS 20000
-#endif
+// So try_wait carries a suspend-time hint: the thread sleeps in hardware until the phase completes or the hint
+// expires.  (A tight try_wait loop and a loop with __nanosleep were the alternatives; the last tree that has them is
+// commit d11af01.)
+constexpr uint32_t kWaitHintNs = 20000;
 __device__ __forceinline__ void bar_wait(uint64_t* bar, uint32_t parity) {
-#if COPTER_POLICY_TC_WAIT == 1
     asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\t"
                  "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-                 "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" :: "r"(smem_addr(bar)), "r"(parity), "r"((uint32_t)COPTER_POLICY_TC_WAIT_NS) : "memory");
-#elif COPTER_POLICY_TC_WAIT == 2
-    uint32_t ok = 0;
-    while (true) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(smem_addr(bar)), "r"(parity) : "memory");
-        if (ok) break;
-        __nanosleep(COPTER_POLICY_TC_WAIT_NS);
-    }
-#else
-    asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\t"
-                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                 "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" :: "r"(smem_addr(bar)), "r"(parity) : "memory");
-#endif
+                 "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" :: "r"(smem_addr(bar)), "r"(parity), "r"(kWaitHintNs) : "memory");
 }
 __device__ __forceinline__ void fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_after_sync()  { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -155,6 +122,10 @@ __device__ __forceinline__ bool elect_one() {
 }
 // Cluster launch control (sm_100): the grid holds one CTA per tile; a running CTA cancels a CTA that has not been
 // launched yet and takes over its block index.  The 16-byte response lands in shared memory through an mbarrier.
+// The warp scheduler favours the warps of the CTA that arrived first on an SM: with a static grid stride the first CTA
+// of an SM finished its 88 tiles after 469 000 cycles and the fifth after 611 000 (the launch's duration) -- with
+// stolen tiles every CTA works until the tiles run out.  (The grid-stride schedule: the last tree that has it is
+// commit d11af01.)
 __device__ __forceinline__ void clc_try_cancel(void* resp16, uint64_t* bar) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 16;" :: "r"(smem_addr(bar)) : "memory");
     asm volatile("clusterlaunchcontrol.try_cancel.async.shared::cta.mbarrier::complete_tx::bytes.b128 [%0], [%1];"
@@ -217,13 +188,6 @@ __device__ __forceinline__ float tanh_mufu(float x) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-// two hidden activations as one fp16 pair: rounded to fp16 first, one packed MUFU instruction
-__device__ __forceinline__ uint32_t tanh_pair_f16(float lo, float hi) {
-    uint32_t h, y;
-    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(h) : "f"(hi), "f"(lo));
-    asm("tanh.approx.f16x2 %0, %1;" : "=r"(y) : "r"(h));
-    return y;
-}
 __device__ __forceinline__ uint32_t pack2_f16(float lo, float hi) {
     uint32_t h;
     asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(h) : "f"(hi), "f"(lo));
@@ -234,20 +198,24 @@ __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
     return *reinterpret_cast<const uint32_t*>(&v);
 }
 
-// this thread's hidden accumulator row (64 columns of TMEM) -> tanh -> fp16 (bf16 without COPTER_POLICY_TC_F16) -> its row of the A tile.
+// this thread's hidden accumulator row (64 columns of TMEM) -> tanh -> fp16 -> its row of the A tile.
 // TMEM is read at 64 B per clock per SM (B300_MICROARCH.md): the 32 KB of a tile's hidden accumulator
 // take as long to read (512 cycles) as its 8192 tanh take on the four MUFU pipes, so the two must
 // overlap: the load of chunk q + 1 is in flight while the tanh of chunk q issue (tcgen05.wait::ld waits
 // for every outstanding load, so it is placed after the next load has been issued AND the previous
 // chunk's work is done -- by then the load has landed).
-// tanh on the FMA pipe: clamp to |x| <= 3.25 and evaluate the odd degree-13 polynomial x P(x^2) fitted in
-// tools/fit_tanh_poly.py (copter_policy.cuh: tanh_poly_coef; |error| <= 2.0e-3, inside the half-ulp of the bf16
-// rounding that follows).  In this kernel the warps issue no MMAs, so three quarters of the issue slots and
-// the whole FMA pipe are idle while the MUFU pipe is the floor: COPTER_POLICY_TC_POLY of every 16 hidden
+// tanh on the FMA pipe: clamp to |x| <= 3.25 and evaluate the odd degree-13 polynomial x P(x^2) (weighted minimax
+// fit, tools/fit_tanh_poly.py).  |error| <= 2.0e-3 absolute and <= 2.3e-3 relative, inside the half-ulp of the
+// 16-bit rounding that follows; MUFU.TANH is 5e-4.  In this kernel the warps issue no MMAs, so three quarters of
+// the issue slots and the whole FMA pipe are idle while the MUFU pipe is the floor: kPolyLanes of every 16 hidden
 // activations take this route (the FlashAttention-4 exp2 trick, applied to tanh).
-#ifndef COPTER_POLICY_TC_POLY
-#define COPTER_POLICY_TC_POLY 4         // measured, 2^23 envs: 0: 0.375 ms, 4: 0.344 ms, 6: 0.348 ms, 8: 0.380 ms (warp-MMA kernel: 0.358 ms)
-#endif
+constexpr float kTanhClamp = 3.25f;
+__host__ __device__ constexpr float tanh_poly_coef(int k) {    // coefficient of x^(2k+1)
+    constexpr float c[7] = {9.977270291e-01f, -3.117916466e-01f, 9.229137325e-02f, -1.838625564e-02f,
+                            2.184749761e-03f, -1.380842544e-04f, 3.552717362e-06f};
+    return c[k];
+}
+constexpr int kPolyLanes = 4;         // measured, 2^23 envs: 0: 0.375 ms, 4: 0.344 ms, 6: 0.348 ms, 8: 0.380 ms (warp-MMA kernel: 0.358 ms)
 __device__ __forceinline__ float tanh_fma(float x) {
     x = fminf(fmaxf(x, -kTanhClamp), kTanhClamp);
     const float u = x * x;
@@ -258,42 +226,31 @@ __device__ __forceinline__ float tanh_fma(float x) {
 }
 // PIPELINED: the load of chunk q + 1 is in flight under the tanh of chunk q (two 16-register buffers); without it
 // one buffer, each load awaited before use (16 registers fewer: the fused rollout kernel, which also holds an env).
-template <int NCHUNK, bool PIPELINED = true>      // NCHUNK chunks of 16 columns starting at column col0 (the row's 64 columns may be split between two threads)
-__device__ __forceinline__ void hidden_epilogue(uint32_t taddr_row, __nv_bfloat16* a_tile, int row, int col0, int trace_round = 0, int trace_event = 0) {
+template <bool PIPELINED>      // the row's 4 chunks of 16 columns
+__device__ __forceinline__ void hidden_epilogue(uint32_t taddr_row, __nv_bfloat16* a_tile, int row, int trace_round = 0, int trace_event = 0) {
+    constexpr int kChunks = kH / 16;
     uint32_t r[PIPELINED ? 2 : 1][16];
-    tmem_ld16(taddr_row + col0, r[0]);
+    tmem_ld16(taddr_row, r[0]);
 #pragma unroll
-    for (int q = 0; q < NCHUNK; ++q) {
+    for (int q = 0; q < kChunks; ++q) {
         tmem_wait();                                               // chunk q has landed
         TC_TRACE((threadIdx.x & 31) == 0, (threadIdx.x >> 5) & 3, trace_round, trace_event + 2 * q);
         constexpr int kMask = PIPELINED ? 1 : 0;
-        if (PIPELINED && q + 1 < NCHUNK) tmem_ld16(taddr_row + col0 + 16 * (q + 1), r[(q + 1) & kMask]);
-        uint32_t w[8];
-        if constexpr (kPackedTanh) {
-            // pair p = columns 2p, 2p + 1; COPTER_POLICY_TC_POLY / 2 of the 8 pairs take the polynomial, spread over the chunk
+        if (PIPELINED && q + 1 < kChunks) tmem_ld16(taddr_row + 16 * (q + 1), r[(q + 1) & kMask]);
+        float y[16];
 #pragma unroll
-            for (int p = 0; p < 8; ++p) {
-                const float x0 = __uint_as_float(r[q & kMask][2 * p]), x1 = __uint_as_float(r[q & kMask][2 * p + 1]);
-                constexpr int kPolyPairs = COPTER_POLICY_TC_POLY / 2;
-                const bool poly = kPolyPairs > 0 && ((p * kPolyPairs) % 8) < kPolyPairs;
-                w[p] = poly ? pack2_f16(tanh_fma(x0), tanh_fma(x1)) : tanh_pair_f16(x0, x1);
-            }
-            if (!PIPELINED && q + 1 < NCHUNK) tmem_ld16(taddr_row + col0 + 16 * (q + 1), r[0]);      // r[0] is dead: lands under the stores
-        } else {
-            float y[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-                const float x = __uint_as_float(r[q & kMask][j]);
-                // the polynomial lanes are spread over the chunk so that the two pipes interleave
-                const bool poly = COPTER_POLICY_TC_POLY > 0 && ((j * COPTER_POLICY_TC_POLY) % 16) < COPTER_POLICY_TC_POLY;
-                y[j] = poly ? tanh_fma(x) : tanh_mufu(x);
-            }
-            if (!PIPELINED && q + 1 < NCHUNK) tmem_ld16(taddr_row + col0 + 16 * (q + 1), r[0]);      // r[0] is dead: lands under the packs and stores
-#pragma unroll
-            for (int j = 0; j < 8; ++j) w[j] = kF16 ? pack2_f16(y[2 * j], y[2 * j + 1]) : pack2(y[2 * j], y[2 * j + 1]);
+        for (int j = 0; j < 16; ++j) {
+            const float x = __uint_as_float(r[q & kMask][j]);
+            // the polynomial lanes are spread over the chunk so that the two pipes interleave
+            const bool poly = ((j * kPolyLanes) % 16) < kPolyLanes;
+            y[j] = poly ? tanh_fma(x) : tanh_mufu(x);
         }
-        *reinterpret_cast<uint4*>(a_tile + canon(row, col0 + 16 * q, kH / 8)) = make_uint4(w[0], w[1], w[2], w[3]);
-        *reinterpret_cast<uint4*>(a_tile + canon(row, col0 + 16 * q + 8, kH / 8)) = make_uint4(w[4], w[5], w[6], w[7]);
+        if (!PIPELINED && q + 1 < kChunks) tmem_ld16(taddr_row + 16 * (q + 1), r[0]);      // r[0] is dead: lands under the packs and stores
+        uint32_t w[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) w[j] = pack2_f16(y[2 * j], y[2 * j + 1]);
+        *reinterpret_cast<uint4*>(a_tile + canon(row, 16 * q, kH / 8)) = make_uint4(w[0], w[1], w[2], w[3]);
+        *reinterpret_cast<uint4*>(a_tile + canon(row, 16 * q + 8, kH / 8)) = make_uint4(w[4], w[5], w[6], w[7]);
         TC_TRACE((threadIdx.x & 31) == 0, (threadIdx.x >> 5) & 3, trace_round, trace_event + 2 * q + 1);
     }
 }
@@ -304,15 +261,12 @@ __device__ __forceinline__ void hidden_epilogue(uint32_t taddr_row, __nv_bfloat1
 template <int OBS, int ACT>
 __device__ __forceinline__ void load_weights(Smem& sm, const float* w1, const float* b1, const float* w2, const float* b2,
                                              const float* w3, const float* b3) {
-    const __nv_bfloat16 zero = __float2bfloat16(0.0f), one = __float2bfloat16(1.0f);
+    const __nv_bfloat16 zero = __float2bfloat16(0.0f);
     auto hi = [](float b) { return __float2bfloat16(b); };
     auto lo = [](float b) { return __float2bfloat16(b - __bfloat162float(__float2bfloat16(b))); };
-    // layers 2 and 3: the operand format of the hidden activations (fp16 bit patterns in the same 16-bit tiles when kF16)
-    auto hid = [](float v) { return kF16 ? __ushort_as_bfloat16(__half_as_ushort(__float2half_rn(v))) : __float2bfloat16(v); };
-    auto hid_lo = [](float b) {
-        return kF16 ? __ushort_as_bfloat16(__half_as_ushort(__float2half_rn(b - __half2float(__float2half_rn(b)))))
-                    : __float2bfloat16(b - __bfloat162float(__float2bfloat16(b)));
-    };
+    // layers 2 and 3: the operand format of the hidden activations (fp16 bit patterns in the same 16-bit tiles)
+    auto hid = [](float v) { return __ushort_as_bfloat16(__half_as_ushort(__float2half_rn(v))); };
+    auto hid_lo = [](float b) { return __ushort_as_bfloat16(__half_as_ushort(__float2half_rn(b - __half2float(__float2half_rn(b))))); };
     constexpr int kWBatch = 8;
     const int tid = threadIdx.x, nt = blockDim.x;
     for (int base = 0; base < kH * kH; base += kWBatch * nt) {
@@ -352,9 +306,9 @@ __device__ __forceinline__ void load_weights(Smem& sm, const float* w1, const fl
 #pragma unroll
         for (int k = 0; k < kK1; ++k) sm.b3[canon(tid, k, kK1 / 8)] = (tid < ACT && k == 0) ? hid(vb3) : ((tid < ACT && k == 1) ? hid_lo(vb3) : zero);
     }
-    for (int e = tid; e < kOnesRows * kK1; e += nt) {
+    for (int e = tid; e < 8 * kK1; e += nt) {
         const int r = e / kK1, k = e % kK1;
-        sm.ones[canon(r, k, kK1 / 8)] = k < 2 ? (kF16 ? __ushort_as_bfloat16((unsigned short)0x3C00u) : one) : zero;     // 1.0 in the hidden A format (fp16: 0x3C00)
+        sm.ones[canon(r, k, kK1 / 8)] = k < 2 ? __ushort_as_bfloat16((unsigned short)0x3C00u) : zero;     // 1.0 in the hidden A format (fp16: 0x3C00)
     }
 }
 
@@ -365,43 +319,19 @@ struct Args {
     float* action;                                   // [n][ACT]
 };
 
-// One elected thread issues the MMAs of layer `layer` (1..3) of a slot and commits them to the slot's mbarrier.
-__device__ __forceinline__ void issue_layer(Smem& sm, int slot, int layer, uint32_t tmem_base) {
-    constexpr uint32_t kLBO = 128, kSBO16 = (kK1 / 8) * 128, kSBO64 = (kH / 8) * 128, kStep = 256;   // one K = 16 step = two chunks
-    constexpr uint32_t idesc1 = make_idesc(kH), idesc64 = make_idesc(kH, !kF16), idesc16 = make_idesc(kN3, !kF16);
-    SlotSmem& ss = sm.slot[slot];
-    fence_after_sync();
-    if (layer == 1) {            // D[128 x 64] = A1[128 x 16] W1^T (bias in columns 14, 15)
-        mma_bf16(tmem_base + col_hidden(slot), make_desc(ss.a1(), kLBO, kSBO16), make_desc(sm.w1, kLBO, kSBO16), idesc1, 0u);
-    } else if (layer == 2) {     // D[128 x 64] = A[128 x 64] W2^T + ones b2^T
-#pragma unroll
-        for (int j = 0; j < kH / 16; ++j)
-            mma_bf16(tmem_base + col_hidden(slot), make_desc(reinterpret_cast<const char*>(ss.a) + j * kStep, kLBO, kSBO64),
-                     make_desc(reinterpret_cast<const char*>(sm.w2) + j * kStep, kLBO, kSBO64), idesc64, j > 0 ? 1u : 0u);
-        mma_bf16(tmem_base + col_hidden(slot), make_desc(sm.ones, kLBO, kOnesSBO), make_desc(sm.b2, kLBO, kSBO16), idesc64, 1u);
-    } else {                     // D[128 x 16] = A[128 x 64] W3^T + ones b3^T
-#pragma unroll
-        for (int j = 0; j < kH / 16; ++j)
-            mma_bf16(tmem_base + col_out(slot), make_desc(reinterpret_cast<const char*>(ss.a) + j * kStep, kLBO, kSBO64),
-                     make_desc(reinterpret_cast<const char*>(sm.w3) + j * kStep, kLBO, kSBO64), idesc16, j > 0 ? 1u : 0u);
-        mma_bf16(tmem_base + col_out(slot), make_desc(sm.ones, kLBO, kOnesSBO), make_desc(sm.b3, kLBO, kSBO16), idesc16, 1u);
-    }
-    mma_commit(&sm.done[slot]);
-}
-
-// The same for a warp-uniform MMA warp: every descriptor of a slot is built once, outside the elected branch, so the
-// compiler keeps them in uniform registers; the elected lane then issues a layer's MMAs and the commit back to back.
-// (Issued from inside an `if (lane == 0)` branch, each MMA was preceded by R2UR moves and descriptor arithmetic: the
-// timeline of tools/microbench/policy_tc_trace.cu showed 250 / 570 / 600 cycles to ISSUE layers 1 / 2 / 3 -- 28 % of
-// a tile's 5100-cycle chain.)
+// The MMA warp runs warp-uniformly: every descriptor is built once, outside the elected branch, so the compiler keeps
+// them in uniform registers; the elected lane then issues a layer's MMAs and the commit back to back.  (Issued from
+// inside an `if (lane == 0)` branch, each MMA was preceded by R2UR moves and descriptor arithmetic: the timeline of
+// tools/microbench/policy_tc_trace.cu showed 250 / 570 / 600 cycles to ISSUE layers 1 / 2 / 3 -- 28 % of a tile's
+// 5100-cycle chain.)
 struct LayerDescs {
     uint64_t a1, w1, a[kH / 16], w2[kH / 16], ones, b2, w3[kH / 16], b3;
     uint32_t d_hidden, d_out;
 };
-__device__ __forceinline__ LayerDescs make_layer_descs(Smem& sm, int slot, uint32_t tmem_base) {
-    constexpr uint32_t kLBO = 128, kSBO16 = (kK1 / 8) * 128, kSBO64 = (kH / 8) * 128, kStep = 256;
+__device__ __forceinline__ LayerDescs make_layer_descs(Smem& sm, uint32_t tmem_base) {
+    constexpr uint32_t kLBO = 128, kSBO16 = (kK1 / 8) * 128, kSBO64 = (kH / 8) * 128, kStep = 256;   // one K = 16 step = two chunks
     LayerDescs d;
-    SlotSmem& ss = sm.slot[slot];
+    SlotSmem& ss = sm.slot;
     d.a1 = make_desc(ss.a1(), kLBO, kSBO16); d.w1 = make_desc(sm.w1, kLBO, kSBO16);
 #pragma unroll
     for (int j = 0; j < kH / 16; ++j) {
@@ -410,20 +340,21 @@ __device__ __forceinline__ LayerDescs make_layer_descs(Smem& sm, int slot, uint3
         d.w3[j] = make_desc(reinterpret_cast<const char*>(sm.w3) + j * kStep, kLBO, kSBO64);
     }
     d.ones = make_desc(sm.ones, kLBO, kOnesSBO); d.b2 = make_desc(sm.b2, kLBO, kSBO16); d.b3 = make_desc(sm.b3, kLBO, kSBO16);
-    d.d_hidden = tmem_base + col_hidden(slot); d.d_out = tmem_base + col_out(slot);
+    d.d_hidden = tmem_base + kColHidden; d.d_out = tmem_base + kColOut;
     return d;
 }
+// the MMAs of layer `layer` (1..3), committed to `done`
 __device__ __forceinline__ void issue_layer_uniform(const LayerDescs& d, int layer, uint64_t* done) {     // whole warp, converged
-    constexpr uint32_t idesc1 = make_idesc(kH), idesc64 = make_idesc(kH, !kF16), idesc16 = make_idesc(kN3, !kF16);
+    constexpr uint32_t idesc1 = make_idesc(kH), idesc64 = make_idesc(kH, false), idesc16 = make_idesc(kN3, false);
     fence_after_sync();
     if (elect_one()) {
-        if (layer == 1) {
+        if (layer == 1) {            // D[128 x 64] = A1[128 x 16] W1^T (bias in columns 14, 15)
             mma_bf16(d.d_hidden, d.a1, d.w1, idesc1, 0u);
-        } else if (layer == 2) {
+        } else if (layer == 2) {     // D[128 x 64] = A[128 x 64] W2^T + ones b2^T
 #pragma unroll
             for (int j = 0; j < kH / 16; ++j) mma_bf16(d.d_hidden, d.a[j], d.w2[j], idesc64, j > 0 ? 1u : 0u);
             mma_bf16(d.d_hidden, d.ones, d.b2, idesc64, 1u);
-        } else {
+        } else {                     // D[128 x 16] = A[128 x 64] W3^T + ones b3^T
 #pragma unroll
             for (int j = 0; j < kH / 16; ++j) mma_bf16(d.d_out, d.a[j], d.w3[j], idesc16, j > 0 ? 1u : 0u);
             mma_bf16(d.d_out, d.ones, d.b3, idesc16, 1u);
@@ -459,52 +390,28 @@ __device__ __forceinline__ void tmem_free(uint32_t base) {     // warp 0, conver
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(base), "n"(kTmemCols) : "memory");
 }
 
-#ifndef COPTER_POLICY_TC_SPLIT
-#define COPTER_POLICY_TC_SPLIT 1             // epilogue threads per env row: 1, or 2 (each takes 32 of the 64 hidden columns)
-#endif
-#ifndef COPTER_POLICY_TC_CTAS_PER_SM
-#define COPTER_POLICY_TC_CTAS_PER_SM (COPTER_POLICY_TC_SLOTS == 1 ? (COPTER_POLICY_TC_SPLIT == 1 ? 7 : 3) : 2)   // x kTmemCols <= the SM's 512 TMEM columns
-#endif
-// Tile scheduling of the one-tile-in-flight shape: 1 = cluster launch control (grid = one CTA per tile; a resident CTA
-// cancels a pending one and takes over its tile), 0 = static grid stride.  The warp scheduler favours the warps of the
-// CTA that arrived first on an SM: with a static split the first CTA of an SM finished its 88 tiles after 469 000 cycles
-// and the fifth after 611 000 (the launch's duration) -- with stolen tiles every CTA works until the tiles run out.
-#ifndef COPTER_POLICY_TC_CLC
-#define COPTER_POLICY_TC_CLC 1
-#endif
-constexpr int kSplit = COPTER_POLICY_TC_SPLIT;
-constexpr bool kSimple = COPTER_POLICY_TC_SLOTS == 1 && COPTER_POLICY_TC_SPLIT == 1;      // the shipped shape: its own, leaner loop
-constexpr bool kClc = kSimple && COPTER_POLICY_TC_CLC != 0;
+constexpr int kCtasPerSm = 7;                       // x kTmemCols <= the SM's 512 TMEM columns
 // Tile k + 1 of a CTA (tile 0 is blockIdx.x): the answer to try_cancel k, read by every thread of both roles from
-// clc_resp[k & 1] once clc_bar[k & 1] has completed -- or, without cluster launch control, a grid stride.
-__device__ __forceinline__ uint32_t next_tile(Smem& sm, int k, uint32_t cur, uint32_t& clc_phase, int64_t n_tiles) {
-    if constexpr (kClc) {
-        bar_wait(&sm.clc_bar[k & 1], (clc_phase >> (k & 1)) & 1u); clc_phase ^= 1u << (k & 1);
-        return clc_response(&sm.clc_resp[k & 1]);
-    } else {
-        return (int64_t)cur + gridDim.x < n_tiles ? cur + gridDim.x : kNoTile;
-    }
+// clc_resp[k & 1] once clc_bar[k & 1] has completed.
+__device__ __forceinline__ uint32_t next_tile(Smem& sm, int k, uint32_t& clc_phase) {
+    bar_wait(&sm.clc_bar[k & 1], (clc_phase >> (k & 1)) & 1u); clc_phase ^= 1u << (k & 1);
+    return clc_response(&sm.clc_resp[k & 1]);
 }
 // the MMA warp (converged): ask for the tile after next -- answer k + 1 -- unless answer k was "nothing left"
 __device__ __forceinline__ void request_tile(Smem& sm, int k_next) {
-    if constexpr (kClc) {
-        if (elect_one()) { fence_async_smem(); clc_try_cancel(&sm.clc_resp[k_next & 1], &sm.clc_bar[k_next & 1]); }
-        __syncwarp();
-    }
+    if (elect_one()) { fence_async_smem(); clc_try_cancel(&sm.clc_resp[k_next & 1], &sm.clc_bar[k_next & 1]); }
+    __syncwarp();
 }
-constexpr int kEpilogueThreads = kTile * kSplit;
-constexpr int kThreads = kEpilogueThreads + 32;      // the epilogue warps + the MMA warp
+constexpr int kThreads = kTile + 32;      // the epilogue warps + the MMA warp
 
 // state planes -> action rows.  Persistent, warp-specialised CTAs (weights converted once per CTA), 128 envs
-// per tile, kSlots tiles in flight per CTA.
-//   epilogue warps   kSplit threads per env row (a warp may only touch the TMEM lanes 32 (warp % 4) .. + 31, so
-//              with kSplit = 2 warps w and w + 4 share a lane quarter and split the 64 hidden columns): pull
-//              the accumulator out of TMEM, tanh, bf16, write it to shared memory as the next layer's A
-//              operand, arrive on ready[slot]; after layer 3 the first thread of a row stores its action
-//              and puts the NEXT tile's observation row in place.  They never wait for one another: the only
-//              thing a thread waits for is done[slot] of the layer it is about to read.
-//   last warp  one elected lane: waits for ready[slot] (all epilogue threads), issues the layer's
-//              tcgen05.mma, commits them to done[slot].
+// per tile, one tile in flight per CTA, the tiles taken by cluster launch control (next_tile).
+//   epilogue warps   one thread per env row: pull the accumulator out of TMEM, tanh, fp16, write it to shared
+//              memory as the next layer's A operand, arrive on ready; after layer 3 store the env's action and
+//              put the NEXT tile's observation row in place.  They never wait for one another: the only thing
+//              a thread waits for is done of the layer it is about to read.
+//   last warp  warp-uniform, one elected lane issuing: waits for ready (all epilogue threads), issues the
+//              layer's tcgen05.mma, commits them to done.
 // The MUFU pipe is the floor (132 tanh per env) and what keeps it busy is WARPS: every wait in an epilogue
 // warp (mbarrier, TMEM load, shared-memory fence) has to be covered by another warp's tanh.
 // History, 2^23 envs (warp-MMA kernel of copter_policy.cuh: 0.358 ms, XU 72 %):
@@ -519,17 +426,19 @@ constexpr int kThreads = kEpilogueThreads + 32;      // the epilogue warps + the
 //   6 of 16 tanh as polynomials 0.330, 8 of 16 0.355 (profiles/r2_sweep_policy_tc_ctas.txt)
 //   (tools/microbench/tmem_rates.cu, profiles/r2_tmem_rates.txt: TMEM read-back is NOT the floor -- 184 B/clk/SM from
 //   one CTA, 370 B/clk/SM from four, and tcgen05.ld overlaps tanh.approx completely; the MUFU floor is 0.19 ms)
+// (The loop with several tiles in flight per CTA or two epilogue threads per row: the last tree that has it is
+// commit d11af01.)
 template <int FIRST, int OBS, int ACT>
-__global__ void __launch_bounds__(kThreads, COPTER_POLICY_TC_CTAS_PER_SM)
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
 copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     static_assert(OBS <= 12 && ACT <= 4, "tile shapes");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
     const int t = threadIdx.x, warp = t >> 5;
-    constexpr int kMmaWarp = kEpilogueThreads / 32;
+    constexpr int kMmaWarp = kTile / 32;
     TC_TRACE_CTA(0);
     if (t == 0) {
-        for (int q = 0; q < kSlots; ++q) { bar_init(&sm.done[q], 1); bar_init(&sm.ready[q], kEpilogueThreads); }
+        bar_init(&sm.done, 1); bar_init(&sm.ready, kTile);
         bar_init(&sm.clc_bar[0], 1); bar_init(&sm.clc_bar[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -541,188 +450,87 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     fence_after_sync();
     TC_TRACE_CTA(1);
     const uint32_t tmem_base = sm.tmem_base;
-    const int64_t n_tiles = (a.n + kTile - 1) / kTile;
-    // slot s works through tiles blockIdx.x + (kSlots r + s) gridDim.x, r = 0, 1, ...: both roles walk the same sequence
-    const int64_t stride = kSlots * (int64_t)gridDim.x;
-    auto any = [](const int (&l)[kSlots]) { int v = 0; for (int q = 0; q < kSlots; ++q) v |= l[q]; return v != 0; };
 
-    if constexpr (kSimple) {
-        // ===== one tile in flight per CTA, one epilogue thread per env row =====
-        // Tile k of this CTA: k = 0 is blockIdx.x; tile k + 1 is the answer to try_cancel k (CLC) or tile k + gridDim.x.
-        // The MMA warp keeps one try_cancel in flight; both roles read answer k from clc_resp[k & 1] after clc_bar[k & 1]
-        // -- the epilogue threads after they have handed layer 2 its A tile, i.e. while they would only wait -- and
-        // clc_resp[k & 1] is re-armed (try_cancel k + 2) only after every epilogue thread has arrived for layer 1 of tile
-        // k + 1, which it does after that read.
-        if (warp == kMmaWarp) {
-            const LayerDescs d = make_layer_descs(sm, 0, tmem_base);
-            uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
-            request_tile(sm, 0);
-            for (int k = 0; tile != kNoTile; ++k) {
-                bar_wait(&sm.ready[0], phase); phase ^= 1u;
-                TC_TRACE((t & 31) == 0, 4, k, 0);
-                issue_layer_uniform(d, 1, &sm.done[0]);
-                TC_TRACE((t & 31) == 0, 4, k, 2);
-                const uint32_t nxt = next_tile(sm, k, tile, clc_phase, n_tiles);
-                if (nxt != kNoTile) request_tile(sm, k + 1);          // (a failed try_cancel is the last one)
-#pragma unroll
-                for (int layer = 2; layer <= 3; ++layer) {
-                    bar_wait(&sm.ready[0], phase); phase ^= 1u;
-                    TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1));
-                    issue_layer_uniform(d, layer, &sm.done[0]);
-                    TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1) + 2);
-                }
-                tile = nxt;
-            }
-        } else {
-            const int row = t;
-            const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);       // this warp's quarter of the 128 TMEM lanes
-            const float4* planes = reinterpret_cast<const float4*>(a.state);
-            auto fetch = [&](uint32_t tl, float4 (&p)[3]) {
-                const int64_t i = (int64_t)tl * kTile + row;
-                if (tl != kNoTile && i < a.n) { p[0] = planes[i]; p[1] = planes[a.stride + i]; p[2] = planes[2 * a.stride + i]; }
-                else p[0] = p[1] = p[2] = make_float4(0.f, 0.f, 0.f, 0.f);
-            };
-            uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
-            float4 nxt[3];
-            fetch(tile, nxt);
-            write_obs_row<FIRST, OBS>(sm.slot[0], row, nxt);
-            fence_before_sync();
-            bar_arrive(&sm.ready[0]);
-            for (int k = 0; tile != kNoTile; ++k) {
-                uint32_t nxt_tile = kNoTile;
-#pragma unroll
-                for (int layer = 1; layer <= 2; ++layer) {
-                    bar_wait(&sm.done[0], phase); phase ^= 1u;
-                    fence_after_sync();
-                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1));
-                    hidden_epilogue<4>(lane_base + col_hidden(0), sm.slot[0].a, row, 0, k, 12 + 8 * (layer - 1));      // (layer 2 overwrites the tile its finished MMAs read)
-                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 1);
-                    fence_async_smem();
-                    fence_before_sync();
-                    bar_arrive(&sm.ready[0]);
-                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 2);
-                    if (layer == 1) {                                    // under layer 2's MMAs: which tile is next, and its state on the way
-                        nxt_tile = next_tile(sm, k, tile, clc_phase, n_tiles);
-                        fetch(nxt_tile, nxt);
-                    }
-                }
-                bar_wait(&sm.done[0], phase); phase ^= 1u;
-                fence_after_sync();
-                TC_TRACE((t & 31) == 0, warp, k, 6);
-                float pre[4];
-                tmem_ld4(lane_base + col_out(0), pre);
-                TC_TRACE((t & 31) == 0, warp, k, 7);
-                if (nxt_tile != kNoTile) {                               // the next tile's observation row first: the MMA warp is waiting for it
-                    write_obs_row<FIRST, OBS>(sm.slot[0], row, nxt);
-                    fence_before_sync();
-                    bar_arrive(&sm.ready[0]);
-                    TC_TRACE((t & 31) == 0, warp, k, 8);
-                }
-                const int64_t i = (int64_t)tile * kTile + row;
-                if (i < a.n) {
-                    float act[4];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) act[j] = fmaf(a.out_scale, tanh_mufu(pre[j]), a.out_offset);
-                    if constexpr (ACT == 4) reinterpret_cast<float4*>(a.action)[i] = make_float4(act[0], act[1], act[2], act[3]);
-                    else if constexpr (ACT == 2) reinterpret_cast<float2*>(a.action)[i] = make_float2(act[0], act[1]);
-                    else a.action[i] = act[0];
-                }
-                tile = nxt_tile;
-            }
-        }
-    } else
+    // Tile k of this CTA: k = 0 is blockIdx.x; tile k + 1 is the answer to try_cancel k.
+    // The MMA warp keeps one try_cancel in flight; both roles read answer k from clc_resp[k & 1] after clc_bar[k & 1]
+    // -- the epilogue threads after they have handed layer 2 its A tile, i.e. while they would only wait -- and
+    // clc_resp[k & 1] is re-armed (try_cancel k + 2) only after every epilogue thread has arrived for layer 1 of tile
+    // k + 1, which it does after that read.
     if (warp == kMmaWarp) {
-        // ===== MMA issuer =====
-        if ((t & 31) == 0) {
-            int64_t tile[kSlots];
-            int rnd[kSlots] = {};                                                         // tiles done by the slot (trace builds)
-            int layer[kSlots];                                                            // the layer to issue next
-            uint32_t phase[kSlots];
+        const LayerDescs d = make_layer_descs(sm, tmem_base);
+        uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
+        request_tile(sm, 0);
+        for (int k = 0; tile != kNoTile; ++k) {
+            bar_wait(&sm.ready, phase); phase ^= 1u;
+            TC_TRACE((t & 31) == 0, 4, k, 0);
+            issue_layer_uniform(d, 1, &sm.done);
+            TC_TRACE((t & 31) == 0, 4, k, 2);
+            const uint32_t nxt = next_tile(sm, k, clc_phase);
+            if (nxt != kNoTile) request_tile(sm, k + 1);          // (a failed try_cancel is the last one)
 #pragma unroll
-            for (int s = 0; s < kSlots; ++s) { tile[s] = (int64_t)blockIdx.x + s * (int64_t)gridDim.x; layer[s] = tile[s] < n_tiles ? 1 : 0; phase[s] = 0; }
-            while (any(layer)) {
-#pragma unroll
-                for (int s = 0; s < kSlots; ++s) {
-                    if (layer[s] == 0) continue;
-                    bar_wait(&sm.ready[s], phase[s]); phase[s] ^= 1u;
-                    TC_TRACE(true, 4, rnd[s], 3 * (layer[s] - 1));
-                    issue_layer(sm, s, layer[s], tmem_base);
-                    TC_TRACE(true, 4, rnd[s], 3 * (layer[s] - 1) + 2);
-                    if (layer[s] < 3) ++layer[s];
-                    else { tile[s] += stride; ++rnd[s]; layer[s] = tile[s] < n_tiles ? 1 : 0; }
-                }
+            for (int layer = 2; layer <= 3; ++layer) {
+                bar_wait(&sm.ready, phase); phase ^= 1u;
+                TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1));
+                issue_layer_uniform(d, layer, &sm.done);
+                TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1) + 2);
             }
+            tile = nxt;
         }
     } else {
-        // ===== epilogue warps: thread <-> (env row, column half) <-> TMEM lane `row` =====
-        const int row = t & (kTile - 1), half = t / kTile;                          // half is warp-uniform
-        const bool owner = half == 0;                                               // holds the env's state, writes its observation row, stores its action
-        const uint32_t lane_base = tmem_base + ((uint32_t)((warp & 3) * 32) << 16); // this warp's quarter of the 128 TMEM lanes
+        const int row = t;
+        const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);       // this warp's quarter of the 128 TMEM lanes
         const float4* planes = reinterpret_cast<const float4*>(a.state);
-        auto fetch = [&](int64_t tl, float4 (&p)[3]) {
-            const int64_t i = tl * kTile + row;
-            if (owner && tl < n_tiles && i < a.n) { p[0] = planes[i]; p[1] = planes[a.stride + i]; p[2] = planes[2 * a.stride + i]; }
+        auto fetch = [&](uint32_t tl, float4 (&p)[3]) {
+            const int64_t i = (int64_t)tl * kTile + row;
+            if (tl != kNoTile && i < a.n) { p[0] = planes[i]; p[1] = planes[a.stride + i]; p[2] = planes[2 * a.stride + i]; }
             else p[0] = p[1] = p[2] = make_float4(0.f, 0.f, 0.f, 0.f);
         };
-        int64_t tile[kSlots];
-        int rnd[kSlots] = {};                   // tiles done by the slot (trace builds)
-        int layer[kSlots];                      // the layer whose result this thread reads next (0: the slot has run out of tiles)
-        uint32_t phase[kSlots];
-        float4 nxt[kSlots][3];
+        uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
+        float4 nxt[3];
+        fetch(tile, nxt);
+        write_obs_row<FIRST, OBS>(sm.slot, row, nxt);
+        fence_before_sync();
+        bar_arrive(&sm.ready);
+        for (int k = 0; tile != kNoTile; ++k) {
+            uint32_t nxt_tile = kNoTile;
 #pragma unroll
-        for (int s = 0; s < kSlots; ++s) {
-            tile[s] = (int64_t)blockIdx.x + s * (int64_t)gridDim.x; layer[s] = 0; phase[s] = 0;
-            fetch(tile[s], nxt[s]);
-            if (tile[s] < n_tiles) {
-                if (owner) write_obs_row<FIRST, OBS>(sm.slot[s], row, nxt[s]);
-                fence_before_sync();
-                bar_arrive(&sm.ready[s]);
-                layer[s] = 1;
-                fetch(tile[s] + stride, nxt[s]);                // arrives under the three layers
-            }
-        }
-        while (any(layer)) {
-#pragma unroll
-            for (int s = 0; s < kSlots; ++s) {
-                if (layer[s] == 0) continue;
-                bar_wait(&sm.done[s], phase[s]); phase[s] ^= 1u;
+            for (int layer = 1; layer <= 2; ++layer) {
+                bar_wait(&sm.done, phase); phase ^= 1u;
                 fence_after_sync();
-                TC_TRACE((t & 31) == 0, warp & 3, rnd[s], 3 * (layer[s] - 1));
-                if (layer[s] < 3) {
-                    // (layer 2 overwrites the tile its finished MMAs read)
-                    hidden_epilogue<4 / kSplit>(lane_base + col_hidden(s), sm.slot[s].a, row, half * (kH / kSplit), rnd[s], 12 + 8 * (layer[s] - 1));
-                    TC_TRACE((t & 31) == 0, warp & 3, rnd[s], 3 * (layer[s] - 1) + 1);
-                    fence_async_smem();
-                    fence_before_sync();
-                    bar_arrive(&sm.ready[s]);
-                    TC_TRACE((t & 31) == 0, warp & 3, rnd[s], 3 * (layer[s] - 1) + 2);
-                    ++layer[s];
-                } else {
-                    float pre[4] = {0.f, 0.f, 0.f, 0.f};
-                    if (owner) tmem_ld4(lane_base + col_out(s), pre);
-                    const int64_t i = tile[s] * kTile + row;
-                    TC_TRACE((t & 31) == 0, warp & 3, rnd[s], 7);
-                    tile[s] += stride; ++rnd[s];
-                    if (tile[s] < n_tiles) {                                       // the next tile's observation row first: the MMA warp is waiting for it
-                        if (owner) write_obs_row<FIRST, OBS>(sm.slot[s], row, nxt[s]);
-                        fence_before_sync();
-                        bar_arrive(&sm.ready[s]);
-                        TC_TRACE((t & 31) == 0, warp & 3, rnd[s] - 1, 8);
-                        layer[s] = 1;
-                        fetch(tile[s] + stride, nxt[s]);
-                    } else {
-                        layer[s] = 0;
-                    }
-                    if (owner && i < a.n) {
-                        float act[4];
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) act[j] = fmaf(a.out_scale, tanh_mufu(pre[j]), a.out_offset);
-                        if constexpr (ACT == 4) reinterpret_cast<float4*>(a.action)[i] = make_float4(act[0], act[1], act[2], act[3]);
-                        else if constexpr (ACT == 2) reinterpret_cast<float2*>(a.action)[i] = make_float2(act[0], act[1]);
-                        else a.action[i] = act[0];
-                    }
+                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1));
+                hidden_epilogue<true>(lane_base + kColHidden, sm.slot.a, row, k, 12 + 8 * (layer - 1));      // (layer 2 overwrites the tile its finished MMAs read)
+                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 1);
+                fence_async_smem();
+                fence_before_sync();
+                bar_arrive(&sm.ready);
+                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 2);
+                if (layer == 1) {                                    // under layer 2's MMAs: which tile is next, and its state on the way
+                    nxt_tile = next_tile(sm, k, clc_phase);
+                    fetch(nxt_tile, nxt);
                 }
             }
+            bar_wait(&sm.done, phase); phase ^= 1u;
+            fence_after_sync();
+            TC_TRACE((t & 31) == 0, warp, k, 6);
+            float pre[4];
+            tmem_ld4(lane_base + kColOut, pre);
+            TC_TRACE((t & 31) == 0, warp, k, 7);
+            if (nxt_tile != kNoTile) {                               // the next tile's observation row first: the MMA warp is waiting for it
+                write_obs_row<FIRST, OBS>(sm.slot, row, nxt);
+                fence_before_sync();
+                bar_arrive(&sm.ready);
+                TC_TRACE((t & 31) == 0, warp, k, 8);
+            }
+            const int64_t i = (int64_t)tile * kTile + row;
+            if (i < a.n) {
+                float act[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) act[j] = fmaf(a.out_scale, tanh_mufu(pre[j]), a.out_offset);
+                if constexpr (ACT == 4) reinterpret_cast<float4*>(a.action)[i] = make_float4(act[0], act[1], act[2], act[3]);
+                else if constexpr (ACT == 2) reinterpret_cast<float2*>(a.action)[i] = make_float2(act[0], act[1]);
+                else a.action[i] = act[0];
+            }
+            tile = nxt_tile;
         }
     }
     TC_TRACE_CTA(2);

@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
 """
 Developer tool (CPU only): the polynomial tanh of the policy kernels' FMA-pipe route
-(gym_copter_b200/csrc/copter_policy.cuh: tanh_poly_coef / kTanhClamp; used by tanh_pack_poly there and by
-tanh_fma in copter_policy_tc.cuh).
+(gym_copter_b200/csrc/copter_policy_tc.cuh: tanh_poly_coef / kTanhClamp, used by tanh_fma there).
 
     tanh(x) ~ x * P(x^2),  P of degree 6 (odd polynomial of degree 13), |x| clamped to 3.25
 

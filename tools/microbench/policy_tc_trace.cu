@@ -35,8 +35,7 @@ int main(int argc, char** argv) {
     constexpr auto kernel = tc::copter_mlp_policy_tc_kernel<0, 10, 4>;
     constexpr int smem = (int)sizeof(tc::Smem) + 128;
     CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0));
-    const int grid = tc::kClc ? (int)((n + tc::kTile - 1) / tc::kTile) : sms * COPTER_POLICY_TC_CTAS_PER_SM;
+    const int grid = (int)((n + tc::kTile - 1) / tc::kTile);          // one CTA per tile: cluster launch control
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     for (int i = 0; i < 3; ++i) kernel<<<grid, tc::kThreads, smem>>>(a);
     CK(cudaDeviceSynchronize());

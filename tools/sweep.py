@@ -1,8 +1,9 @@
 #!/usr/bin/env python3
 """
-Developer tool: build-time parameter sweep (step kernel: CTAs/SM target, block size; policy
-kernels: the COPTER_POLICY_* knobs).  `build` cross-compiles the variants here (no GPU needed) into
-tools/variants/; `run` times each on the GPU box (one subprocess per variant) and prints achieved GB/s.
+Developer tool: times builds of the library against each other.  `build` cross-compiles the current
+sources here (no GPU needed) into tools/variants/lib_current.so; `run` times it and every hand-built
+tools/variants/lib_v*.so on the GPU box (one subprocess per build) and prints achieved GB/s and the
+policy kernel's time and error.
 
     python tools/sweep.py build
     gpurun -- python tools/sweep.py run [--envs N] [--k K]
@@ -21,21 +22,6 @@ from gym_copter_b200.build import NVCC_FLAGS          # noqa: E402  (the product
 
 VARIANTS = {}
 VARIANTS['current'] = []
-VARIANTS['tc_s1'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=1']    # tcgen05 policy kernel: 1 tile in flight per CTA, 4 CTAs per SM, one thread per row
-VARIANTS['tc_s1x2'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=2']  # two threads per row, 3 CTAs per SM
-VARIANTS['tc_s1x2c4'] = ['-DCOPTER_POLICY_TC_SLOTS=1', '-DCOPTER_POLICY_TC_SPLIT=2', '-DCOPTER_POLICY_TC_CTAS_PER_SM=4']  # 4 CTAs per SM (<= 56 registers)
-VARIANTS['tc_p4'] = ['-DCOPTER_POLICY_TC_POLY=4']     # 4 of every 16 hidden tanh on the FMA pipe
-VARIANTS['tc_p6'] = ['-DCOPTER_POLICY_TC_POLY=6']
-VARIANTS['tc_p8'] = ['-DCOPTER_POLICY_TC_POLY=8']
-VARIANTS['tc_c5'] = ['-DCOPTER_POLICY_TC_CTAS_PER_SM=5']          # 64 TMEM columns per tile: five / six CTAs per SM
-VARIANTS['tc_c6'] = ['-DCOPTER_POLICY_TC_CTAS_PER_SM=6']
-VARIANTS['tc_c5p6'] = ['-DCOPTER_POLICY_TC_CTAS_PER_SM=5', '-DCOPTER_POLICY_TC_POLY=6']
-VARIANTS['tc_c6p6'] = ['-DCOPTER_POLICY_TC_CTAS_PER_SM=6', '-DCOPTER_POLICY_TC_POLY=6']
-VARIANTS['tc_c6p8'] = ['-DCOPTER_POLICY_TC_CTAS_PER_SM=6', '-DCOPTER_POLICY_TC_POLY=8']
-VARIANTS['tc_ro5'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=5']  # fused rollout: 5 CTAs per SM (<= 80 registers)
-VARIANTS['tc_ro5c5'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=5', '-DCOPTER_POLICY_TC_CTAS_PER_SM=5']
-VARIANTS['tc_ro3'] = ['-DCOPTER_POLICY_ROLLOUT_TC_CTAS_PER_SM=3']
-VARIANTS['tc_s2x2'] = ['-DCOPTER_POLICY_TC_SLOTS=2', '-DCOPTER_POLICY_TC_SPLIT=2']  # 2 tiles in flight, 2 CTAs per SM, two threads per row
 if os.environ.get('COPTER_SWEEP_ONLY'):
     VARIANTS = {k: v for k, v in VARIANTS.items() if k.startswith(tuple(os.environ['COPTER_SWEEP_ONLY'].split(',')))}
 
