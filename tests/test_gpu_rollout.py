@@ -450,7 +450,7 @@ def test_fused_mlp_policy_vs_torch_fp32(pkg, variant, kernel, policy_kernel_choi
 
 @pytest.mark.parametrize('kernel', ['1', '0'])
 @pytest.mark.parametrize('variant,n', [('Lander3D', 4099), ('Lander2D', 1000), ('Hover3D', 257), ('Lander1D', 31), ('Takeoff', 129),
-                                       ('Lander3D', 128 * 148 * 8 + 77)])
+                                       ('Hover2D', 517), ('Hover1D', 33), ('Lander3D', 128 * 148 * 8 + 77)])
 def test_fused_policy_rollout_equals_policy_kernel_plus_step(pkg, variant, n, kernel, policy_kernel_choice):
     """copter_policy_rollout_f32 (policy + env step for T steps in one launch, state in
     registers) against the same network evaluated by copter_policy_mlp_f32 and stepped by

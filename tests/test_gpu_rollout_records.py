@@ -106,7 +106,7 @@ def test_rollout_records_equal_the_step_loop(pkg, variant, source, scale, offset
 @pytest.mark.parametrize('kernel', ['1', '0'])
 @pytest.mark.parametrize('std', [False, True])
 @pytest.mark.parametrize('variant,n', [('Lander3D', 4099), ('Lander2D', 1000), ('Hover3D', 257), ('Lander1D', 31),
-                                       ('Lander3D', 128 * 148 * 8 + 77)])
+                                       ('Hover2D', 517), ('Hover1D', 33), ('Lander3D', 128 * 148 * 8 + 77)])
 def test_fused_policy_rollout_records_equal_policy_rollout(pkg, variant, n, std, kernel, policy_kernel_choice):
     """copter_policy_rollout_f32 records (tcgen05 kernel '1', warp-MMA kernel '0') against PolicyRollout, the step
     loop under the standalone policy kernel of the same kind: causes, terminal observations, terminated and truncated
