@@ -9,7 +9,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 # COPTER_B200_LIB: developer knob used by tools/sweep.py to time alternative builds
 LIB_PATH = os.environ.get('COPTER_B200_LIB') or os.path.join(PKG, 'libcopter_b200.so')
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 STATS_LEN = 16
 STATS_SLOTS = 64
 F_AUTO_RESET, F_KEEP_EPISODE = 1, 2
@@ -38,7 +38,7 @@ class CopterBuffers(C.Structure):
                 ('obs', C.c_void_p), ('reward', C.c_void_p), ('done', C.c_void_p),
                 ('init_force', C.c_void_p), ('ep_return', C.c_void_p), ('stats', C.c_void_p),
                 ('final_obs', C.c_void_p), ('cause', C.c_void_p), ('state_stride', C.c_int64),
-                ('meta_hi', C.c_void_p)]
+                ('meta_hi', C.c_void_p), ('state_env_stride', C.c_int64)]
 
 
 class CopterActionSource(C.Structure):
@@ -112,6 +112,8 @@ def load():
     lib.copter_default_pid_gains.argtypes, lib.copter_default_pid_gains.restype = [C.POINTER(CopterPidGains)], None
     lib.copter_policy_mlp_f32.argtypes = [vp, i64, i64, i32, i32, vp, vp, vp, vp, vp, vp, C.c_float, C.c_float, vp, vp]
     lib.copter_policy_mlp_f32.restype = i32
+    lib.copter_policy_mlp_strided_f32.argtypes = [vp, i64, i64, i64, i32, i32, vp, vp, vp, vp, vp, vp, C.c_float, C.c_float, vp, vp]
+    lib.copter_policy_mlp_strided_f32.restype = i32
     lib.copter_policy_rollout_f32.argtypes = [P, B, C.POINTER(CopterMlpPolicy), i64, i64, u64, i64, i32, i32, i32, vp, vp, vp, vp,
                                               vp, vp, vp]
     lib.copter_policy_rollout_f32.restype = i32

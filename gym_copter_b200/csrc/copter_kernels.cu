@@ -24,7 +24,7 @@ template <typename T>
 struct StepArgs {
     T* state; uint32_t* meta; uint32_t* meta_hi; const T* action; float* obs; T* reward; uint8_t* done;
     const T* init_force; T* ep_return; double* stats; float* final_obs; uint8_t* cause;
-    int64_t n, stride, env_offset; uint64_t seed; int k; int auto_reset;
+    int64_t n, stride, env_stride, env_offset; uint64_t seed; int k; int auto_reset;
 };
 
 // One env's inputs exactly as they sit in HBM (128-bit vectors): load_raw issues every load, and
@@ -44,10 +44,10 @@ template <typename T, int A>
 __device__ __forceinline__ void load_raw(const StepArgs<T>& a, int64_t i, RawEnv<T, A>& r) {
     using V4 = typename Vec<T>::type;
     constexpr int V = Vec<T>::V;
-    const V4* planes = reinterpret_cast<const V4*>(a.state);
+    const V4* env = reinterpret_cast<const V4*>(a.state) + i * a.env_stride;       // as load_state
 #pragma unroll
     for (int pl = 0; pl < 12 / V; ++pl)
-        r.plane[pl] = planes[(int64_t)pl * a.stride + i];
+        r.plane[pl] = env[(int64_t)pl * a.stride];
     r.meta = a.meta[i];
     r.meta_hi = a.meta_hi ? a.meta_hi[i] : 0u;
     if constexpr (A == 4 && sizeof(T) == 4) {
@@ -290,7 +290,7 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
     }
 
     if (valid) {
-        store_state<T>(a.state, a.stride, i, s);
+        store_state<T>(a.state, a.stride, a.env_stride, i, s);
         store_meta(a.meta, a.meta_hi, i, st, steps, episode);
         a.reward[i] = total;
         a.done[i] = done_any ? 1 : 0;
@@ -329,7 +329,7 @@ struct RolloutArgs {
     T* state; uint32_t* meta; uint32_t* meta_hi; float* obs; T* reward_sum; uint8_t* done_any;
     const T* init_force; T* ep_return; double* stats;
     T* reward_tn; uint8_t* done_tn; T* action_tn;
-    int64_t n, stride, env_offset, first_step; uint64_t seed;
+    int64_t n, stride, env_stride, env_offset, first_step; uint64_t seed;
     int n_steps, auto_reset, src_kind; T src_scale, src_offset;
     T* controller;              // [n][16] PID memories (COPTER_SRC_PID), [n][24] (COPTER_SRC_PID_HOVER)
     T rate_kp, rate_ki, rate_kd, rate_windup, rate_big, pos_kp, pos_ki, pos_kd, pos_windup, pos_target, descent_kp, descent_kd;
@@ -527,7 +527,7 @@ copter_rollout_kernel(const __grid_constant__ KParams<T> kp, const __grid_consta
         int st = ST_LANDED, steps = 1; uint32_t episode = 0;
         T total = (T)0, ret = (T)0; bool done_any = false;
         if (valid) {
-            load_state<T>(a.state, a.stride, i, s);
+            load_state<T>(a.state, a.stride, a.env_stride, i, s);
             decode_meta(a.meta[i], a.meta_hi, i, st, steps, episode);
             if (STATS && a.ep_return) ret = a.ep_return[i];
         } else {
@@ -611,7 +611,7 @@ copter_rollout_kernel(const __grid_constant__ KParams<T> kp, const __grid_consta
             if (STATS) ret += seg;
         }
         if (valid) {
-            store_state<T>(a.state, a.stride, i, s);
+            store_state<T>(a.state, a.stride, a.env_stride, i, s);
             store_meta(a.meta, a.meta_hi, i, st, steps, episode);
             if (a.reward_sum) a.reward_sum[i] = total;
             if (a.done_any) a.done_any[i] = done_any ? 1 : 0;
@@ -638,7 +638,7 @@ struct PolicyRolloutArgs {
     float* state; uint32_t* meta; uint32_t* meta_hi; float* obs; float* reward_sum; uint8_t* done_any;
     const float* init_force; float* ep_return; double* stats;
     float* reward_tn; uint8_t* done_tn; float* action_tn; float* obs_tn;
-    int64_t n, stride, env_offset, first_step; uint64_t seed; int n_steps, auto_reset;
+    int64_t n, stride, env_stride, env_offset, first_step; uint64_t seed; int n_steps, auto_reset;
     PolicyWeights w;
     const float* action_std;    // [A] or null: Gaussian exploration noise around the network's output
     uint8_t* cause_tn; float* final_obs_tn;   // ending records (RECORD instantiations only)
@@ -670,7 +670,7 @@ copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __
         int st = ST_LANDED, steps = 1; uint32_t episode = 0;
         T total = (T)0, ret = (T)0; bool done_any = false;
         if (valid) {
-            load_state<T>(a.state, a.stride, i, s);
+            load_state<T>(a.state, a.stride, a.env_stride, i, s);
             decode_meta(a.meta[i], a.meta_hi, i, st, steps, episode);
             if (STATS && a.ep_return) ret = a.ep_return[i];
         } else {
@@ -728,7 +728,7 @@ copter_policy_rollout_kernel(const __grid_constant__ KParams<float> kp, const __
             if (STATS) flush_episode_stats<T>(a.stats, lane, dn, cause, ep_len, ep_ret, a.ep_return != nullptr);
         }
         if (valid) {
-            store_state<T>(a.state, a.stride, i, s);
+            store_state<T>(a.state, a.stride, a.env_stride, i, s);
             store_meta(a.meta, a.meta_hi, i, st, steps, episode);
             if (a.reward_sum) a.reward_sum[i] = total;
             if (a.done_any) a.done_any[i] = done_any ? 1 : 0;
@@ -837,7 +837,7 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
             int st = ST_LANDED, steps = 1; uint32_t episode = 0;
             T total = (T)0, ret = (T)0; bool done_any = false;
             if (valid) {
-                load_state<T>(a.state, a.stride, i, s);
+                load_state<T>(a.state, a.stride, a.env_stride, i, s);
                 decode_meta(a.meta[i], a.meta_hi, i, st, steps, episode);
                 if (STATS && a.ep_return) ret = a.ep_return[i];
             } else {
@@ -912,7 +912,7 @@ copter_policy_rollout_tc_kernel(const __grid_constant__ KParams<float> kp, const
                 if (STATS) flush_episode_stats<T>(a.stats, lane, dn, cause, ep_len, ep_ret, a.ep_return != nullptr);
             }
             if (valid) {
-                store_state<T>(a.state, a.stride, i, s);
+                store_state<T>(a.state, a.stride, a.env_stride, i, s);
                 store_meta(a.meta, a.meta_hi, i, st, steps, episode);
                 if (a.reward_sum) a.reward_sum[i] = total;
                 if (a.done_any) a.done_any[i] = done_any ? 1 : 0;
@@ -982,7 +982,7 @@ __global__ void __launch_bounds__(kGaeBlock) copter_gae_kernel(const __grid_cons
 template <typename T, int VARIANT>
 __global__ void __launch_bounds__(kBlock)
 copter_reset_kernel(const __grid_constant__ KParams<T> kp, T* state, uint32_t* meta, uint32_t* meta_hi, float* obs, T* ep_return,
-                    int64_t n, int64_t stride, int keep_episode) {
+                    int64_t n, int64_t stride, int64_t env_stride, int keep_episode) {
     constexpr int O = Variant<VARIANT>::O;
     __shared__ __align__(16) float tiles[kWarpsPerBlock][32 * O];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -993,7 +993,7 @@ copter_reset_kernel(const __grid_constant__ KParams<T> kp, T* state, uint32_t* m
         T s[12]; int st, steps;
         reset_state<T>(kp, s, st, steps);
         if (i < n) {
-            store_state<T>(state, stride, i, s);
+            store_state<T>(state, stride, env_stride, i, s);
             // COPTER_F_KEEP_EPISODE: the env's next episode index, so that a reset() per episode draws a new
             // reset force every time (the reference draws fresh np.random.uniform forces, task.py:175-184)
             uint32_t episode = 0;
@@ -1016,7 +1016,7 @@ copter_dynamics_kernel(const __grid_constant__ KParams<T> kp, T* state, uint8_t*
                        T* perturb, const T* motors, int64_t n) {
     for (int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (int64_t)gridDim.x * kBlock) {
         T s[12], p[6], m[4];
-        load_state<T>(state, n, i, s);
+        load_state<T>(state, n, 1, i, s);
         int st = status[i];
 #pragma unroll
         for (int j = 0; j < 6; ++j) p[j] = perturb[6 * i + j];
@@ -1025,7 +1025,7 @@ copter_dynamics_kernel(const __grid_constant__ KParams<T> kp, T* state, uint8_t*
         const Forces<T> f = motor_forces<T>(kp, m[0], m[1], m[2], m[3]);
         T na, nc;
         const bool finished = dynamics_update<T, 6, true>(kp, s, st, f, p, na, nc);
-        store_state<T>(state, n, i, s);
+        store_state<T>(state, n, 1, i, s);
         status[i] = (uint8_t)st;
         if (finished) {                                            // :194-197
 #pragma unroll
@@ -1096,6 +1096,16 @@ constexpr int64_t kMaxEnvsPerLaunch = (int64_t)0x7fffffff * kBlock;
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// The state addressing of a call (include/copter_b200.h, "Memory layout"): vectors between planes (0: n) and between
+// envs (0: 1).  False when the 12/V planes of the n envs would overlap.
+template <typename T>
+bool state_layout(int64_t n, int64_t state_stride, int64_t state_env_stride, int64_t& stride, int64_t& env_stride) {
+    constexpr int64_t planes = 12 / Vec<T>::V;
+    stride = state_stride > 0 ? state_stride : n;
+    env_stride = state_env_stride > 0 ? state_env_stride : 1;
+    return env_stride <= stride ? stride / env_stride >= n : env_stride / planes >= stride;
+}
+
 int check_params(const CopterParams* p, bool wide = false) {
     if (!p) return COPTER_E_ARG;
     if (p->max_steps < 1 || p->max_steps > (wide ? COPTER_MAX_STEPS_LIMIT_WIDE : COPTER_MAX_STEPS_LIMIT)) return COPTER_E_RANGE;
@@ -1117,16 +1127,16 @@ int launch_step(const CopterParams* p, const CopterBuffers* b, int64_t n, int64_
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
     if (!b->state || !b->meta || !b->action || !b->reward || !b->done) return COPTER_E_ARG;
-    if (n < 0 || n > kMaxEnvsPerLaunch || env_offset < 0 || k < 1 || (b->state_stride > 0 && b->state_stride < n)) return COPTER_E_RANGE;
+    StepArgs<T> a;
+    if (n < 0 || n > kMaxEnvsPerLaunch || env_offset < 0 || k < 1 || !state_layout<T>(n, b->state_stride, b->state_env_stride, a.stride, a.env_stride)) return COPTER_E_RANGE;
     if (variant < 0 || variant >= COPTER_NUM_VARIANTS) return COPTER_E_VARIANT;
     if (!aligned16(b->state) || !aligned16(b->action) || (b->obs && !aligned16(b->obs))) return COPTER_E_ALIGN;
     if (n == 0) return 0;
     const KParams<T> kp = make_kparams<T>(*p, b->meta_hi != nullptr);
-    StepArgs<T> a;
     a.state = (T*)b->state; a.meta = b->meta; a.meta_hi = b->meta_hi; a.action = (const T*)b->action; a.obs = b->obs;
     a.reward = (T*)b->reward; a.done = b->done; a.init_force = (const T*)b->init_force;
     a.ep_return = (T*)b->ep_return; a.stats = b->stats; a.final_obs = b->final_obs; a.cause = b->cause;
-    a.n = n; a.stride = b->state_stride > 0 ? b->state_stride : n; a.env_offset = env_offset; a.seed = seed; a.k = k; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
+    a.n = n; a.env_offset = env_offset; a.seed = seed; a.k = k; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
     cudaStream_t s = (cudaStream_t)stream;
     switch (variant) {
         case COPTER_LANDER3D: return launch_step_v<T, COPTER_LANDER3D>(kp, a, s);
@@ -1174,17 +1184,17 @@ int launch_rollout(const CopterParams* p, const CopterBuffers* b, const CopterAc
     if (e) return e;
     if (!b->state || !b->meta || !src) return COPTER_E_ARG;
     if ((src->kind == COPTER_SRC_PID || src->kind == COPTER_SRC_PID_HOVER) && (!controller || !aligned16(controller))) return COPTER_E_ARG;
-    if (n < 0 || env_offset < 0 || n_steps < 1 || first_step < 0 || (b->state_stride > 0 && b->state_stride < n)) return COPTER_E_RANGE;
+    RolloutArgs<T> a;
+    if (n < 0 || env_offset < 0 || n_steps < 1 || first_step < 0 || !state_layout<T>(n, b->state_stride, b->state_env_stride, a.stride, a.env_stride)) return COPTER_E_RANGE;
     if (src->kind < COPTER_SRC_CONST || src->kind > COPTER_SRC_PID_HOVER) return COPTER_E_RANGE;
     if (variant < 0 || variant >= COPTER_NUM_VARIANTS) return COPTER_E_VARIANT;
     if (!aligned16(b->state) || (b->obs && !aligned16(b->obs))) return COPTER_E_ALIGN;
     if (n == 0) return 0;
     const KParams<T> kp = make_kparams<T>(*p, b->meta_hi != nullptr);
-    RolloutArgs<T> a;
     a.state = (T*)b->state; a.meta = b->meta; a.meta_hi = b->meta_hi; a.obs = b->obs; a.reward_sum = (T*)b->reward; a.done_any = b->done;
     a.init_force = (const T*)b->init_force; a.ep_return = (T*)b->ep_return; a.stats = b->stats;
     a.reward_tn = (T*)reward_tn; a.done_tn = done_tn; a.action_tn = (T*)action_tn; a.cause_tn = cause_tn; a.final_obs_tn = final_obs_tn;
-    a.n = n; a.stride = b->state_stride > 0 ? b->state_stride : n; a.env_offset = env_offset; a.first_step = first_step;
+    a.n = n; a.env_offset = env_offset; a.first_step = first_step;
     a.seed = seed; a.n_steps = n_steps; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
     a.src_kind = src->kind; a.src_scale = (T)src->scale; a.src_offset = (T)src->offset;
     CopterPidGains g;
@@ -1207,8 +1217,8 @@ int launch_rollout(const CopterParams* p, const CopterBuffers* b, const CopterAc
 }
 
 template <typename T, int VARIANT>
-int launch_reset_v(const KParams<T>& kp, const CopterBuffers* b, int64_t n, int keep_episode, cudaStream_t s) {
-    copter_reset_kernel<T, VARIANT><<<grid_for(n), kBlock, 0, s>>>(kp, (T*)b->state, b->meta, b->meta_hi, b->obs, (T*)b->ep_return, n, b->state_stride > 0 ? b->state_stride : n, keep_episode);
+int launch_reset_v(const KParams<T>& kp, const CopterBuffers* b, int64_t n, int64_t stride, int64_t env_stride, int keep_episode, cudaStream_t s) {
+    copter_reset_kernel<T, VARIANT><<<grid_for(n), kBlock, 0, s>>>(kp, (T*)b->state, b->meta, b->meta_hi, b->obs, (T*)b->ep_return, n, stride, env_stride, keep_episode);
     return (int)cudaGetLastError();
 }
 
@@ -1218,7 +1228,8 @@ int launch_reset(const CopterParams* p, const CopterBuffers* b, int64_t n, int v
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
     if (!b->state || !b->meta) return COPTER_E_ARG;
-    if (n < 0 || (b->state_stride > 0 && b->state_stride < n)) return COPTER_E_RANGE;
+    int64_t stride, env_stride;
+    if (n < 0 || !state_layout<T>(n, b->state_stride, b->state_env_stride, stride, env_stride)) return COPTER_E_RANGE;
     if (variant < 0 || variant >= COPTER_NUM_VARIANTS) return COPTER_E_VARIANT;
     if (!aligned16(b->state) || (b->obs && !aligned16(b->obs))) return COPTER_E_ALIGN;
     if (n == 0) return 0;
@@ -1226,13 +1237,13 @@ int launch_reset(const CopterParams* p, const CopterBuffers* b, int64_t n, int v
     const int keep = (flags & COPTER_F_KEEP_EPISODE) ? 1 : 0;
     cudaStream_t s = (cudaStream_t)stream;
     switch (variant) {
-        case COPTER_LANDER3D: return launch_reset_v<T, COPTER_LANDER3D>(kp, b, n, keep, s);
-        case COPTER_LANDER2D: return launch_reset_v<T, COPTER_LANDER2D>(kp, b, n, keep, s);
-        case COPTER_LANDER1D: return launch_reset_v<T, COPTER_LANDER1D>(kp, b, n, keep, s);
-        case COPTER_HOVER3D:  return launch_reset_v<T, COPTER_HOVER3D>(kp, b, n, keep, s);
-        case COPTER_HOVER2D:  return launch_reset_v<T, COPTER_HOVER2D>(kp, b, n, keep, s);
-        case COPTER_HOVER1D:  return launch_reset_v<T, COPTER_HOVER1D>(kp, b, n, keep, s);
-        default:              return launch_reset_v<T, COPTER_TAKEOFF>(kp, b, n, keep, s);
+        case COPTER_LANDER3D: return launch_reset_v<T, COPTER_LANDER3D>(kp, b, n, stride, env_stride, keep, s);
+        case COPTER_LANDER2D: return launch_reset_v<T, COPTER_LANDER2D>(kp, b, n, stride, env_stride, keep, s);
+        case COPTER_LANDER1D: return launch_reset_v<T, COPTER_LANDER1D>(kp, b, n, stride, env_stride, keep, s);
+        case COPTER_HOVER3D:  return launch_reset_v<T, COPTER_HOVER3D>(kp, b, n, stride, env_stride, keep, s);
+        case COPTER_HOVER2D:  return launch_reset_v<T, COPTER_HOVER2D>(kp, b, n, stride, env_stride, keep, s);
+        case COPTER_HOVER1D:  return launch_reset_v<T, COPTER_HOVER1D>(kp, b, n, stride, env_stride, keep, s);
+        default:              return launch_reset_v<T, COPTER_TAKEOFF>(kp, b, n, stride, env_stride, keep, s);
     }
 }
 
@@ -1289,7 +1300,7 @@ int launch_policy_v(const PolicyArgs& a, cudaStream_t s) {
     using V = Variant<VARIANT>;
     if (policy_tc_setting()) {
         tc::Args t;
-        t.state = a.state; t.stride = a.stride; t.n = a.n;
+        t.state = a.state; t.stride = a.stride; t.env_stride = a.env_stride; t.n = a.n;
         t.w1 = a.w.w1; t.b1 = a.w.b1; t.w2 = a.w.w2; t.b2 = a.w.b2; t.w3 = a.w.w3; t.b3 = a.w.b3;
         t.out_scale = a.w.out_scale; t.out_offset = a.w.out_offset; t.action = a.action;
         constexpr auto kernel = tc::copter_mlp_policy_tc_kernel<V::first, V::O, V::A>;
@@ -1389,7 +1400,8 @@ int step_host(Pipeline* pl, const CopterParams* p, const CopterBuffers* dev, con
     const int O = copter_obs_size(variant), A = copter_action_size(variant);
     constexpr int V = Vec<T>::V;
     chunk = (chunk + 255) / 256 * 256;                    // keeps every sub-shard 16-byte aligned
-    const int64_t stride = dev->state_stride > 0 ? dev->state_stride : n;
+    int64_t stride, env_stride;
+    if (!state_layout<T>(n, dev->state_stride, dev->state_env_stride, stride, env_stride)) return COPTER_E_RANGE;
     cudaError_t ce;
     static const int64_t direct_max = [] { const char* e = getenv("COPTER_B200_DIRECT_MAX_ENVS"); return e ? (int64_t)atoll(e) : (int64_t)COPTER_DIRECT_MAX_ENVS; }();
     if (n > 0 && n <= direct_max) {                       // the direct path: see mapped_device_pointer
@@ -1421,7 +1433,7 @@ int step_host(Pipeline* pl, const CopterParams* p, const CopterBuffers* dev, con
         const int64_t m = (n - lo < chunk) ? (n - lo) : chunk;
         cudaStream_t st = pl->streams[c % pl->n_streams];
         CopterBuffers b = *dev;
-        b.state = (T*)dev->state + lo * V;               // same planes, shifted by `lo` vectors
+        b.state = (T*)dev->state + lo * env_stride * V;  // same layout, shifted by `lo` envs
         b.state_stride = stride;
         b.meta = dev->meta + lo;
         b.meta_hi = dev->meta_hi ? dev->meta_hi + lo : nullptr;
@@ -1533,13 +1545,19 @@ int copter_reset_force_f64(const CopterParams* p, double* out, const uint32_t* e
 int copter_policy_mlp_f32(const void* state, int64_t state_stride, int64_t n, int variant, int hidden,
                           const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
                           float out_scale, float out_offset, float* action, void* stream) {
+    return copter_policy_mlp_strided_f32(state, state_stride, 0, n, variant, hidden, w1, b1, w2, b2, w3, b3, out_scale, out_offset, action, stream);
+}
+
+int copter_policy_mlp_strided_f32(const void* state, int64_t state_stride, int64_t state_env_stride, int64_t n, int variant, int hidden,
+                                  const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                                  float out_scale, float out_offset, float* action, void* stream) {
     if (!state || !w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !action) return COPTER_E_ARG;
     if (variant < 0 || variant >= COPTER_NUM_VARIANTS) return COPTER_E_VARIANT;
-    if (n < 0 || hidden != kPolH || (state_stride > 0 && state_stride < n)) return COPTER_E_RANGE;
+    PolicyArgs a;
+    if (n < 0 || hidden != kPolH || !state_layout<float>(n, state_stride, state_env_stride, a.stride, a.env_stride)) return COPTER_E_RANGE;
     if (!aligned16(state) || !aligned16(action)) return COPTER_E_ALIGN;
     if (n == 0) return 0;
-    PolicyArgs a;
-    a.state = (const float*)state; a.stride = state_stride > 0 ? state_stride : n; a.n = n;
+    a.state = (const float*)state; a.n = n;
     a.w.w1 = w1; a.w.b1 = b1; a.w.w2 = w2; a.w.b2 = b2; a.w.w3 = w3; a.w.b3 = b3;
     a.w.out_scale = out_scale; a.w.out_offset = out_offset; a.action = action;
     cudaStream_t s = (cudaStream_t)stream;
@@ -1562,17 +1580,18 @@ int copter_policy_rollout_f32(const CopterParams* p, const CopterBuffers* b, con
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
     if (!b->state || !b->meta || !policy_ok(policy)) return COPTER_E_ARG;
-    if (n < 0 || env_offset < 0 || first_step < 0 || n_steps < 1 || policy->hidden != kPolH || (b->state_stride > 0 && b->state_stride < n)) return COPTER_E_RANGE;
+    PolicyRolloutArgs a;
+    if (n < 0 || env_offset < 0 || first_step < 0 || n_steps < 1 || policy->hidden != kPolH ||
+        !state_layout<float>(n, b->state_stride, b->state_env_stride, a.stride, a.env_stride)) return COPTER_E_RANGE;
     if (variant < 0 || variant >= COPTER_NUM_VARIANTS) return COPTER_E_VARIANT;
     if (!aligned16(b->state) || (b->obs && !aligned16(b->obs)) || (action_tn && !aligned16(action_tn)) || (obs_tn && !aligned16(obs_tn))) return COPTER_E_ALIGN;
     if (n == 0) return 0;
     const KParams<float> kp = make_kparams<float>(*p, b->meta_hi != nullptr);
-    PolicyRolloutArgs a;
     a.state = (float*)b->state; a.meta = b->meta; a.meta_hi = b->meta_hi; a.obs = b->obs; a.reward_sum = (float*)b->reward; a.done_any = b->done;
     a.init_force = (const float*)b->init_force; a.ep_return = (float*)b->ep_return; a.stats = b->stats;
     a.reward_tn = reward_tn; a.done_tn = done_tn; a.action_tn = action_tn; a.obs_tn = obs_tn;
     a.cause_tn = cause_tn; a.final_obs_tn = final_obs_tn;
-    a.n = n; a.stride = b->state_stride > 0 ? b->state_stride : n; a.env_offset = env_offset; a.seed = seed;
+    a.n = n; a.env_offset = env_offset; a.seed = seed;
     a.first_step = first_step; a.n_steps = n_steps; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
     a.w = policy_weights(policy); a.action_std = policy->action_std;
     cudaStream_t s = (cudaStream_t)stream;

@@ -43,14 +43,17 @@ template <typename T> struct Vec;
 template <> struct Vec<float>  { using type = float4;  static constexpr int V = 4; };
 template <> struct Vec<double> { using type = double2; static constexpr int V = 2; };
 
+// Vector `pl` (components pl*V .. pl*V+V-1) of env i sits at vector pl * stride + i * env_stride of the
+// allocation (include/copter_b200.h, "Memory layout"): planes (stride >= n, env_stride 1) or one row per
+// env (stride 1, env_stride 12/V).  Every kernel that reads or writes state addresses it this way.
 template <typename T>
-__device__ __forceinline__ void load_state(const T* __restrict__ state, int64_t stride, int64_t i, T (&s)[12]) {
+__device__ __forceinline__ void load_state(const T* __restrict__ state, int64_t stride, int64_t env_stride, int64_t i, T (&s)[12]) {
     using V4 = typename Vec<T>::type;
     constexpr int V = Vec<T>::V;
-    const V4* planes = reinterpret_cast<const V4*>(state);
+    const V4* env = reinterpret_cast<const V4*>(state) + i * env_stride;
 #pragma unroll
     for (int pl = 0; pl < 12 / V; ++pl) {
-        V4 v = planes[(int64_t)pl * stride + i];
+        V4 v = env[(int64_t)pl * stride];
         const T* e = reinterpret_cast<const T*>(&v);
 #pragma unroll
         for (int j = 0; j < V; ++j) s[pl * V + j] = e[j];
@@ -58,17 +61,17 @@ __device__ __forceinline__ void load_state(const T* __restrict__ state, int64_t 
 }
 
 template <typename T>
-__device__ __forceinline__ void store_state(T* __restrict__ state, int64_t stride, int64_t i, const T (&s)[12]) {
+__device__ __forceinline__ void store_state(T* __restrict__ state, int64_t stride, int64_t env_stride, int64_t i, const T (&s)[12]) {
     using V4 = typename Vec<T>::type;
     constexpr int V = Vec<T>::V;
-    V4* planes = reinterpret_cast<V4*>(state);
+    V4* env = reinterpret_cast<V4*>(state) + i * env_stride;
 #pragma unroll
     for (int pl = 0; pl < 12 / V; ++pl) {
         V4 v;
         T* e = reinterpret_cast<T*>(&v);
 #pragma unroll
         for (int j = 0; j < V; ++j) e[j] = s[pl * V + j];
-        planes[(int64_t)pl * stride + i] = v;
+        env[(int64_t)pl * stride] = v;
     }
 }
 

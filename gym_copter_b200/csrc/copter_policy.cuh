@@ -1,7 +1,7 @@
 // copter_policy.cuh -- the small tanh MLP policy of BASELINE.json configs[4] (O -> 64 -> 64 -> A,
 // SURVEY.md 8d "config 5") evaluated by a warp for its 32 envs straight from the fp32 state each
 // lane holds in registers.  Two kernels use it (copter_kernels.cu): copter_mlp_policy_kernel
-// (state planes -> action rows, for policy-in-the-loop rollouts that step with copter_step_*)
+// (env state -> action rows, for policy-in-the-loop rollouts that step with copter_step_*)
 // and copter_policy_rollout_kernel (policy + env step for T steps in ONE launch, the state
 // never leaving registers).  In PyTorch this policy costs 4.2 ms per step for 2^23 envs (three
 // GEMMs with [N,64] intermediates through HBM plus separate tanh passes) against 0.21 ms for
@@ -219,14 +219,14 @@ __device__ __forceinline__ void policy_forward_warp(const PolicySmem& sm, Policy
 }
 
 struct PolicyArgs {
-    const float* state; int64_t stride, n;           // fp32 state planes [3][stride][4]
+    const float* state; int64_t stride, env_stride, n;   // fp32 state: float4 `pl` of env i at pl * stride + i * env_stride
     PolicyWeights w;
     float* action;                                   // [n][act]
 };
 
 constexpr int kPolicyCtasPerSm = 5;      // measured (profiles/r1_sweep_policy_occupancy.txt, 2^23 envs): 3: 0.386, 4: 0.373, 5: 0.359, 6: 0.368 ms
 
-// state planes -> action rows.  Persistent CTAs: the weights are converted once per CTA.
+// env state -> action rows.  Persistent CTAs: the weights are converted once per CTA.
 template <int FIRST, int OBS, int ACT>
 __global__ void __launch_bounds__(128, kPolicyCtasPerSm)
 copter_mlp_policy_kernel(const __grid_constant__ PolicyArgs a) {
@@ -241,10 +241,14 @@ copter_mlp_policy_kernel(const __grid_constant__ PolicyArgs a) {
         const int64_t i = wt * 32 + lane;
         float s[12];
         if (i < a.n) {
-            const float4* planes = reinterpret_cast<const float4*>(a.state);
+            // (env_stride made opaque inside the loop: otherwise the compiler carries i * env_stride as one more 64-bit
+            // induction variable across the network, and this 96-register kernel spills 136 instead of 56 bytes)
+            int64_t env_stride = a.env_stride;
+            asm volatile("" : "+l"(env_stride));
+            const float4* env = reinterpret_cast<const float4*>(a.state) + i * env_stride;
 #pragma unroll
             for (int pl = 0; pl < 3; ++pl) {
-                const float4 v = planes[(int64_t)pl * a.stride + i];
+                const float4 v = env[(int64_t)pl * a.stride];
                 s[4 * pl] = v.x; s[4 * pl + 1] = v.y; s[4 * pl + 2] = v.z; s[4 * pl + 3] = v.w;
             }
         } else {

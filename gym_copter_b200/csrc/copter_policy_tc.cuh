@@ -317,7 +317,7 @@ __device__ __forceinline__ void load_weights(Smem& sm, const float* w1, const fl
 }
 
 struct Args {
-    const float* state; int64_t stride, n;           // fp32 state planes [3][stride][4]
+    const float* state; int64_t stride, env_stride, n;   // fp32 state: float4 `pl` of env i at pl * stride + i * env_stride
     const float *w1, *b1, *w2, *b2, *w3, *b3;
     float out_scale, out_offset;
     float* action;                                   // [n][ACT]
@@ -408,7 +408,7 @@ __device__ __forceinline__ void request_tile(Smem& sm, int k_next) {
 }
 constexpr int kThreads = kTile + 32;      // the epilogue warps + the MMA warp
 
-// state planes -> action rows.  Persistent, warp-specialised CTAs (weights converted once per CTA), 128 envs
+// env state -> action rows.  Persistent, warp-specialised CTAs (weights converted once per CTA), 128 envs
 // per tile, one tile in flight per CTA, the tiles taken by cluster launch control (next_tile).
 //   epilogue warps   one thread per env row: pull the accumulator out of TMEM, tanh, fp16, write it to shared
 //              memory as the next layer's A operand, arrive on ready; after layer 3 store the env's action and
@@ -483,10 +483,10 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     } else {
         const int row = t;
         const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);       // this warp's quarter of the 128 TMEM lanes
-        const float4* planes = reinterpret_cast<const float4*>(a.state);
         auto fetch = [&](uint32_t tl, float4 (&p)[3]) {
             const int64_t i = (int64_t)tl * kTile + row;
-            if (tl != kNoTile && i < a.n) { p[0] = planes[i]; p[1] = planes[a.stride + i]; p[2] = planes[2 * a.stride + i]; }
+            const float4* env = reinterpret_cast<const float4*>(a.state) + i * a.env_stride;
+            if (tl != kNoTile && i < a.n) { p[0] = env[0]; p[1] = env[a.stride]; p[2] = env[2 * a.stride]; }
             else p[0] = p[1] = p[2] = make_float4(0.f, 0.f, 0.f, 0.f);
         };
         uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;

@@ -81,9 +81,9 @@ class CopterVecEnv:
     track_returns  also keep a running per-env episode return (one more T[N] array read and
                  written per step) so that `stats()` reports return sums / means
     keep_final_obs  also record the terminal observation of finished envs (`info['final_obs']`)
-    write_obs    False: the step kernel skips the [N,O] observation write (40 of 165 B per env
-                 for Lander3D); on the fp32 path consumers can read the state planes in place
-                 instead (`planar_obs()`, `rollout.PlanarLinear`) -- the zero-copy observation
+    write_obs    False: step() returns None for the observation, and the fp64 step kernel and
+                 step_host skip the [N,O] observation write.  On the fp32 path the observation is a
+                 view of the state rows (`obs`), which the kernels never write twice
     report_cause  record why each env finished (`info['cause']`, COPTER_CAUSE_* bits) and report
                  the env's own step limit as `truncated` the way gymnasium's
                  TimeLimit(max_episode_steps) wrapper does for the reference (gym_copter/__init__.py:9-13)
@@ -130,10 +130,24 @@ class CopterVecEnv:
         n, dev = self.num_envs, self.device
         V = 4 if dtype == torch.float32 else 2
         self._f32 = dtype == torch.float32
-        self.state_planes = torch.zeros((12 // V, n, V), dtype=dtype, device=dev)
+        # `state_planes` is the state seen as [12/V, N, V] vector planes; the kernels take its layout from its strides
+        # (_state_layout, include/copter_b200.h "Memory layout").  fp32: one [N,12] row per env, and the observation
+        # is the row slice first..first+O-1, so the step kernel writes it once, as state (125 instead of 165 B per
+        # Lander3D env-step).  fp64: the observation is a cast, a buffer of its own, so rows would save nothing, and
+        # the planes are kept: rows' 96-byte stride made the fp64 step 16 % slower (DESIGN.md, "State layout").
+        if self._f32:
+            rows = torch.zeros((n, 12), dtype=dtype, device=dev)
+            self.state_planes = rows.as_strided((12 // V, n, V), (V, 12, 1))
+            first = _OBS_IDX[variant][0]
+            self.obs = rows[:, first:first + self.obs_size]
+        else:
+            self.state_planes = torch.zeros((12 // V, n, V), dtype=dtype, device=dev)
+            self.obs = torch.zeros((n, self.obs_size), dtype=torch.float32, device=dev)
         self.meta = torch.zeros(n, dtype=torch.int32, device=dev)
         self.meta_hi = torch.zeros(n, dtype=torch.int32, device=dev) if self.wide else None
-        self.obs = torch.zeros((n, self.obs_size), dtype=torch.float32, device=dev)
+        # packed [N,O] rows the kernels write the observation into: fp64 `obs`; fp32 step_host's device-side
+        # staging rows, made by host_buffers()
+        self._obs_rows = None if self._f32 else self.obs
         self.reward = torch.zeros(n, dtype=dtype, device=dev)
         self.done = torch.zeros(n, dtype=torch.uint8, device=dev)
         self._truncated = torch.zeros(n, dtype=torch.bool, device=dev)
@@ -154,11 +168,15 @@ class CopterVecEnv:
 
     # ---- plumbing -----------------------------------------------------------------------
 
-    def _buffers(self, action=None, force=None, reward=None, done=None):
+    def _buffers(self, action=None, force=None, reward=None, done=None, device=False):
+        """The launch's CopterBuffers.  device=True: a launch whose observation stays on the device, which on the
+        fp32 path is the state itself, so the kernel is given no packed observation rows to write."""
         b = CopterBuffers()
         b.state, b.meta = self.state_planes.data_ptr(), self.meta.data_ptr()
+        b.state_stride, b.state_env_stride = self._state_layout()
         b.action = action.data_ptr() if action is not None else None
-        b.obs = self.obs.data_ptr() if (self.write_obs or action is None) else None
+        rows = None if device and self._f32 else self._obs_rows
+        b.obs = rows.data_ptr() if rows is not None and (self.write_obs or action is None) else None
         b.cause = self.cause.data_ptr() if (self.cause is not None and action is not None) else None
         b.reward = (self.reward if reward is None else reward).data_ptr()
         b.done = (self.done if done is None else done).data_ptr()
@@ -168,6 +186,11 @@ class CopterVecEnv:
         b.final_obs = self.final_obs.data_ptr() if self.final_obs is not None else None
         b.meta_hi = self.meta_hi.data_ptr() if self.meta_hi is not None else None
         return b
+
+    def _state_layout(self):
+        """(state_stride, state_env_stride) of the C ABI: vectors between planes and between envs."""
+        V = self.state_planes.shape[2]
+        return self.state_planes.stride(0) // V, self.state_planes.stride(1) // V
 
     def _stream(self):
         # (the raw handle: torch.cuda.current_stream() builds a Stream object, several microseconds of a 25 us single-env step)
@@ -215,7 +238,7 @@ class CopterVecEnv:
             self._force = f.to(device=self.device, dtype=self.dtype).reshape(self.num_envs, 3).contiguous()
         with torch.cuda.device(self.device):
             fn = self._lib.copter_reset_f32 if self._f32 else self._lib.copter_reset_f64
-            b = self._buffers()
+            b = self._buffers(device=True)
             _lib.check(fn(C.byref(self.params), C.byref(b), self.num_envs, VARIANT_IDS[self.variant],
                           _lib.F_KEEP_EPISODE if keep else 0, self._stream()), 'copter_reset')
         self.launches += 1
@@ -229,7 +252,8 @@ class CopterVecEnv:
         One batched `_Task.step` (envs/task.py:77-137), k_substeps times under one action.
         Returns (obs f32 [N,O], reward [N], terminated bool [N], truncated bool [N], info).
         The returned tensors are the env's own output buffers: they are overwritten by the
-        next step (clone them to keep them) -- or pass `reward_out` ([N], env dtype) and
+        next step (clone them to keep them) -- on the fp32 path the observation is a view of the
+        env state, so it is overwritten by the next step and must not be written into -- or pass `reward_out` ([N], env dtype) and
         `done_out` ([N] uint8) to have the kernel write this step's reward / done flags
         straight into a slice of a rollout buffer.  `cause_out` ([N] uint8) and `final_obs_out`
         ([N,O] f32) do the same for the ending's COPTER_CAUSE_* bits (0 where the episode goes
@@ -248,7 +272,7 @@ class CopterVecEnv:
                                  'uint8 / uint8 and an [N,O] float32 tensor on the env device')
         with torch.cuda.device(self.device):
             fn = self._lib.copter_step_f32 if self._f32 else self._lib.copter_step_f64
-            b = self._buffers(t, self._force, reward_out, done_out)
+            b = self._buffers(t, self._force, reward_out, done_out, device=True)
             if cause_out is not None:
                 b.cause = cause_out.data_ptr()
             if final_obs_out is not None:
@@ -327,7 +351,7 @@ class CopterVecEnv:
         fin = torch.zeros((T, n, self.obs_size), dtype=torch.float32, device=self.device) if record_final_obs else None
         with torch.cuda.device(self.device):
             fn = self._lib.copter_rollout_f32 if self._f32 else self._lib.copter_rollout_f64
-            b = self._buffers(None, self._force)
+            b = self._buffers(None, self._force, device=True)
             _lib.check(fn(C.byref(self.params), C.byref(b), C.byref(src), n, self.env_offset,
                           self.seed_value & 0xFFFFFFFFFFFFFFFF, self.rollout_step, T,
                           VARIANT_IDS[self.variant], _lib.F_AUTO_RESET if self.auto_reset else 0,
@@ -372,6 +396,8 @@ class CopterVecEnv:
                 t['final_obs'] = torch.zeros((n, self.obs_size), dtype=torch.float32).pin_memory()
             self._host_t = t
             self._host = {k: v.numpy() for k, v in t.items()}
+            if self._f32:           # the kernel writes packed rows for the device -> host copy
+                self._obs_rows = torch.zeros((n, self.obs_size), dtype=torch.float32, device=self.device)
         return self._host
 
     def step_host(self, action=None, chunk_envs=1 << 20, n_streams=4):
@@ -383,8 +409,8 @@ class CopterVecEnv:
         the step kernel and the device->host copies of obs/reward/done are chunked and
         pipelined over `n_streams` CUDA streams inside copter_step_host_*.  Shards of at most 65 536 envs take a
         direct path instead: one launch whose kernel reads the commands from and writes its results to the
-        page-locked host buffers themselves (the env's device-side obs / reward / done tensors are then not
-        refreshed by this call; state and counters are).
+        page-locked host buffers themselves (the env's device-side reward / done tensors and the fp64 obs are
+        then not refreshed by this call; state and counters are, and so is the fp32 obs, a view of the state).
         """
         if not self._is_reset:
             raise CopterError('step() called before reset()')
@@ -466,9 +492,9 @@ class CopterVecEnv:
     # ---- state access -------------------------------------------------------------------
 
     def planar_obs(self):
-        """Zero-copy observation on the fp32 path: the state planes themselves, [3, N, 4] float32
-        (plane p holds components 4p..4p+3 of dynamics/__init__.py:48-59).  For Lander3D the
-        observation is components 0..9, i.e. planes 0, 1 and the first two lanes of plane 2."""
+        """The fp32 state seen as planes, [3, N, 4] float32 (plane p holds components 4p..4p+3 of
+        dynamics/__init__.py:48-59; a view of the state rows).  For Lander3D the observation is
+        components 0..9, i.e. planes 0, 1 and the first two lanes of plane 2."""
         if not self._f32:
             raise CopterError('planar_obs() needs the float32 path (observations are float32)')
         return self.state_planes
@@ -476,7 +502,7 @@ class CopterVecEnv:
     @property
     def state(self):
         """[N,12] copy of the state in the reference's component order (dynamics:48-59)."""
-        return self.state_planes.permute(1, 0, 2).reshape(self.num_envs, 12)
+        return self.state_planes.permute(1, 0, 2).clone(memory_format=torch.contiguous_format).view(self.num_envs, 12)
 
     def set_state(self, state, status=None, steps=None):
         """
@@ -495,7 +521,8 @@ class CopterVecEnv:
             torch.as_tensor(steps, device=self.device).to(torch.int64).expand(self.num_envs)
         m = (st | (stp << 2)) if self.wide else ((m & ~0x1FFF) | st | (stp << 2))
         self.meta.copy_(torch.where(m >= 2 ** 31, m - 2 ** 32, m).to(torch.int32))
-        self.obs.copy_(s[:, list(_OBS_IDX[self.variant])].to(torch.float32))
+        if not self._f32:           # (fp32: obs is a view of the state just written)
+            self.obs.copy_(s[:, list(_OBS_IDX[self.variant])].to(torch.float32))
 
     def _meta64(self):
         return self.meta.to(torch.int64) & 0xFFFFFFFF
@@ -568,7 +595,8 @@ class CopterVecEnv:
         self.rollout_step = d.get('rollout_step', 0)
         self.state_planes.copy_(d['state_planes'])
         self.meta.copy_(d['meta'])
-        self.obs.copy_(d['obs'])
+        if not self._f32:           # (fp32: obs is a view of the state just loaded)
+            self.obs.copy_(d['obs'])
         for k in ('meta_hi', '_stats', 'ep_return', 'cause', 'final_obs'):
             v = getattr(self, k)
             if v is not None and k.lstrip('_') in d:
@@ -663,7 +691,7 @@ class SingleEnv:
         """(x, y, z, phi, theta, psi) as envs/task.py:102 sets it for the renderer thread; read from
         the device on demand (psi is not part of the Lander observation), so a plain step() loop does
         not pay for it."""
-        s = self.vec.state_planes.reshape(12).cpu().numpy()         # one env: plane-major order is component order
+        s = self.vec.state_planes.reshape(12).cpu().numpy()         # one env: component order
         return (s[0], s[2], s[4], s[6], s[8], s[10])
 
     def reset(self, seed=None, options=None, force=None):

@@ -137,8 +137,8 @@ class PlanarLinear(torch.nn.Module):
 
 class FusedMLPPolicy:
     """
-    The tanh MLP O -> 64 -> 64 -> A evaluated by ONE hand-written kernel (copter_policy_mlp_f32)
-    straight from the env's fp32 state planes -- no observation tensor, no [N,64] intermediates in
+    The tanh MLP O -> 64 -> 64 -> A evaluated by ONE hand-written kernel (copter_policy_mlp_strided_f32)
+    straight from the env's fp32 state rows -- no observation tensor, no [N,64] intermediates in
     HBM.  Two implementations, 16-bit operands (bf16; fp16 for the hidden layers of the tcgen05 kernel) with fp32
     accumulation in both: tcgen05.mma with the
     accumulators in tensor memory, 128 envs per tile (the default; csrc/copter_policy_tc.cuh), and
@@ -146,7 +146,7 @@ class FusedMLPPolicy:
     COPTER_B200_POLICY_TC=0 in the environment); FusedPolicyRollout has a fused kernel of each kind.  `net` is a torch.nn.Sequential(Linear, Tanh, Linear, Tanh, Linear,
     Tanh) (e.g. mlp_policy(...).net); its weights are read in place, so optimizer updates to
     fp32 parameters are picked up by the next call.  action = out_offset + out_scale * net(obs).
-    Use with PolicyRollout(..., planar=True) and CopterVecEnv(write_obs=False).
+    Use with PolicyRollout(..., planar=True).
     """
 
     def __init__(self, env, net, out_scale=1.0, out_offset=0.0):
@@ -155,7 +155,7 @@ class FusedMLPPolicy:
                 or lin[0].in_features != env.obs_size or lin[2].out_features != env.action_size:
             raise CopterError('FusedMLPPolicy needs Linear(O,64), Linear(64,64), Linear(64,A) with tanh activations')
         if env.dtype != torch.float32:
-            raise CopterError('FusedMLPPolicy reads the fp32 state planes: build the env with dtype=torch.float32')
+            raise CopterError('FusedMLPPolicy reads the fp32 state: build the env with dtype=torch.float32')
         self.env, self.lib = env, _lib.load()
         self.params = []
         for m in lin:
@@ -170,8 +170,8 @@ class FusedMLPPolicy:
     def __call__(self, planes=None):
         env = self.env
         with torch.cuda.device(env.device):
-            _lib.check(self.lib.copter_policy_mlp_f32(
-                env.state_planes.data_ptr(), env.num_envs, env.num_envs, VARIANT_IDS[env.variant], 64,
+            _lib.check(self.lib.copter_policy_mlp_strided_f32(
+                env.state_planes.data_ptr(), *env._state_layout(), env.num_envs, VARIANT_IDS[env.variant], 64,
                 *[p.data_ptr() for p in self.params], C.c_float(self.out_scale), C.c_float(self.out_offset),
                 self.action.data_ptr(), C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)),
                 'copter_policy_mlp')
@@ -233,9 +233,7 @@ class FusedPolicyRollout(_EndingRecords):
         if not env._is_reset:
             raise CopterError('reset() the env before rolling out')
         with torch.cuda.device(env.device):
-            b = env._buffers(None, env._force)
-            if not env.write_obs:
-                b.obs = None
+            b = env._buffers(None, env._force, device=True)
             _lib.check(self.lib.copter_policy_rollout_f32(
                 C.byref(env.params), C.byref(b), C.byref(self.policy), env.num_envs, env.env_offset,
                 env.seed_value & 0xFFFFFFFFFFFFFFFF, env.rollout_step, self.horizon, VARIANT_IDS[env.variant],

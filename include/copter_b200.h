@@ -32,8 +32,16 @@
  * torch.cuda.device) and passes the stream.  Launches are asynchronous.
  *
  * Memory layout (N envs, T = float or double, V = 16/sizeof(T) elements per 128-bit vector):
- *   state   T[12/V][N][V]   "vector planes": component j of env i is state[j/V][i][j%V], so a
- *                           thread reads its env with 12/V coalesced 128-bit loads.
+ *   state   12/V 128-bit vectors per env; vector p (components pV .. pV+V-1) of env i is vector
+ *                           p * state_stride + i * state_env_stride of the allocation
+ *                           (CopterBuffers), so a thread reads its env with 12/V 128-bit loads.  Two layouts:
+ *                             planes  T[12/V][N][V]  state_stride N, state_env_stride 1 (the default);
+ *                             rows    T[N][12]       state_stride 1, state_env_stride 12/V: one 48- / 96-byte
+ *                                                    row per env, whose components first .. first+O-1 are the
+ *                                                    observation when T = float -- what a float32
+ *                                                    CopterVecEnv keeps, so its steps pass obs = NULL and
+ *                                                    write 40 bytes less (a float64 one keeps planes).
+ *                           A warp's 12/V accesses cover one contiguous span in either layout.
  *                           Component order = the reference's state vector
  *                           (dynamics/__init__.py:48-59): x dx y dy z dz phi dphi theta dtheta psi dpsi.
  *   meta    uint32[N]       bits 0-1 flight status (COPTER_STATUS_*), bits 2-12 the env's
@@ -57,7 +65,7 @@
 extern "C" {
 #endif
 
-#define COPTER_ABI_VERSION 4
+#define COPTER_ABI_VERSION 5
 
 /* dynamics/__init__.py:65-68 */
 enum { COPTER_STATUS_CRASHED = 0, COPTER_STATUS_LANDED = 1, COPTER_STATUS_LEVELING = 2, COPTER_STATUS_AIRBORNE = 3 };
@@ -134,7 +142,7 @@ int copter_action_size(int variant);   /* A, or COPTER_E_VARIANT */
 
 /* Buffers of one shard of envs; all device pointers. Nullable members are marked. */
 typedef struct CopterBuffers {
-    void*       state;       /* T[12/V][n][V] */
+    void*       state;       /* 12/V vectors per env, addressed as in "Memory layout" */
     uint32_t*   meta;        /* [n] */
     const void* action;      /* T[n][A]            (unused by reset) */
     float*      obs;         /* [n][O]             nullable: skip the observation write */
@@ -146,9 +154,11 @@ typedef struct CopterBuffers {
     float*      final_obs;   /* [n][O] nullable: observation of the terminal state of envs that finished */
     uint8_t*    cause;       /* [n] nullable (step only): why the env finished in this launch, bit set of
                                 COPTER_CAUSE_*; 0 when it did not finish */
-    int64_t     state_stride;/* vectors per state plane in the allocation; 0 means n. Lets a call step a
-                                sub-range [lo, lo+n) of a larger shard: pass state + lo vectors, stride = shard size */
+    int64_t     state_stride;/* vectors between the state planes; 0 means n. Lets a call step a sub-range
+                                [lo, lo+n) of a larger shard: pass state + lo vectors, stride = shard size */
     uint32_t*   meta_hi;     /* [n] nullable: wide counters (see "Memory layout"): 32-bit episode index */
+    int64_t     state_env_stride; /* vectors between consecutive envs; 0 means 1 (planes).  12/V with
+                                state_stride 1 is the row layout.  Layouts whose envs overlap are COPTER_E_RANGE */
 } CopterBuffers;
 
 /*
@@ -265,7 +275,7 @@ int copter_reset_force_f64(const CopterParams* p, double* out, const uint32_t* e
 /*
  * The policy network of the rollout loop the reference's consumers run on the host -- obs -> net
  * -> clip -> env.step (attic/drl/3dtest.py:36-61) -- as one kernel: the tanh MLP
- * O -> 64 -> 64 -> A of BASELINE.json configs[4], reading the env's fp32 state planes in place
+ * O -> 64 -> 64 -> A of BASELINE.json configs[4], reading the env's fp32 state in place
  * (observation = state components first..first+O-1 of the variant) and writing the action rows
  * copter_step_f32 consumes:  action = out_offset + out_scale * tanh(W3 tanh(W2 tanh(W1 obs + b1) + b2) + b3).
  * Weights use the torch.nn.Linear layouts W[out][in] (fp32, device memory); they and the
@@ -284,6 +294,12 @@ int copter_policy_mlp_f32(const void* state, int64_t state_stride, int64_t n, in
                           const float* w1, const float* b1, const float* w2, const float* b2,
                           const float* w3, const float* b3, float out_scale, float out_offset,
                           float* action, void* stream);
+/* The same on any state layout: state_env_stride vectors between consecutive envs (0 means 1, which is
+   copter_policy_mlp_f32); the row layout of "Memory layout" is state_stride 1, state_env_stride 3. */
+int copter_policy_mlp_strided_f32(const void* state, int64_t state_stride, int64_t state_env_stride, int64_t n,
+                                  int variant, int hidden, const float* w1, const float* b1, const float* w2,
+                                  const float* b2, const float* w3, const float* b3, float out_scale,
+                                  float out_offset, float* action, void* stream);
 
 /*
  * Policy-in-the-loop rollout in ONE launch: for n_steps steps, action_t = policy(obs_t) with the

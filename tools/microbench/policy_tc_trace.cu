@@ -29,7 +29,7 @@ int main(int argc, char** argv) {
     CK(cudaMemcpy(state, h.data(), h.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(wd, w.data(), w.size() * 4, cudaMemcpyHostToDevice));
     tc::Args a;
-    a.state = state; a.stride = n; a.n = n;
+    a.state = state; a.stride = n; a.env_stride = 1; a.n = n;
     a.w1 = wd; a.b1 = wd + 640; a.w2 = wd + 704; a.b2 = wd + 704 + 4096; a.w3 = wd + 704 + 4160; a.b3 = wd + 704 + 4160 + 256;
     a.out_scale = 1.f; a.out_offset = 0.f; a.action = action;
     constexpr auto kernel = tc::copter_mlp_policy_tc_kernel<0, 10, 4>;
