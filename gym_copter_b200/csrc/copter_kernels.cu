@@ -113,7 +113,11 @@ __device__ __forceinline__ void flush_episode_stats(double* stats, int lane, boo
     const unsigned full = 0xffffffffu;
     const unsigned ended = __ballot_sync(full, ended_lane);
     if (!ended) return;
-    const int len_sum = __reduce_add_sync(full, ended_lane ? ep_len : 0);
+    // The lengths are summed as 16-bit halves: with wide counters an episode lasts up to 2^30 - 2 steps, and
+    // 32 of those overflow a 32-bit sum (which the REDUX would return wrapped).
+    const unsigned len = ended_lane ? (unsigned)ep_len : 0u;
+    const unsigned len_lo = __reduce_add_sync(full, len & 0xFFFFu), len_hi = __reduce_add_sync(full, len >> 16);
+    const double len_sum = (double)len_hi * 65536.0 + (double)len_lo;
     double ret_sum = ended_lane ? (double)ep_ret : 0.0;
     if (has_returns) {
 #pragma unroll
@@ -125,7 +129,7 @@ __device__ __forceinline__ void flush_episode_stats(double* stats, int lane, boo
     if (lane == 0) {
         double* row = stats + (size_t)((blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5)) % COPTER_STATS_SLOTS) * COPTER_STATS_LEN;
         atomicAdd(&row[COPTER_STAT_EPISODES], (double)__popc(ended));
-        atomicAdd(&row[COPTER_STAT_LENGTH_SUM], (double)len_sum);
+        atomicAdd(&row[COPTER_STAT_LENGTH_SUM], len_sum);
         if (has_returns) atomicAdd(&row[COPTER_STAT_RETURN_SUM], ret_sum);
         // cause bits: LANDED, BONUS, OOB, ANGLE, CRASHED, TIMEOUT
         const int slot[6] = {COPTER_STAT_LANDED, COPTER_STAT_BONUS, COPTER_STAT_OOB, COPTER_STAT_ANGLE, COPTER_STAT_CRASHED, COPTER_STAT_TIMEOUT};

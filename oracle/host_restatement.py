@@ -66,12 +66,22 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
 
 
+# the episode statistics of include/copter_b200.h (COPTER_STAT_*), in the order of CopterVecEnv.stats()
+STAT_NAMES = ('episodes', 'return_sum', 'length_sum', 'landed', 'bonus', 'crashed', 'oob', 'angle', 'timeout', 'env_steps')
+CAUSE_STATS = (('landed', 1), ('bonus', 2), ('oob', 4), ('angle', 8), ('crashed', 16), ('timeout', 32))
+
+
 class HostEnvBatch:
     """N envs stepped by the host instantiation of the kernels' arithmetic.  `x` [N,12], `status`,
-    `steps`, `episode` are the per-env state; obs / reward / done of the last call are attributes."""
+    `steps`, `episode` are the per-env state; obs / reward / done of the last call are attributes.
+
+    It also keeps the ledger the kernels keep with track_stats / track_returns (`stats()`, `ep_return`):
+    per ended episode one count, its length final_steps - 1 and its cause bits; every executed substep
+    in env_steps; with `track_returns` the running return of each env in the env dtype, added to
+    return_sum and zeroed where an episode ends (with or without auto-reset) and by reset()."""
 
     def __init__(self, variant, n, params=None, dtype=np.float32, seed=0, env_offset=0, auto_reset=True,
-                 env_ids=None, wide=False, **param_overrides):
+                 env_ids=None, wide=False, track_returns=False, **param_overrides):
         self.lib = load()
         self.variant, self.vid, self.n = variant, VARIANT_ID[variant], int(n)
         self.obs_size, self.act_size = len(_SHAPES[variant][1]), _SHAPES[variant][2]
@@ -90,6 +100,9 @@ class HostEnvBatch:
         self.cause, self.executed = np.zeros(n, np.uint8), np.zeros(n, np.int32)
         self.final_steps = np.zeros(n, np.int32)
         self._ever_reset = False
+        self.ep_return = np.zeros(n, self.dtype) if track_returns else None
+        self.ledger = dict.fromkeys(STAT_NAMES, 0)
+        self.ledger['return_sum'] = 0.0
 
     def reset(self, force=None, keep_episode=None):
         """keep_episode=None mirrors the product's host shell: the first reset starts every env at
@@ -99,6 +112,8 @@ class HostEnvBatch:
         fn(C.byref(self.p), self.vid, int(self.wide), C.c_int64(self.n), _p(self.x), _p(self.status), _p(self.steps),
            _p(self.episode), int(keep), _p(self.obs))
         self._ever_reset = True
+        if self.ep_return is not None:
+            self.ep_return[:] = 0
         return self.obs
 
     def step(self, action, k_substeps=1, force=None):
@@ -110,8 +125,28 @@ class HostEnvBatch:
                       int(k_substeps), int(self.auto_reset), _p(self.obs), _p(self.reward), _p(self.done), _p(self.cause),
                       _p(self.executed), _p(self.final_obs), _p(self.final_steps))
         assert executed >= 0
+        self._book(self.done.view(np.bool_))
         return self.obs, self.reward, self.done.view(np.bool_), {
             'cause': self.cause, 'executed': self.executed, 'final_obs': self.final_obs, 'final_steps': self.final_steps}
+
+    def _book(self, ended):
+        led = self.ledger
+        led['episodes'] += int(ended.sum())
+        led['length_sum'] += int((self.final_steps[ended].astype(np.int64) - 1).sum())
+        for name, bit in CAUSE_STATS:
+            led[name] += int(((self.cause & bit) != 0)[ended].sum())
+        led['env_steps'] += int(self.executed.astype(np.int64).sum())
+        if self.ep_return is not None:
+            self.ep_return += self.reward                  # one rounding in the env dtype, as the kernels' `ret += total`
+            led['return_sum'] += float(self.ep_return[ended].astype(np.float64).sum())
+            self.ep_return[ended] = 0
+
+    def stats(self):
+        """The ledger with the keys (and the two means) of CopterVecEnv.stats()."""
+        out = {k: float(v) for k, v in self.ledger.items()}
+        ep = max(out['episodes'], 1.0)
+        out['mean_return'], out['mean_length'] = out['return_sum'] / ep, out['length_sum'] / ep
+        return out
 
 
 class HostDynamicsBatch:

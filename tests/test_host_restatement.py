@@ -16,7 +16,7 @@ import pytest
 
 from oracle.copter_oracle import ALL_VARIANTS, DynamicsBatch, EnvBatch, OracleParams, reset_force
 from oracle.c_oracle import CEnvBatch
-from oracle.host_restatement import HostDynamicsBatch, HostEnvBatch, sincos_f32, load, make_params
+from oracle.host_restatement import CAUSE_STATS, STAT_NAMES, HostDynamicsBatch, HostEnvBatch, sincos_f32, load, make_params
 
 HOVER = 0.016560178212092172
 
@@ -70,6 +70,53 @@ def test_fp64_instantiation_matches_the_reference_pinned_oracle(variant, k):
     assert episodes >= 40
     if variant == 'Takeoff':
         assert (h.x[:, 4] < -0.5).any() and (h.status == 3).any()       # vehicles did leave the ground
+
+
+@pytest.mark.parametrize('auto_reset', [True, False], ids=['auto', 'noreset'])
+@pytest.mark.parametrize('k', [1, 3, 16])
+@pytest.mark.parametrize('variant', list(ALL_VARIANTS))
+def test_host_ledger_counts_equal_the_oracle(variant, k, auto_reset):
+    """HostEnvBatch.stats() -- the statistics the kernels keep -- against the same counts derived from the
+    numpy oracle's endings (steps_taken, final_steps, cause) on the same commands: exact.  A short step limit,
+    a low start and tight bounds end episodes of every kind; the runs stay below 2047 steps, where the oracle's
+    unsaturated counter and the counter field agree."""
+    N, T = 64, 384 // k
+    rng = np.random.default_rng(5 * k + sum(map(ord, variant)))
+    A = ALL_VARIANTS[variant][2]
+    act = mixed_streams(rng, N, T, A).astype(np.float64)
+    kw = dict(max_steps=60, initial_altitude=1.0, bounds=2.0)
+    if variant == 'Takeoff':
+        kw.update(initial_altitude=0.0, initial_random_force=0.0)
+        act = np.abs(act) + rng.uniform(0, 0.01, act.shape)
+    h = HostEnvBatch(variant, N, OracleParams(**kw), dtype=np.float64, seed=9, auto_reset=auto_reset, track_returns=True)
+    o = EnvBatch(variant, N, OracleParams(**kw), seed=9, auto_reset=auto_reset)
+    h.reset(); o.reset()
+    want = dict.fromkeys(('episodes', 'length_sum', 'env_steps') + tuple(c for c, _ in CAUSE_STATS), 0)
+    o_ret, o_return_sum = np.zeros(N), 0.0
+    for t in range(T):
+        _, r, d, _ = h.step(act[t], k)
+        _, o_r, o_d, o_info = o.step(act[t], k)
+        assert np.array_equal(d, o_d), t
+        want['episodes'] += int(o_d.sum())
+        want['length_sum'] += int((o_info['final_steps'][o_d] - 1).sum())
+        want['env_steps'] += int(o_info['steps_taken'].sum())
+        for name, bit in CAUSE_STATS:
+            want[name] += int(((o_info['cause'][o_d] & bit) != 0).sum())
+        o_ret += o_r
+        o_return_sum += float(o_ret[o_d].sum())
+        o_ret[o_d] = 0.0
+    assert int(o.steps.max()) < 2047
+    s = h.stats()
+    assert {k_: s[k_] for k_ in want} == {k_: float(v) for k_, v in want.items()}, (s, want)
+    assert set(s) == set(STAT_NAMES) | {'mean_return', 'mean_length'}
+    assert s['episodes'] >= N and s['timeout'] > 0
+    assert variant == 'Takeoff' or sum(s[c] > 0 for c, _ in CAUSE_STATS) >= (2 if variant.endswith('1D') else 3), s
+    # the returns: the K-fused host telescopes what the oracle sums step by step
+    assert abs(s['return_sum'] - o_return_sum) <= 1e-9 * max(abs(o_return_sum), 1.0) * T, (s['return_sum'], o_return_sum)
+    assert np.allclose(h.ep_return, o_ret, rtol=1e-9, atol=1e-9)
+    # reset() zeroes the running returns, not the ledger
+    h.reset()
+    assert not h.ep_return.any() and h.stats() == s
 
 
 def fp32_flip_study(variant, kind, k, n, t, seed=3):
