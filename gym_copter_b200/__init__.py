@@ -12,7 +12,8 @@ from .envs import (CopterVecEnv, LanderVec, Lander3DVec, Lander2DVec, Lander1DVe
                    Lander1D, Hover3D, Hover2D, Hover1D, Takeoff, SingleEnv, make)
 from .dynamics import Dynamics                                                         # noqa: F401
 from .sharding import shard_range, make_sharded_env, all_reduce_stats                  # noqa: F401
-from .rollout import FusedMLPPolicy, FusedPolicyRollout, PolicyRollout, PlanarLinear, gae, mlp_policy                                    # noqa: F401
+from .rollout import (FusedMLPPolicy, FusedMLPValue, FusedPolicyRollout, PolicyRollout, PlanarLinear,   # noqa: F401
+                      gae, mlp_policy)
 from .gym_compat import register_envs, make_vector_env                                 # noqa: F401
 from .export import CsvTrajectoryWriter                                                # noqa: F401
 

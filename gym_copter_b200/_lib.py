@@ -9,7 +9,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 # COPTER_B200_LIB: developer knob used by tools/sweep.py to time alternative builds
 LIB_PATH = os.environ.get('COPTER_B200_LIB') or os.path.join(PKG, 'libcopter_b200.so')
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 STATS_LEN = 16
 STATS_SLOTS = 64
 F_AUTO_RESET, F_KEEP_EPISODE = 1, 2
@@ -119,6 +119,10 @@ def load():
     lib.copter_policy_rollout_f32.restype = i32
     lib.copter_gae_f32.argtypes = [vp, vp, vp, vp, vp, i64, i32, C.c_float, C.c_float, vp, vp, vp]
     lib.copter_gae_f32.restype = i32
+    lib.copter_value_mlp_f32.argtypes = [vp, i64, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp, C.c_uint32, vp, vp]
+    lib.copter_value_mlp_f32.restype = i32
+    lib.copter_policy_logp_f32.argtypes = [u64, i64, i64, i64, i32, i32, vp, vp, vp]
+    lib.copter_policy_logp_f32.restype = i32
     lib.copter_pipeline_create.argtypes, lib.copter_pipeline_create.restype = [i32, C.POINTER(vp)], i32
     lib.copter_pipeline_destroy.argtypes, lib.copter_pipeline_destroy.restype = [vp], i32
     for f in (lib.copter_step_host_f32, lib.copter_step_host_f64):

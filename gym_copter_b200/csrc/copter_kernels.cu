@@ -983,6 +983,37 @@ __global__ void __launch_bounds__(kGaeBlock) copter_gae_kernel(const __grid_cons
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// Log-probability of the policy rollout's sampled actions (copter_policy_logp_f32).  The rollout
+// draws action = mu + std * xi with xi = draw_variates(seed, env, step, tag 2), so the density of
+// what it sampled needs no network: log N(a; mu, std^2) = -1/2 sum xi_j^2 - sum log std_j - A/2 log 2 pi,
+// from the same xi bits the rollout drew (the same device function).  One thread per env walks
+// its T steps; every row t is one coalesced store of the warp.  Philox and the Box-Muller
+// transform are the cost (HBM sees 4 bytes per env-step).
+// ------------------------------------------------------------------------------------------
+struct LogpArgs {
+    uint64_t seed; int64_t env_offset, n, first_step; int n_steps;
+    const float* action_std; float* logp;
+};
+constexpr int kLogpBlock = 256;
+
+template <int A>
+__global__ void __launch_bounds__(kLogpBlock) copter_policy_logp_kernel(const __grid_constant__ LogpArgs a) {
+    const int64_t i = (int64_t)blockIdx.x * kLogpBlock + threadIdx.x;
+    if (i >= a.n) return;
+    float c = -0.5f * (float)A * 1.8378770664093453f;              // log 2 pi
+#pragma unroll
+    for (int j = 0; j < A; ++j) c -= logf(a.action_std[j]);
+    for (int t = 0; t < a.n_steps; ++t) {
+        float xi[4];
+        draw_variates<float>(a.seed, (uint64_t)(a.env_offset + i), (uint64_t)(a.first_step + t), 2u, false, xi);
+        float q = 0.0f;
+#pragma unroll
+        for (int j = 0; j < A; ++j) q = fmaf(xi[j], xi[j], q);
+        __stcs(a.logp + (int64_t)t * a.n + i, fmaf(-0.5f, q, c));
+    }
+}
+
 template <typename T, int VARIANT>
 __global__ void __launch_bounds__(kBlock)
 copter_reset_kernel(const __grid_constant__ KParams<T> kp, T* state, uint32_t* meta, uint32_t* meta_hi, float* obs, T* ep_return,
@@ -1324,6 +1355,22 @@ int launch_policy_v(const PolicyArgs& a, cudaStream_t s) {
     return (int)cudaGetLastError();
 }
 
+// the critic: one instantiation per observation size (Variant<>: 2, 6, 10, 12)
+template <int OBS>
+int launch_value_o(const tc::ValueArgs& a, cudaStream_t s) {
+    constexpr auto kernel = tc::copter_value_tc_kernel<OBS>;
+    constexpr int smem = (int)sizeof(tc::Smem) + 128;
+    static bool configured[kMaxDevices] = {false};
+    const int dev = current_device();
+    if (!configured[dev]) {
+        if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
+        configured[dev] = true;
+    }
+    const int64_t tiles = (a.n + tc::kTile - 1) / tc::kTile;
+    kernel<<<(int)tiles, tc::kThreads, smem, s>>>(a);                // cluster launch control, as above
+    return (int)cudaGetLastError();
+}
+
 template <int VARIANT, bool STATS, bool RECORD>
 int launch_policy_rollout_tc(const KParams<float>& kp, const PolicyRolloutArgs& a, cudaStream_t s) {
     constexpr auto kernel = copter_policy_rollout_tc_kernel<VARIANT, STATS, RECORD>;
@@ -1621,6 +1668,48 @@ int copter_gae_f32(const float* reward_tn, const float* value_tn, const float* l
     a.reward = reward_tn; a.value = value_tn; a.last_value = last_value; a.cause = cause_tn; a.final_value = final_value_tn;
     a.adv = adv_tn; a.ret = ret_tn; a.n = n; a.n_steps = n_steps; a.gamma = gamma; a.lam = lam;
     copter_gae_kernel<<<(int)blocks, kGaeBlock, 0, (cudaStream_t)stream>>>(a);
+    return (int)cudaGetLastError();
+}
+
+int copter_value_mlp_f32(const float* rows, int64_t row_stride, int64_t m, int variant, int hidden,
+                         const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                         const uint8_t* select, uint32_t select_mask, float* value, void* stream) {
+    if (!rows || !w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !value || m < 0) return COPTER_E_ARG;
+    const int obs = copter_obs_size(variant);
+    if (obs < 0) return COPTER_E_VARIANT;
+    if (row_stride < obs || hidden != kPolH || (m + tc::kTile - 1) / tc::kTile > 0x7fffffff) return COPTER_E_RANGE;
+    for (const void* ptr : {(const void*)rows, (const void*)w1, (const void*)b1, (const void*)w2, (const void*)b2, (const void*)w3,
+                            (const void*)b3, (const void*)value})
+        if (reinterpret_cast<uintptr_t>(ptr) & 3u) return COPTER_E_ALIGN;
+    if (m == 0) return 0;
+    tc::ValueArgs a;
+    a.rows = rows; a.row_stride = row_stride; a.n = m; a.select = select; a.select_mask = select_mask;
+    a.w1 = w1; a.b1 = b1; a.w2 = w2; a.b2 = b2; a.w3 = w3; a.b3 = b3; a.value = value;
+    cudaStream_t s = (cudaStream_t)stream;
+    switch (obs) {
+        case 2:  return launch_value_o<2>(a, s);
+        case 6:  return launch_value_o<6>(a, s);
+        case 10: return launch_value_o<10>(a, s);
+        default: return launch_value_o<12>(a, s);
+    }
+}
+
+int copter_policy_logp_f32(uint64_t seed, int64_t env_offset, int64_t n, int64_t first_step, int n_steps, int variant,
+                           const float* action_std, float* logp_tn, void* stream) {
+    if (!action_std || !logp_tn || n < 0 || n_steps < 1) return COPTER_E_ARG;
+    const int act = copter_action_size(variant);
+    if (act < 0) return COPTER_E_VARIANT;
+    if (env_offset < 0 || first_step < 0 || (n + kLogpBlock - 1) / kLogpBlock > 0x7fffffff) return COPTER_E_RANGE;
+    if ((reinterpret_cast<uintptr_t>(action_std) & 3u) || (reinterpret_cast<uintptr_t>(logp_tn) & 3u)) return COPTER_E_ALIGN;
+    if (n == 0) return 0;
+    LogpArgs a;
+    a.seed = seed; a.env_offset = env_offset; a.n = n; a.first_step = first_step; a.n_steps = n_steps;
+    a.action_std = action_std; a.logp = logp_tn;
+    const int blocks = (int)((n + kLogpBlock - 1) / kLogpBlock);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (act == 4) copter_policy_logp_kernel<4><<<blocks, kLogpBlock, 0, s>>>(a);
+    else if (act == 2) copter_policy_logp_kernel<2><<<blocks, kLogpBlock, 0, s>>>(a);
+    else copter_policy_logp_kernel<1><<<blocks, kLogpBlock, 0, s>>>(a);
     return (int)cudaGetLastError();
 }
 

@@ -408,7 +408,71 @@ __device__ __forceinline__ void request_tile(Smem& sm, int k_next) {
 }
 constexpr int kThreads = kTile + 32;      // the epilogue warps + the MMA warp
 
-// env state -> action rows.  Persistent, warp-specialised CTAs (weights converted once per CTA), 128 envs
+// ---- where a tile's observation rows come from (the source) and where its outputs go (the head) ----
+// Sources and heads are types only: they read their pointers and sizes from the kernel's __grid_constant__ arguments
+// in place (copied into a struct, the policy kernel's values stayed in registers and spilled).  A source also says
+// which rows are evaluated: selected(i) for one row and, where kSelect, tile_live(tile) for the whole tile (called by
+// every warp of both roles, converged; each reaches the same answer from the same bytes, with no message between them).
+// The env state (Args): float4 `pl` of env i at pl * stride + i * env_stride; the observation is components
+// FIRST .. FIRST + OBS - 1.
+template <int FIRST_, int OBS_>
+struct StateRows {
+    static constexpr int FIRST = FIRST_, OBS = OBS_;
+    static constexpr bool kSelect = false;
+    template <class A> __device__ static __forceinline__ void fetch(const A& a, int64_t i, float4 (&p)[3]) {
+        const float4* env = reinterpret_cast<const float4*>(a.state) + i * a.env_stride;
+        p[0] = env[0]; p[1] = env[a.stride]; p[2] = env[2 * a.stride];
+    }
+    template <class A> __device__ static __forceinline__ bool selected(const A&, int64_t) { return true; }
+    template <class A> __device__ static __forceinline__ bool tile_live(const A&, uint32_t) { return true; }
+};
+// Packed fp32 observation rows (ValueArgs): row r at rows + r * row_stride floats (row_stride >= OBS; 4-byte alignment
+// is enough: the loads are scalar, and they are not the bound).  With `select`, only rows with select[r] & mask are
+// evaluated; a tile without one skips its MMAs and epilogue.
+template <int OBS_>
+struct ObsRows {
+    static constexpr int FIRST = 0, OBS = OBS_;
+    static constexpr bool kSelect = true;
+    template <class A> __device__ static __forceinline__ void fetch(const A& a, int64_t i, float4 (&p)[3]) {
+        float s[12];
+#pragma unroll
+        for (int j = 0; j < 12; ++j) s[j] = j < OBS ? __ldg(a.rows + i * a.row_stride + j) : 0.0f;
+        p[0] = make_float4(s[0], s[1], s[2], s[3]); p[1] = make_float4(s[4], s[5], s[6], s[7]); p[2] = make_float4(s[8], s[9], s[10], s[11]);
+    }
+    template <class A> __device__ static __forceinline__ bool selected(const A& a, int64_t i) {
+        return !a.select || (__ldg(a.select + i) & a.select_mask) != 0;
+    }
+    template <class A> __device__ static __forceinline__ bool tile_live(const A& a, uint32_t tile) {   // the tile's 128 select bytes, 4 per lane
+        if (!a.select) return true;
+        bool any = false;
+#pragma unroll
+        for (int q = 0; q < kTile / 32; ++q) {
+            const int64_t i = (int64_t)tile * kTile + q * 32 + (threadIdx.x & 31);
+            any |= i < a.n && (__ldg(a.select + i) & a.select_mask) != 0;
+        }
+        return __any_sync(0xffffffffu, any);
+    }
+};
+// the policy's action rows [n][ACT] (Args): out_offset + out_scale * tanh(layer 3)
+template <int ACT_>
+struct ActionHead {
+    static constexpr int ACT = ACT_;
+    template <class A> __device__ static __forceinline__ void store(const A& a, int64_t i, const float (&pre)[4]) {
+        float act[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) act[j] = fmaf(a.out_scale, tanh_mufu(pre[j]), a.out_offset);
+        if constexpr (ACT == 4) reinterpret_cast<float4*>(a.action)[i] = make_float4(act[0], act[1], act[2], act[3]);
+        else if constexpr (ACT == 2) reinterpret_cast<float2*>(a.action)[i] = make_float2(act[0], act[1]);
+        else a.action[i] = act[0];
+    }
+};
+// the critic's value [n] (ValueArgs): layer 3's accumulator column 0, no tanh
+struct ValueHead {
+    static constexpr int ACT = 1;
+    template <class A> __device__ static __forceinline__ void store(const A& a, int64_t i, const float (&pre)[4]) { a.value[i] = pre[0]; }
+};
+
+// observation rows -> outputs.  Persistent, warp-specialised CTAs (weights converted once per CTA), 128 rows
 // per tile, one tile in flight per CTA, the tiles taken by cluster launch control (next_tile).
 //   epilogue warps   one thread per env row: pull the accumulator out of TMEM, tanh, fp16, write it to shared
 //              memory as the next layer's A operand, arrive on ready; after layer 3 store the env's action and
@@ -432,9 +496,13 @@ constexpr int kThreads = kTile + 32;      // the epilogue warps + the MMA warp
 //   one CTA, 370 B/clk/SM from four, and tcgen05.ld overlaps tanh.approx completely; the MUFU floor is 0.19 ms)
 // (The loop with several tiles in flight per CTA or two epilogue threads per row: the last tree that has it is
 // commit d11af01.)
-template <int FIRST, int OBS, int ACT>
-__global__ void __launch_bounds__(kThreads, kCtasPerSm)
-copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
+// A tile without a selected row (tile_live false, ObsRows only) costs one handshake instead of three layers: the
+// epilogue threads arrive on ready once (the next tile's rows), the MMA warp waits for it, issues nothing and arrives on
+// done once, and the epilogue threads wait for that before they read the next tile's answer -- without that wait they
+// could complete two phases of ready before the MMA warp has seen the first.
+template <class Src, class Head, class A>
+__device__ __forceinline__ void mlp_tc_tiles(const A& a) {
+    constexpr int FIRST = Src::FIRST, OBS = Src::OBS, ACT = Head::ACT;
     static_assert(OBS <= 12 && ACT <= 4, "tile shapes");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
@@ -454,6 +522,10 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     fence_after_sync();
     TC_TRACE_CTA(1);
     const uint32_t tmem_base = sm.tmem_base;
+    auto tile_live = [&](uint32_t tl) {          // whole warp, converged
+        if constexpr (Src::kSelect) return tl != kNoTile && Src::tile_live(a, tl);
+        else return true;
+    };
 
     // Tile k of this CTA: k = 0 is blockIdx.x; tile k + 1 is the answer to try_cancel k.
     // The MMA warp keeps one try_cancel in flight; both roles read answer k from clc_resp[k & 1] after clc_bar[k & 1]
@@ -463,62 +535,76 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     if (warp == kMmaWarp) {
         const LayerDescs d = make_layer_descs(sm, tmem_base);
         uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
+        bool live = tile_live(tile);
         request_tile(sm, 0);
         for (int k = 0; tile != kNoTile; ++k) {
             bar_wait(&sm.ready, phase); phase ^= 1u;
             TC_TRACE((t & 31) == 0, 4, k, 0);
-            issue_layer_uniform(d, 1, &sm.done);
+            if (live) issue_layer_uniform(d, 1, &sm.done);
+            else { if (elect_one()) bar_arrive(&sm.done); __syncwarp(); }
             TC_TRACE((t & 31) == 0, 4, k, 2);
             const uint32_t nxt = next_tile(sm, k, clc_phase);
             if (nxt != kNoTile) request_tile(sm, k + 1);          // (a failed try_cancel is the last one)
+            if (live) {
 #pragma unroll
-            for (int layer = 2; layer <= 3; ++layer) {
-                bar_wait(&sm.ready, phase); phase ^= 1u;
-                TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1));
-                issue_layer_uniform(d, layer, &sm.done);
-                TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1) + 2);
+                for (int layer = 2; layer <= 3; ++layer) {
+                    bar_wait(&sm.ready, phase); phase ^= 1u;
+                    TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1));
+                    issue_layer_uniform(d, layer, &sm.done);
+                    TC_TRACE((t & 31) == 0, 4, k, 3 * (layer - 1) + 2);
+                }
             }
             tile = nxt;
+            live = tile_live(tile);
         }
     } else {
         const int row = t;
         const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);       // this warp's quarter of the 128 TMEM lanes
-        auto fetch = [&](uint32_t tl, float4 (&p)[3]) {
+        auto fetch = [&](uint32_t tl, bool tl_live, float4 (&p)[3]) {
             const int64_t i = (int64_t)tl * kTile + row;
-            const float4* env = reinterpret_cast<const float4*>(a.state) + i * a.env_stride;
-            if (tl != kNoTile && i < a.n) { p[0] = env[0]; p[1] = env[a.stride]; p[2] = env[2 * a.stride]; }
+            if (tl != kNoTile && tl_live && i < a.n) Src::fetch(a, i, p);
             else p[0] = p[1] = p[2] = make_float4(0.f, 0.f, 0.f, 0.f);
         };
         uint32_t tile = blockIdx.x, phase = 0, clc_phase = 0;
+        bool live = tile_live(tile);
         float4 nxt[3];
-        fetch(tile, nxt);
+        fetch(tile, live, nxt);
         write_obs_row<FIRST, OBS>(sm.slot, row, nxt);
         fence_before_sync();
         bar_arrive(&sm.ready);
         for (int k = 0; tile != kNoTile; ++k) {
             uint32_t nxt_tile = kNoTile;
+            bool nxt_live = false;
+            float pre[4];
+            if (live) {
 #pragma unroll
-            for (int layer = 1; layer <= 2; ++layer) {
+                for (int layer = 1; layer <= 2; ++layer) {
+                    bar_wait(&sm.done, phase); phase ^= 1u;
+                    fence_after_sync();
+                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1));
+                    hidden_epilogue<true>(lane_base + kColHidden, sm.slot.a, row, k, 12 + 8 * (layer - 1));      // (layer 2 overwrites the tile its finished MMAs read)
+                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 1);
+                    fence_async_smem();
+                    fence_before_sync();
+                    bar_arrive(&sm.ready);
+                    TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 2);
+                    if (layer == 1) {                                    // under layer 2's MMAs: which tile is next, and its state on the way
+                        nxt_tile = next_tile(sm, k, clc_phase);
+                        nxt_live = tile_live(nxt_tile);
+                        fetch(nxt_tile, nxt_live, nxt);
+                    }
+                }
                 bar_wait(&sm.done, phase); phase ^= 1u;
                 fence_after_sync();
-                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1));
-                hidden_epilogue<true>(lane_base + kColHidden, sm.slot.a, row, k, 12 + 8 * (layer - 1));      // (layer 2 overwrites the tile its finished MMAs read)
-                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 1);
-                fence_async_smem();
-                fence_before_sync();
-                bar_arrive(&sm.ready);
-                TC_TRACE((t & 31) == 0, warp, k, 3 * (layer - 1) + 2);
-                if (layer == 1) {                                    // under layer 2's MMAs: which tile is next, and its state on the way
-                    nxt_tile = next_tile(sm, k, clc_phase);
-                    fetch(nxt_tile, nxt);
-                }
+                TC_TRACE((t & 31) == 0, warp, k, 6);
+                tmem_ld4(lane_base + kColOut, pre);
+                TC_TRACE((t & 31) == 0, warp, k, 7);
+            } else {                                                 // the MMA warp has taken this tile's handshake
+                bar_wait(&sm.done, phase); phase ^= 1u;
+                nxt_tile = next_tile(sm, k, clc_phase);
+                nxt_live = tile_live(nxt_tile);
+                fetch(nxt_tile, nxt_live, nxt);
             }
-            bar_wait(&sm.done, phase); phase ^= 1u;
-            fence_after_sync();
-            TC_TRACE((t & 31) == 0, warp, k, 6);
-            float pre[4];
-            tmem_ld4(lane_base + kColOut, pre);
-            TC_TRACE((t & 31) == 0, warp, k, 7);
             if (nxt_tile != kNoTile) {                               // the next tile's observation row first: the MMA warp is waiting for it
                 write_obs_row<FIRST, OBS>(sm.slot, row, nxt);
                 fence_before_sync();
@@ -526,15 +612,9 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
                 TC_TRACE((t & 31) == 0, warp, k, 8);
             }
             const int64_t i = (int64_t)tile * kTile + row;
-            if (i < a.n) {
-                float act[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) act[j] = fmaf(a.out_scale, tanh_mufu(pre[j]), a.out_offset);
-                if constexpr (ACT == 4) reinterpret_cast<float4*>(a.action)[i] = make_float4(act[0], act[1], act[2], act[3]);
-                else if constexpr (ACT == 2) reinterpret_cast<float2*>(a.action)[i] = make_float2(act[0], act[1]);
-                else a.action[i] = act[0];
-            }
+            if (live && i < a.n && Src::selected(a, i)) Head::store(a, i, pre);
             tile = nxt_tile;
+            live = nxt_live;
         }
     }
     TC_TRACE_CTA(2);
@@ -542,6 +622,30 @@ copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
     __syncthreads();
     if (warp == kMmaWarp) tmem_free(tmem_base);
     TC_TRACE_CTA(3);
+}
+
+// env state -> action rows (copter_policy_mlp_strided_f32)
+template <int FIRST, int OBS, int ACT>
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
+copter_mlp_policy_tc_kernel(const __grid_constant__ Args a) {
+    mlp_tc_tiles<StateRows<FIRST, OBS>, ActionHead<ACT>>(a);
+}
+
+// observation rows -> values (copter_value_mlp_f32): the critic O -> 64 -> 64 -> 1, layer 3 linear
+struct ValueArgs {
+    const float* rows; int64_t row_stride, n;
+    const uint8_t* select; uint32_t select_mask;     // select nullable
+    const float *w1, *b1, *w2, *b2, *w3, *b3;        // w3 [1][64], b3 [1]
+    float* value;                                    // [n]
+};
+// 5 CTAs per SM, 80 registers (__maxnreg__): the selection adds state to every role, and at the policy's 7 CTAs (56 registers) or at
+// 6 (64) the kernel spilled 8-52 bytes per thread; unbounded it takes 72-80.  The policy kernel measured 0.321 ms at 5
+// CTAs per SM and 0.322 at 6 (profiles/r2_sweep_policy_tc_ctas.txt).
+constexpr int kValueCtasPerSm = 5;
+template <int OBS>
+__global__ void __maxnreg__(65536 / (kThreads * kValueCtasPerSm) / 8 * 8)
+copter_value_tc_kernel(const __grid_constant__ ValueArgs a) {
+    mlp_tc_tiles<ObsRows<OBS>, ValueHead>(a);
 }
 
 }  // namespace tc

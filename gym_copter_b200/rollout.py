@@ -179,6 +179,94 @@ class FusedMLPPolicy:
         return self.action
 
 
+class FusedMLPValue:
+    """
+    The critic Linear(O,64) -> Tanh -> Linear(64,64) -> Tanh -> Linear(64,1) (linear output) evaluated by ONE
+    tcgen05 kernel (copter_value_mlp_f32) on fp32 observation rows read in place: a rollout's `obs` / `final_obs`
+    [T,N,O], the env's `obs` (a view of its state rows), or any [..., O] tensor whose last dimension has stride 1
+    and whose leading dimensions flatten to one stride.  The same rounding as the tcgen05 policy kernel (bf16 rows,
+    fp16 hidden activations, fp32 accumulation).  Weights are read in place (fp32), so optimizer updates are seen by
+    the next call.
+
+    net             torch.nn.Sequential with those three Linear layers (bias included), fp32, contiguous, on a
+                    CUDA device
+    variant_or_env  a CopterVecEnv or a variant name: sets O (and the device the parameters must be on)
+    """
+
+    def __init__(self, net, variant_or_env):
+        if isinstance(variant_or_env, str):
+            if variant_or_env not in VARIANT_IDS:
+                raise CopterError('unknown variant %r' % (variant_or_env,))
+            self.variant, device = variant_or_env, None
+        else:
+            self.variant, device = variant_or_env.variant, variant_or_env.device
+        self.lib = _lib.load()
+        self.obs_size = self.lib.copter_obs_size(VARIANT_IDS[self.variant])
+        lin = [m for m in net if isinstance(m, torch.nn.Linear)]
+        if len(lin) != 3 or lin[0].in_features != self.obs_size or lin[0].out_features != 64 or lin[1].in_features != 64 \
+                or lin[1].out_features != 64 or lin[2].in_features != 64 or lin[2].out_features != 1:
+            raise CopterError('FusedMLPValue needs Linear(O,64), Linear(64,64), Linear(64,1) with tanh activations')
+        if device is None:
+            device = lin[0].weight.device
+        self.device = torch.device(device)
+        self.params = []
+        for m in lin:
+            for p in (m.weight, m.bias):
+                if p is None or p.dtype != torch.float32 or p.device.type != 'cuda' or p.device != self.device \
+                        or not p.is_contiguous():
+                    raise CopterError('critic parameters must be contiguous fp32 tensors (with bias) on the CUDA device')
+                self.params.append(p)
+        self.launches = 0
+
+    def __call__(self, rows, select=None, mask=_lib.CAUSE_TIMEOUT, out=None):
+        """values [rows.shape[:-1]] fp32.  With `select` (uint8, rows.shape[:-1]) only rows where select & mask != 0
+        are evaluated; the other values are left as they were in `out` (zeros when out is None)."""
+        O = self.obs_size
+        if not isinstance(rows, torch.Tensor) or rows.dtype != torch.float32 or rows.dim() < 1 or rows.shape[-1] != O:
+            raise CopterError('rows must be an fp32 tensor [..., %d]' % O)
+        if rows.device != self.device:
+            raise CopterError('rows must be on the critic device %s' % self.device)
+        shape = tuple(rows.shape[:-1])
+        if rows.stride(-1) != 1:
+            raise CopterError('the last dimension of rows must have stride 1')
+        try:
+            flat = rows.view(-1, O)
+        except RuntimeError:
+            raise CopterError('the leading dimensions of rows must flatten to one stride') from None
+        m = flat.shape[0]
+        stride = flat.stride(0) if m > 1 else O
+        if select is not None and (not isinstance(select, torch.Tensor) or select.dtype != torch.uint8
+                                   or tuple(select.shape) != shape or select.device != self.device
+                                   or not select.is_contiguous()):
+            raise CopterError('select must be a contiguous uint8 tensor of shape %s on the critic device' % (shape,))
+        if out is None:
+            out = (torch.zeros if select is not None else torch.empty)(shape, dtype=torch.float32, device=self.device)
+        elif not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or tuple(out.shape) != shape \
+                or out.device != self.device or not out.is_contiguous():
+            raise CopterError('out must be a contiguous fp32 tensor of shape %s on the critic device' % (shape,))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.copter_value_mlp_f32(
+                flat.data_ptr(), stride, m, VARIANT_IDS[self.variant], 64, *[p.data_ptr() for p in self.params],
+                select.data_ptr() if select is not None else None, int(mask) & 0xFFFFFFFF, out.data_ptr(),
+                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), 'copter_value_mlp')
+        self.launches += 1
+        return out
+
+
+def policy_log_probs(env, action_std, first_step, horizon, out=None):
+    """log N(action; policy(obs), std^2) [T,N] of the actions a FusedPolicyRollout with `action_std` sampled on `env`
+    over steps first_step .. first_step + T - 1 (copter_policy_logp_f32): regenerated from the rollout's own noise
+    draws, so no network runs and the value is that of the distribution the action was drawn from."""
+    if out is None:
+        out = torch.empty((int(horizon), env.num_envs), dtype=torch.float32, device=env.device)
+    with torch.cuda.device(env.device):
+        _lib.check(_lib.load().copter_policy_logp_f32(
+            env.seed_value & 0xFFFFFFFFFFFFFFFF, env.env_offset, env.num_envs, int(first_step), int(horizon),
+            VARIANT_IDS[env.variant], action_std.data_ptr(), out.data_ptr(),
+            C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)), 'copter_policy_logp')
+    return out
+
+
 class FusedPolicyRollout(_EndingRecords):
     """
     The whole policy-in-the-loop horizon as ONE kernel launch (copter_policy_rollout_f32): every
@@ -199,10 +287,19 @@ class FusedPolicyRollout(_EndingRecords):
     store_causes / store_final_obs   also record `causes` [T,N] uint8 and `final_obs` [T,N,O] as
                 PolicyRollout does (the step-limit truncations a learner bootstraps from the value of
                 final_obs; `terminated` / `truncated` [T,N] bool are derived from causes)
+    critic      None, or the critic torch.nn.Sequential(Linear(O,64), Tanh, Linear(64,64), Tanh, Linear(64,1))
+                (fp32, read in place; see FusedMLPValue).  run() then also queues, on the same stream:
+                  values [T,N]       the critic on obs (needs store_obs)
+                  last_values [N]    the critic on the env's observation after the last step
+                  final_values [T,N] the critic on final_obs where the step limit fired, 0 elsewhere
+                                     (when store_causes and store_final_obs are set; else None)
+    store_log_probs  also record log_probs [T,N]: log N(action; policy(obs), action_std^2) of each sampled
+                action, regenerated from the rollout's own noise draws (needs action_std)
+    advantages(gamma, lam) is gae() on exactly those buffers (needs a critic and store_causes).
     """
 
     def __init__(self, env, net, horizon, out_scale=1.0, out_offset=0.0, store_obs=False, store_actions=False,
-                 action_std=None, store_causes=False, store_final_obs=False):
+                 action_std=None, store_causes=False, store_final_obs=False, critic=None, store_log_probs=False):
         probe = FusedMLPPolicy(env, net, out_scale, out_offset)       # same parameter checks
         if env.k_substeps != 1:
             raise CopterError('FusedPolicyRollout steps with k_substeps == 1')
@@ -225,7 +322,20 @@ class FusedPolicyRollout(_EndingRecords):
         self.actions = torch.zeros((self.horizon, n, env.action_size), dtype=torch.float32, device=dev) if store_actions else None
         self.causes = torch.zeros((self.horizon, n), dtype=torch.uint8, device=dev) if store_causes else None
         self.final_obs = torch.zeros((self.horizon, n, env.obs_size), dtype=torch.float32, device=dev) if store_final_obs else None
-        self.launches_per_rollout = 1
+        self.critic = self.values = self.last_values = self.final_values = self.log_probs = None
+        if critic is not None:
+            if not store_obs:
+                raise CopterError('a critic needs store_obs=True (the values are those of obs)')
+            self.critic = FusedMLPValue(critic, env)
+            self.values = torch.zeros((self.horizon, n), dtype=torch.float32, device=dev)
+            self.last_values = torch.zeros(n, dtype=torch.float32, device=dev)
+            if store_causes and store_final_obs:
+                self.final_values = torch.zeros((self.horizon, n), dtype=torch.float32, device=dev)
+        if store_log_probs:
+            if action_std is None:
+                raise CopterError('store_log_probs needs action_std (a deterministic policy has no density)')
+            self.log_probs = torch.zeros((self.horizon, n), dtype=torch.float32, device=dev)
+        self.launches_per_rollout = 1 + (0 if critic is None else 2 + (self.final_values is not None)) + bool(store_log_probs)
 
     def run(self):
         """One horizon. Returns (rewards [T,N], dones [T,N] bool view, last_obs [N,O] or None)."""
@@ -243,9 +353,25 @@ class FusedPolicyRollout(_EndingRecords):
                 self.causes.data_ptr() if self.causes is not None else None,
                 self.final_obs.data_ptr() if self.final_obs is not None else None,
                 C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)), 'copter_policy_rollout')
+            first_step = env.rollout_step
+            if self.critic is not None:
+                self.critic(self.obs, out=self.values)
+                self.critic(env.obs, out=self.last_values)
+                if self.final_values is not None:
+                    self.final_values.zero_()
+                    self.critic(self.final_obs, select=self.causes, mask=_lib.CAUSE_TIMEOUT, out=self.final_values)
+            if self.log_probs is not None:
+                policy_log_probs(env, self.action_std, first_step, self.horizon, out=self.log_probs)
         env.launches += 1
         env.rollout_step += self.horizon
         return self.rewards, self.dones.view(torch.bool), env.obs if env.write_obs else None
+
+    def advantages(self, gamma=0.99, lam=0.95):
+        """gae() on this rollout's rewards, values, last_values, causes and final_values: (advantages, returns)
+        [T,N].  Without final_values (store_final_obs off) truncations are treated as terminations."""
+        if self.critic is None or self.causes is None:
+            raise CopterError('advantages() needs a critic and store_causes=True')
+        return gae(self.rewards, self.values, self.last_values, self.causes, self.final_values, gamma, lam)
 
 
 def gae(rewards, values, last_values, causes, final_values=None, gamma=0.99, lam=0.95):

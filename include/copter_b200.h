@@ -65,7 +65,7 @@
 extern "C" {
 #endif
 
-#define COPTER_ABI_VERSION 5
+#define COPTER_ABI_VERSION 6
 
 /* dynamics/__init__.py:65-68 */
 enum { COPTER_STATUS_CRASHED = 0, COPTER_STATUS_LANDED = 1, COPTER_STATUS_LEVELING = 2, COPTER_STATUS_AIRBORNE = 3 };
@@ -355,6 +355,43 @@ int copter_gae_f32(const float* reward_tn, const float* value_tn, const float* l
                    const uint8_t* cause_tn, const float* final_value_tn_or_null,
                    int64_t n, int n_steps, float gamma, float lam,
                    float* adv_tn, float* ret_tn_or_null, void* stream);
+
+/*
+ * The critic of an on-policy learner, Linear(O,64) -> tanh -> Linear(64,64) -> tanh -> Linear(64,1)
+ * (linear output), on m fp32 observation rows: row r is rows[r * row_stride + 0 .. O-1]
+ * (row_stride >= O floats, O = copter_obs_size(variant); 4-byte alignment is enough), so the
+ * packed obs_tn / final_obs_tn rows of copter_policy_rollout_f32 (stride O) and the fp32 env's
+ * observation inside its state rows (stride 12) are both read in place.  w1 [64][O], b1 [64],
+ * w2 [64][64], b2 [64], w3 [1][64], b3 [1] (torch.nn.Linear layouts, fp32 device memory, read
+ * on every call).  The tcgen05 kernel of copter_policy_mlp_f32 with a value head: bf16 rows and
+ * layer-1 weights, fp16 hidden activations and layer-2 / -3 weights, biases as 16-bit hi + lo,
+ * fp32 accumulation; value[r] = layer 3's accumulator.
+ * select_or_null (uint8[m]): when given, only rows with select[r] & select_mask are evaluated and
+ * every other value[r] is left untouched (e.g. final_obs_tn at cause_tn & COPTER_CAUSE_TIMEOUT,
+ * the only rows copter_gae_f32 reads).
+ * COPTER_E_ARG for a NULL required pointer or m < 0; COPTER_E_VARIANT; COPTER_E_RANGE for
+ * row_stride < O or hidden != 64; COPTER_E_ALIGN for a float pointer that is not 4-byte aligned.
+ * m == 0 is a no-op.
+ */
+int copter_value_mlp_f32(const float* rows, int64_t row_stride, int64_t m, int variant, int hidden,
+                         const float* w1, const float* b1, const float* w2, const float* b2,
+                         const float* w3, const float* b3,
+                         const uint8_t* select_or_null, uint32_t select_mask,
+                         float* value, void* stream);
+
+/*
+ * Log-probability of the actions copter_policy_rollout_f32 sampled with exploration noise
+ * (policy->action_std), for the same seed, env_offset, n, first_step and variant:
+ *     logp_tn[t][i] = -1/2 sum_j xi_j^2 - sum_j log action_std[j] - (A/2) log(2 pi),   j < A
+ * with xi the rollout's own N(0,1) draws of (seed, env_offset + i, first_step + t): exactly the
+ * density the action was drawn from, whichever rollout kernel ran and however the rollout was
+ * sharded or cut into horizons.  action_std float[A] (device, read in place), logp_tn
+ * float[n_steps][n].  COPTER_E_ARG for a NULL pointer, n < 0 or n_steps < 1; COPTER_E_VARIANT;
+ * COPTER_E_RANGE for env_offset < 0 or first_step < 0; COPTER_E_ALIGN for a pointer that is not
+ * 4-byte aligned.  n == 0 is a no-op.
+ */
+int copter_policy_logp_f32(uint64_t seed, int64_t env_offset, int64_t n, int64_t first_step, int n_steps,
+                           int variant, const float* action_std, float* logp_tn, void* stream);
 
 /*
  * The same step for callers that hold HOST arrays (the reference's callers pass numpy
