@@ -259,7 +259,7 @@ def gae_inputs(rng, T, n):
     return f(T, n), f(T, n), f(n), torch.as_tensor(random_causes(rng, T, n), device='cuda'), f(T, n)
 
 
-@pytest.mark.parametrize('T', [1, 7, 32])
+@pytest.mark.parametrize('T', [1, 7, 8, 9, 17, 32])  # kGaeRows = 8: 8 is one block; 9 and 17 end on a one-row block
 @pytest.mark.parametrize('n', [1, 31, 4099, 2 ** 20 + 3])
 def test_gae_equals_float64_definition(pkg, T, n):
     """Tolerance: fp32 rounding of a T-term recursion.  Every step rounds a handful of times (gamma * boot, the two

@@ -16,7 +16,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from oracle import value_oracle as vo                     # noqa: E402
-from oracle.copter_oracle import source_actions           # noqa: E402
+from oracle import noise_oracle as no                     # noqa: E402
 
 CASES = {c['name']: c for c in vo.critic_cases()}
 SENTINEL = 0x7FC0DEAD
@@ -171,16 +171,21 @@ def test_log_probs_formula_and_cross_checks(pkg):
     c = -np.log(s64).sum() - 2.0 * np.log(2 * np.pi)
     c_env = mk()
     mean_k = pkg.FusedMLPPolicy(c_env, pol.net, out_scale=0.01, out_offset=0.0166)
+    s32 = std.cpu().numpy()
     for t in range(T):
-        xi = source_actions(seed, ids, 2 ** 32 + 7 + t, 'randn', 1.0, 0.0, 4, np.float64, tag=2)
+        xi, rad = no.gaussian_variates(seed, ids, 2 ** 32 + 7 + t, 2)
         ref = -0.5 * (xi ** 2).sum(1) + c
-        assert np.max(np.abs(lp[t] - ref)) <= 1e-5 * (1 + np.abs(ref)).max(), t
+        lpb = no.log_prob_bound(xi, s32, 4)
+        assert np.all(np.abs(lp[t] - ref) <= lpb), (t, float(np.max(np.abs(lp[t] - ref) / lpb)))
         st = torch.zeros((n, 12), device='cuda')
         st[:, :10] = ro.obs[t]
         c_env.set_state(st)
-        z = ((ro.actions[t] - mean_k()).cpu().numpy().astype(np.float64)) / s64
-        # (action - mu) / std: fp32 cancellation, 2e-4 per variate (test_fused_policy_rollout_exploration_noise)
-        bound = (np.abs(z) * 2e-4 + 2e-4 ** 2).sum(1) + 1e-5 * (1 + np.abs(ref))
+        a32 = ro.actions[t].cpu().numpy()
+        z = (a32.astype(np.float64) - mean_k().cpu().numpy()) / s64
+        # (action - mu) / std is the device variate to half an ulp of the action over std, and that variate is the
+        # reference to its own error: -1/2 z^2 moves from -1/2 xi^2 by |xi| eta + eta^2 / 2 per component
+        eta = np.spacing(np.abs(a32)) / (2.0 * s64) + no.pair_bound(rad, 4)
+        bound = no.SLACK * (np.abs(xi) * eta + 0.5 * eta ** 2).sum(1) + lpb
         assert np.all(np.abs(lp[t] - (-0.5 * (z ** 2).sum(1) + c)) <= bound), t
     # two shards
     lib = _lib.load()
