@@ -45,21 +45,25 @@ def make_params(op=None, **kw):
     return p
 
 
-_lib = None
+_libs = {}
 
 
-def load():
-    global _lib
-    if _lib is None:
-        srcs = [os.path.join(HERE, 'copter_host.cpp'),
-                os.path.join(HERE, '..', 'gym_copter_b200', 'csrc', 'copter_core.h'),
-                os.path.join(HERE, '..', 'include', 'copter_b200.h')]
-        if not os.path.exists(LIB) or any(os.path.exists(s) and os.path.getmtime(LIB) < os.path.getmtime(s) for s in srcs):
-            subprocess.run(['make', '-s', '-C', HERE, 'libcopter_host.so'], check=True)
-        _lib = C.CDLL(LIB)
-        for f in (_lib.copter_host_step_f32, _lib.copter_host_step_f64):
+def load(lib=None):
+    """The host instantiation: the repository's own (built here on first use), or the one at path `lib`, e.g. a
+    build of a modified copter_core.h."""
+    path = LIB if lib is None else os.path.abspath(lib)
+    if path not in _libs:
+        if lib is None:
+            srcs = [os.path.join(HERE, 'copter_host.cpp'),
+                    os.path.join(HERE, '..', 'gym_copter_b200', 'csrc', 'copter_core.h'),
+                    os.path.join(HERE, '..', 'include', 'copter_b200.h')]
+            if not os.path.exists(LIB) or any(os.path.exists(s) and os.path.getmtime(LIB) < os.path.getmtime(s) for s in srcs):
+                subprocess.run(['make', '-s', '-C', HERE, 'libcopter_host.so'], check=True)
+        h = C.CDLL(path)
+        for f in (h.copter_host_step_f32, h.copter_host_step_f64):
             f.restype = C.c_int64
-    return _lib
+        _libs[path] = h
+    return _libs[path]
 
 
 def _p(a):
@@ -81,8 +85,8 @@ class HostEnvBatch:
     return_sum and zeroed where an episode ends (with or without auto-reset) and by reset()."""
 
     def __init__(self, variant, n, params=None, dtype=np.float32, seed=0, env_offset=0, auto_reset=True,
-                 env_ids=None, wide=False, track_returns=False, **param_overrides):
-        self.lib = load()
+                 env_ids=None, wide=False, track_returns=False, lib=None, **param_overrides):
+        self.lib = load(lib)
         self.variant, self.vid, self.n = variant, VARIANT_ID[variant], int(n)
         self.obs_size, self.act_size = len(_SHAPES[variant][1]), _SHAPES[variant][2]
         self.dtype = np.dtype(dtype)
@@ -152,8 +156,8 @@ class HostEnvBatch:
 class HostDynamicsBatch:
     """Dynamics.setMotors driven directly (the restatement of copter_dynamics_*)."""
 
-    def __init__(self, n, params=None, dtype=np.float64, **param_overrides):
-        self.lib = load()
+    def __init__(self, n, params=None, dtype=np.float64, lib=None, **param_overrides):
+        self.lib = load(lib)
         self.n, self.dtype = int(n), np.dtype(dtype)
         self.p = params if isinstance(params, HostParams) else make_params(params, **param_overrides)
         self.x = np.zeros((n, 12), self.dtype)
