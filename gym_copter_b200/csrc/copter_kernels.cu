@@ -25,6 +25,7 @@ struct StepArgs {
     T* state; uint32_t* meta; uint32_t* meta_hi; const T* action; float* obs; T* reward; uint8_t* done;
     const T* init_force; T* ep_return; double* stats; float* final_obs; uint8_t* cause;
     int64_t n, stride, env_stride, env_offset; uint64_t seed; int k; int auto_reset;
+    int64_t prefetch_ahead;     // > 0: tile t asks L2 for the inputs of tile t + prefetch_ahead (prefetch_tile)
 };
 
 // One env's inputs exactly as they sit in HBM (128-bit vectors): load_raw issues every load, and
@@ -308,6 +309,32 @@ __device__ __forceinline__ void step_tile(const KParams<T>& kp, const StepArgs<T
     }
 }
 
+// A fp32 K = 1 step moves 68 B per env into the SM, but a CTA issues its loads only when it starts and then holds
+// its slot through ~500 warp-instructions of arithmetic per 32 envs, so the bytes in flight from HBM sag whenever
+// the resident CTAs compute at once: the step ran 11-17 % above the same byte pattern without the arithmetic
+// (profiles/k1_ceiling_and_bulk_prefetch.txt).  So thread 0 of each CTA asks L2 for the inputs of the tile
+// `prefetch_ahead` tiles later -- about one wave of resident CTAs ahead, so the lines arrive before that CTA
+// starts and are still in L2 when it does -- with bulk prefetches (cp.async.bulk.prefetch.L2: no registers,
+// no shared memory, nothing to wait for), and that CTA's own loads then hit L2.  The same bytes come from HBM,
+// earlier rather than twice: one wave of tiles is ~13 MB of the 126 MB L2.  Used on device memory in 16-byte
+// aligned rows or planes only (launch_step); a tile past the last full one is not prefetched.  Results are
+// unchanged: the prefetch only moves lines into L2.
+__device__ __forceinline__ void prefetch_l2(const void* p, uint32_t bytes) {
+    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" :: "l"(p), "r"(bytes) : "memory");
+}
+template <typename T, int A>
+__device__ __forceinline__ void prefetch_tile(const StepArgs<T>& a, int64_t tile) {
+    if (threadIdx.x != 0 || (tile + 1) * kBlock > a.n) return;
+    const int64_t row0 = tile * kBlock;
+    if (a.env_stride == 1) {                                          // planes: one block per plane
+        for (int pl = 0; pl < 3; ++pl) prefetch_l2(reinterpret_cast<const float4*>(a.state) + pl * a.stride + row0, kBlock * 16);
+    } else {                                                          // rows: the tile's rows are one block
+        prefetch_l2(a.state + row0 * 12, kBlock * 48);
+    }
+    prefetch_l2(a.action + row0 * A, kBlock * A * sizeof(T));
+    prefetch_l2(a.meta + row0, kBlock * 4);
+}
+
 template <typename T, int VARIANT, bool STATS>
 __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? COPTER_STEP_CTAS_PER_SM : 2)
 copter_step_kernel(const __grid_constant__ KParams<T> kp, const __grid_constant__ StepArgs<T> a) {
@@ -318,6 +345,7 @@ copter_step_kernel(const __grid_constant__ KParams<T> kp, const __grid_constant_
 
     // the grid holds exactly one CTA per tile (launch_step_v), so there is no tile loop and no tile
     // count to derive
+    if constexpr (sizeof(T) == 4) if (a.prefetch_ahead) prefetch_tile<T, Variant<VARIANT>::A>(a, (int64_t)blockIdx.x + a.prefetch_ahead);
     if (a.k == 1) step_tile<T, VARIANT, STATS, true>(kp, a, &tiles[0][0], (int64_t)blockIdx.x);
     else          step_tile<T, VARIANT, STATS, false>(kp, a, &tiles[0][0], (int64_t)blockIdx.x);
 }
@@ -1155,9 +1183,11 @@ int launch_step_v(const KParams<T>& kp, const StepArgs<T>& a, cudaStream_t s) {
     return (int)cudaGetLastError();
 }
 
+// `device_arrays`: every buffer is device memory (not step_host's mapped host arrays), the condition for the
+// L2 prefetches of copter_step_kernel besides the ones launch_step checks itself.
 template <typename T>
 int launch_step(const CopterParams* p, const CopterBuffers* b, int64_t n, int64_t env_offset, uint64_t seed,
-                int k, int variant, int flags, void* stream) {
+                int k, int variant, int flags, void* stream, bool device_arrays = true) {
     if (!b) return COPTER_E_ARG;
     int e = check_params(p, b->meta_hi != nullptr);
     if (e) return e;
@@ -1172,6 +1202,11 @@ int launch_step(const CopterParams* p, const CopterBuffers* b, int64_t n, int64_
     a.reward = (T*)b->reward; a.done = b->done; a.init_force = (const T*)b->init_force;
     a.ep_return = (T*)b->ep_return; a.stats = b->stats; a.final_obs = b->final_obs; a.cause = b->cause;
     a.n = n; a.env_offset = env_offset; a.seed = seed; a.k = k; a.auto_reset = (flags & COPTER_F_AUTO_RESET) ? 1 : 0;
+    // fp32 K = 1 on device memory, rows or planes, 16-byte aligned: one wave of resident CTAs ahead (measured on B200:
+    // half a wave is level with it, two waves lose 3 % -- profiles/k1_l2_prefetch_ab.txt)
+    a.prefetch_ahead = 0;
+    if (sizeof(T) == 4 && k == 1 && device_arrays && aligned16(b->meta) && ((a.stride == 1 && a.env_stride == 3) || a.env_stride == 1))
+        a.prefetch_ahead = (int64_t)sm_count() * COPTER_STEP_CTAS_PER_SM;
     cudaStream_t s = (cudaStream_t)stream;
     switch (variant) {
         case COPTER_LANDER3D: return launch_step_v<T, COPTER_LANDER3D>(kp, a, s);
@@ -1471,7 +1506,7 @@ int step_host(Pipeline* pl, const CopterParams* p, const CopterBuffers* dev, con
             b.obs = want_obs ? (float*)d_obs : (dev->obs ? dev->obs : nullptr);
             b.cause = want_cause ? (uint8_t*)d_cause : dev->cause;
             b.final_obs = want_final ? (float*)d_final : dev->final_obs;
-            const int e = launch_step<T>(p, &b, n, env_offset, seed, k, variant, flags, (cudaStream_t)caller_stream);
+            const int e = launch_step<T>(p, &b, n, env_offset, seed, k, variant, flags, (cudaStream_t)caller_stream, false);
             if (e) return e;
             return (int)cudaStreamSynchronize((cudaStream_t)caller_stream);
         }
@@ -1497,7 +1532,7 @@ int step_host(Pipeline* pl, const CopterParams* p, const CopterBuffers* dev, con
         b.final_obs = dev->final_obs ? dev->final_obs + lo * O : nullptr;
         b.cause = dev->cause ? dev->cause + lo : nullptr;
         if ((ce = cudaMemcpyAsync((void*)b.action, (const T*)h_action + lo * A, sizeof(T) * m * A, cudaMemcpyHostToDevice, st)) != cudaSuccess) return (int)ce;
-        const int e = launch_step<T>(p, &b, m, env_offset + lo, seed, k, variant, flags, st);
+        const int e = launch_step<T>(p, &b, m, env_offset + lo, seed, k, variant, flags, st, false);
         if (e) return e;
         if (h_obs && b.obs && (ce = cudaMemcpyAsync(h_obs + lo * O, b.obs, sizeof(float) * m * O, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return (int)ce;
         if ((ce = cudaMemcpyAsync((T*)h_reward + lo, b.reward, sizeof(T) * m, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return (int)ce;
